@@ -16,6 +16,14 @@ roofline, cpu_baseline and parity sample:
     config5  16384 pairs partitioned across the ranks, NCCL pose gather (N > 1 only)     (strong scaling)
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--pairs P] [--solver gn|subgrad|lm]
+                    [--dump-outputs DIR]
+
+--steps sets the number of timed steps behind every config's `value` (the e2e legs time their own 2 to 5 passes).
+--dump-outputs DIR writes what the headline path returned in its last timed step as DIR/<name>.npy: poses.npy (pairs x 12
+float64: R row-major, then T; every rank's pairs in rank order) and the PairInfo fields of rank 0's pairs (status, npts,
+best_index, iterations_run as float64; best_energy, visible_ratio, laplacian_b as the float32 the library returns).  With
+--impl reference it writes the poses and status of the oracle's last step.  The inputs depend only on the arguments (seeded
+synthetic pairs), so two builds can be compared array for array.
 """
 import argparse
 import json
@@ -56,7 +64,35 @@ def parse():
     ap.add_argument("--total-pairs", type=int, default=16384, help="config5: pairs partitioned across all ranks")
     ap.add_argument("--sequences", type=int, default=148, help="config4: sequences per GPU")
     ap.add_argument("--seq-frames", type=int, default=8, help="config4: frames per sequence")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's outputs as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirpath, arrays):
+    """Each array as dirpath/<name>.npy in float64 (float32 arrays stay float32)."""
+    arrays = {k: np.asarray(v, np.float32 if np.asarray(v).dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(dirpath, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirpath, name + ".npy"), a)
+
+
+def pair_info_arrays(info):
+    """PairInfo records -> one array per field (per-level fields cut to the LEVELS levels in use)."""
+    out = {"status": [inf.status for inf in info], "laplacian_b": np.array([inf.laplacian_b for inf in info], np.float32)}
+    for f in ("npts", "best_index", "iterations_run"):
+        out[f] = [list(getattr(inf, f))[:LEVELS] for inf in info]
+    for f in ("best_energy", "visible_ratio"):
+        out[f] = np.array([list(getattr(inf, f))[:LEVELS] for inf in info], np.float32)
+    return out
 
 
 def solver_setup(args):
@@ -188,9 +224,11 @@ def run_reference(args):
     d = O.synth_batch(0, sample, W, H, K, nthreads=nthreads)
     times = []
     for s in range(args.warmup + args.steps):
-        _, _, secs = O.align_batch(d["ref_gray"], d["ref_depth"], d["now_gray"], LEVELS, iters, K, ocfg, nthreads=nthreads)
+        poses, status, secs = O.align_batch(d["ref_gray"], d["ref_depth"], d["now_gray"], LEVELS, iters, K, ocfg, nthreads=nthreads)
         if s >= args.warmup:
             times.append(secs)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"poses": poses, "status": status})
     per_step = float(np.mean(times))
     v = sample / per_step
     line = {"metric": METRIC, "value": v, "unit": "pairs/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -341,6 +379,9 @@ def bench_config2(env, args):
 
     # ---- parity of the timed batch: a fixed sample of its poses against the CPU oracle (the checker, not the thing measured)
     poses, info = al.get_poses(B)
+    if args.dump_outputs and rank == 0:
+        last = gathered if world > 1 else poses_buf[(step_no[0] - 1) % 2]
+        dump_outputs(args.dump_outputs, {"poses": last.cpu().numpy(), **pair_info_arrays(info)})
     sample_idx = sorted(set([0, 1, B // 3, (2 * B) // 3, B - 1]))
     max_drad = max_dm = 0.0
     for i in sample_idx:
@@ -491,7 +532,7 @@ def bench_config3(env, args, pcie_peak):
         step_dev()
     sampler = ClockSampler(env.local); sampler.start()
     l0 = est.launch_count()
-    nsteps = max(2, min(args.steps, 5))
+    nsteps = args.steps
     ms = env.timed(step_dev, nsteps)
     launches = est.launch_count() - l0
     clocks = sampler.finish()
@@ -566,7 +607,7 @@ def bench_config4(env, args, pcie_peak):
     rel, kind, reason, glob = run_dev()
     sampler = ClockSampler(env.local); sampler.start()
     l0 = al.launch_count()
-    nrun = 2
+    nrun = args.steps
     ms = env.timed(run_dev, nrun)
     launches = (al.launch_count() - l0) // nrun
     clocks = sampler.finish()
@@ -679,7 +720,7 @@ def bench_config5(env, args, pcie_peak):
 
     step()
     sampler = ClockSampler(env.local); sampler.start()
-    nsteps = max(2, min(args.steps, 3))
+    nsteps = args.steps
     ms = env.timed(step, nsteps)
     clocks = sampler.finish()
     parity = None
