@@ -200,6 +200,46 @@ int dvo_run_sequences_mem(dvo_ctx* ctx, int nseq, int nframes, const uint8_t* gr
                           const dvo_solver_params* params, const dvo_keyframe_policy* policy, double* rel_poses, int* kind,
                           int* reason, double* global_poses);
 
+/* ---- pose covariance ----
+ * For a slot whose frames were prepared and solved, the Gauss-Newton covariance of its returned pose (R, T), evaluated at
+ * pyramid level `level` on the frames resident in the slot:
+ *   H      = sum_i w_i J_i^T J_i over the points visible at (R, T), J = the EXACT Jacobian (DVO_JAC_EXACT) in EXACT arithmetic,
+ *            fp64 accumulation as the solver's; weight function, huber_k and residual come from `params` (solver, jacobian
+ *            and arithmetic are ignored: the REFERENCE Jacobian is not the derivative of the residual);
+ *   sigma2 = sum_i double(w_i) double(eps_i)^2 / (nvis - 6);
+ *   Sigma  = sigma2 H^-1 from a Cholesky factor of H (no damping term is added);
+ *   logdet = log det Sigma = 6 log sigma2 - log det H (for entropy-style criteria).
+ * Tangent convention: Sigma is the covariance of psi = (rho, omega), translation first, for the right-multiplicative update
+ * the solver applies, T <- T exp(psi) (cT += cR t(psi), cR <- cR R(psi)).  It describes the local curvature of the robust
+ * cost; nothing here claims it is calibrated against the true error.
+ * A slot whose level has no reference points or no now edges, fewer than 7 visible points, or an H that is not positive
+ * definite gets 36 NaNs (not zeros, which would claim certainty) and a status bit. */
+typedef struct dvo_cov_info {
+    int status;      /* 0 ok; bit0 no reference points / no now edges at the level; bit1 nvis < 7; bit2 H not positive definite */
+    int level;       /* level evaluated */
+    int nvis;        /* visible reference points at the pose */
+    double sigma2;   /* sum w eps^2 / (nvis - 6); NaN when status != 0 */
+    double logdet;   /* log det of the covariance; NaN when status != 0 */
+} dvo_cov_info;
+
+/* 6x6 covariance (row-major, 36 doubles per slot) of the pose the last dvo_run / dvo_process left in each slot, evaluated on
+ * the frames resident in the slots.  level = -1: the finest level with params->iters[l] > 0.  mem = DVO_MEM_HOST: host
+ * buffers, returns when they are filled; DVO_MEM_DEVICE: device buffers, asynchronous on the context stream (info may be NULL).
+ * One kernel launch for the whole range; the result of a slot does not depend on `count`, and no solver state is written.
+ * After dvo_align_batch with count > max_batch only the last chunk's frames and poses are resident. */
+int dvo_pose_covariance(dvo_ctx* ctx, int first, int count, const dvo_solver_params* params, int level,
+                        double* cov36, dvo_cov_info* info, int mem);
+
+/* dvo_run_sequences_mem plus per-frame covariances: rel_cov [nseq][nframes][36] of rel_poses (frame 0: zeros, it anchors
+ * the chain), global_cov [nseq][nframes][36] (may be NULL) of global_poses, first-order propagated along the key-frame chain:
+ *   Sigma_g(i) = Ad(Tr^-1) Sigma_key Ad(Tr^-1)^T + Sigma_rel(i),   Ad(R, t) = [[R, [t]x R], [0, R]],  Tr = rel_poses[i],
+ * Sigma_key = 0 at the start and Sigma_g(i) after every frame with kind[i] != 0.  The key-frame and relative estimates are
+ * treated as independent.  rel_cov[t] is evaluated at the finest level with iterations, against the reference frame t was
+ * finally solved against.  The poses, kinds, reasons and global poses equal those of dvo_run_sequences_mem bit for bit. */
+int dvo_run_sequences_cov(dvo_ctx* ctx, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem,
+                          const dvo_solver_params* params, const dvo_keyframe_policy* policy, double* rel_poses, int* kind,
+                          int* reason, double* global_poses, double* rel_cov, double* global_cov);
+
 /* ---- inspection (parity tests; not on the hot path) ---- */
 int dvo_level_dims(dvo_ctx* ctx, int level, int* w, int* h);
 int dvo_get_level_buffer(dvo_ctx* ctx, int slot, int frame, int level, int which, void* host_dst, size_t bytes);

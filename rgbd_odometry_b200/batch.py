@@ -4,7 +4,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import Config, KeyframePolicy, PairInfo, SolverParams, check
+from ._lib import Config, CovInfo, KeyframePolicy, PairInfo, SolverParams, check
 
 SUBGRAD_REF, GN, LM = 0, 1, 2
 JAC_REFERENCE, JAC_EXACT = 0, 1
@@ -190,6 +190,36 @@ class BatchAligner:
                                              C.byref(params), C.byref(policy), _ptr(rel), _ptr(kind), _ptr(reason), _ptr(glob)),
               "dvo_run_sequences_mem")
         return rel, kind, reason, glob
+
+    def run_sequences_cov(self, gray, depth, nseq, nframes, params, policy, device=False, want_global=True):
+        """dvo_run_sequences_cov: run_sequences_mem's (rel, kind, reason, glob) plus rel_cov (nseq, nframes, 6, 6) -- the covariance of
+        each relative pose, zeros at frame 0 -- and global_cov (nseq, nframes, 6, 6) propagated along the key-frame chain (None
+        unless want_global).  Tangent (rho, omega), translation first, for T <- T exp(psi)."""
+        rel = np.empty((nseq, nframes, 12), np.float64)
+        kind = np.empty((nseq, nframes), np.int32)
+        reason = np.empty((nseq, nframes), np.int32)
+        glob = np.empty((nseq, nframes, 19), np.float64) if want_global else None
+        rel_cov = np.empty((nseq, nframes, 6, 6), np.float64)
+        glob_cov = np.empty((nseq, nframes, 6, 6), np.float64) if want_global else None
+        check(self.lib.dvo_run_sequences_cov(self.h, nseq, nframes, _ptr(gray), _ptr(depth), MEM_DEVICE if device else MEM_HOST,
+                                             C.byref(params), C.byref(policy), _ptr(rel), _ptr(kind), _ptr(reason), _ptr(glob),
+                                             _ptr(rel_cov), _ptr(glob_cov)), "dvo_run_sequences_cov")
+        return rel, kind, reason, glob, rel_cov, glob_cov
+
+    def pose_covariance(self, count, params, first=0, level=-1):
+        """6x6 covariance of the pose the last solve left in slots [first, first+count), evaluated on the resident frames
+        (dvo_pose_covariance): returns (cov (count, 6, 6), info array of CovInfo).  level = -1: finest level with iterations."""
+        cov = np.empty((count, 6, 6), np.float64)
+        info = (CovInfo * max(count, 1))()
+        check(self.lib.dvo_pose_covariance(self.h, first, count, C.byref(params), level, _ptr(cov), C.cast(info, C.c_void_p), MEM_HOST),
+              "dvo_pose_covariance")
+        return cov, info
+
+    def pose_covariance_device(self, count, params, cov_ptr, first=0, level=-1, info_ptr=None):
+        """dvo_pose_covariance into device memory (count x 36 doubles at cov_ptr; optional count dvo_cov_info at info_ptr), asynchronous on
+        the context stream."""
+        check(self.lib.dvo_pose_covariance(self.h, first, count, C.byref(params), level, C.c_void_p(cov_ptr),
+                                           C.c_void_p(info_ptr) if info_ptr else None, MEM_DEVICE), "dvo_pose_covariance")
 
     def level_dims(self, level):
         w, h = C.c_int(), C.c_int()

@@ -169,7 +169,8 @@ int dvo_destroy(dvo_ctx* c) {
     for (int f = 0; f < 2; ++f) { cudaFree(c->gray[f]); cudaFree(c->depth[f]); cudaFree(c->edge[f]); }
     cudaFree(c->gcol); cudaFree(c->d2); cudaFree(c->texel); cudaFree(c->tex8); cudaFree(c->ptsX); cudaFree(c->ptsY); cudaFree(c->ptsZ); cudaFree(c->ptsPix);
     cudaFree(c->npts); cudaFree(c->solve_order); cudaFree(c->seq_mask); cudaFree(c->seq_state); cudaFree(c->nedge); cudaFree(c->maxd2); cudaFree(c->pose0); cudaFree(c->pose); cudaFree(c->info);
-    cudaFree(c->seq_rel); cudaFree(c->seq_kind); cudaFree(c->seq_reason); cudaFree(c->seq_glob);
+    cudaFree(c->seq_rel); cudaFree(c->seq_kind); cudaFree(c->seq_reason); cudaFree(c->seq_glob); cudaFree(c->seq_cov); cudaFree(c->seq_gcov);
+    cudaFree(c->cov_buf); cudaFree(c->cov_info_buf);
     for (int k = 0; k < 2; ++k) {
         cudaFree(c->seq_stage_g[k]); cudaFree(c->seq_stage_d[k]);
         if (c->seq_ev_ready[k]) cudaEventDestroy(c->seq_ev_ready[k]);
@@ -515,11 +516,17 @@ __global__ void seq_init_kernel(int nseq, int nframes, double* __restrict__ pose
 // launched at those frames and (b) the solve against the outgoing key frame, whose result the reference discards
 // (:2210-2227), is skipped.  With the quality gates the decision depends on that solve, so it runs and every frame from t = 2
 // on is followed by the masked pass (its kernels return at once for unflagged slots).
+//
+// rel_cov / global_cov (optional, dvo_run_sequences_cov): after each frame's final solve one cov_kernel launch evaluates every
+// slot at its final relative pose, on the reference it was finally solved against, into the device record at frame t.
 int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem, const dvo_solver_params* p,
-                       const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses) {
-    const char* who = "dvo_run_sequences";
+                       const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses,
+                       double* rel_cov, double* global_cov) {
+    const char* who = rel_cov ? "dvo_run_sequences_cov" : "dvo_run_sequences";
     if (c) { const int jr = join_aux(c); if (jr) return jr; }
-    if (!c || nseq < 1 || nseq > c->cfg.max_batch || nframes < 1 || !gray || !depth || !p || !pol || !rel_poses || !kind) { dvo_set_error("%s: bad argument", who); return DVO_ERR_ARG; }
+    if (!c || nseq < 1 || nseq > c->cfg.max_batch || nframes < 1 || !gray || !depth || !p || !pol || !rel_poses || !kind || (global_cov && !rel_cov)) {
+        dvo_set_error("%s: bad argument", who); return DVO_ERR_ARG;
+    }
     if (!c->prev_gray) { dvo_set_error("%s: create the context with keep_now_depth = 1", who); return DVO_ERR_STATE; }
     if (!c->haveK) { dvo_set_error("%s: intrinsics not set", who); return DVO_ERR_STATE; }
     int finest = -1;
@@ -546,6 +553,10 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
         }
         if (rc == DVO_OK) c->seq_stage_slots = (size_t)nseq;
     }
+    if (rel_cov && c->seq_cov_n < n) {
+        cudaFree(c->seq_cov); c->seq_cov = nullptr; c->seq_cov_n = 0;
+        if (!fail(cudaMalloc((void**)&c->seq_cov, sizeof(double) * 36 * n))) c->seq_cov_n = n;
+    }
     if (rc != DVO_OK) return rc;
     double* d_rel = c->seq_rel; int* d_kind = c->seq_kind; int* d_reason = c->seq_reason; double* d_glob = nullptr;
     uint8_t* stage_g[2] = {c->seq_stage_g[0], c->seq_stage_g[1]}; uint16_t* stage_d[2] = {c->seq_stage_d[0], c->seq_stage_d[1]};
@@ -553,6 +564,7 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
     fail(cudaMemsetAsync(d_rel, 0, sizeof(double) * 12 * n, c->stream));
     fail(cudaMemsetAsync(d_kind, 0, sizeof(int) * n, c->stream));
     fail(cudaMemsetAsync(d_reason, 0, sizeof(int) * n, c->stream));
+    if (rel_cov) fail(cudaMemsetAsync(c->seq_cov, 0, sizeof(double) * 36 * n, c->stream));          // frame 0 anchors the chain: zeros
     if (host_in) { fail(cudaEventRecord(c->ev_entry, c->stream)); fail(cudaStreamWaitEvent(c->copy_stream, c->ev_entry, 0)); }
 
     // frame t of every sequence: host -> staging buffer t & 1 on the copy stream
@@ -625,24 +637,32 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
             c->launches++;
             if (fail(cudaGetLastError())) break;
         }
+        // c->pose of every slot is now frame t's final relative pose, and its frames are the pair it was finally solved on
+        if (rel_cov && (rc = launch_cov(c, 0, nseq, finest, p, c->seq_cov + 36 * (size_t)t, nullptr, nframes))) break;
     }
     c->active = nullptr;
     c->timing = timing;
-    if (rc == DVO_OK && global_poses) {
+    if (rc == DVO_OK && (global_poses || global_cov)) {
         if (c->seq_glob_n < n) {
             cudaFree(c->seq_glob); c->seq_glob = nullptr; c->seq_glob_n = 0;
             if (!fail(cudaMalloc((void**)&c->seq_glob, sizeof(double) * 19 * n))) c->seq_glob_n = n;
         }
+        if (global_cov && rc == DVO_OK && c->seq_gcov_n < n) {
+            cudaFree(c->seq_gcov); c->seq_gcov = nullptr; c->seq_gcov_n = 0;
+            if (!fail(cudaMalloc((void**)&c->seq_gcov, sizeof(double) * 36 * n))) c->seq_gcov_n = n;
+        }
         d_glob = c->seq_glob;
         if (rc == DVO_OK) {
-            rc = launch_gop(c, nseq, nframes, d_kind, d_rel, d_glob);
-            if (rc == DVO_OK) fail(cudaMemcpyAsync(global_poses, d_glob, sizeof(double) * 19 * n, cudaMemcpyDeviceToHost, c->stream));
+            rc = launch_gop(c, nseq, nframes, d_kind, d_rel, d_glob, global_cov ? c->seq_cov : nullptr, global_cov ? c->seq_gcov : nullptr);
+            if (rc == DVO_OK && global_poses) fail(cudaMemcpyAsync(global_poses, d_glob, sizeof(double) * 19 * n, cudaMemcpyDeviceToHost, c->stream));
+            if (rc == DVO_OK && global_cov) fail(cudaMemcpyAsync(global_cov, c->seq_gcov, sizeof(double) * 36 * n, cudaMemcpyDeviceToHost, c->stream));
         }
     }
     if (rc == DVO_OK) {
         fail(cudaMemcpyAsync(rel_poses, d_rel, sizeof(double) * 12 * n, cudaMemcpyDeviceToHost, c->stream));
         fail(cudaMemcpyAsync(kind, d_kind, sizeof(int) * n, cudaMemcpyDeviceToHost, c->stream));
         if (reason) fail(cudaMemcpyAsync(reason, d_reason, sizeof(int) * n, cudaMemcpyDeviceToHost, c->stream));
+        if (rel_cov) fail(cudaMemcpyAsync(rel_cov, c->seq_cov, sizeof(double) * 36 * n, cudaMemcpyDeviceToHost, c->stream));
     }
     cudaStreamSynchronize(c->copy_stream);
     if (cudaStreamSynchronize(c->stream) != cudaSuccess && rc == DVO_OK) { dvo_set_error("%s: %s", who, cudaGetErrorString(cudaGetLastError())); rc = DVO_ERR_CUDA; }
@@ -656,17 +676,50 @@ int dvo_run_sequences(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, co
                       int keyframe_every, double* rel_poses, int* kind, double* global_poses) {
     dvo_keyframe_policy pol; memset(&pol, 0, sizeof(pol));
     pol.keyframe_every = keyframe_every; pol.use_quality_gates = 0; pol.laplacian_thresh = 3.0f; pol.visible_ratio_thresh = 0.8f; pol.min_reprojections = 50;
-    return run_sequences_core(c, nseq, nframes, gray, depth, DVO_MEM_HOST, p, &pol, rel_poses, kind, nullptr, global_poses);
+    return run_sequences_core(c, nseq, nframes, gray, depth, DVO_MEM_HOST, p, &pol, rel_poses, kind, nullptr, global_poses, nullptr, nullptr);
 }
 
 int dvo_run_sequences_gated(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, const dvo_solver_params* p,
                             const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses) {
-    return run_sequences_core(c, nseq, nframes, gray, depth, DVO_MEM_HOST, p, pol, rel_poses, kind, reason, global_poses);
+    return run_sequences_core(c, nseq, nframes, gray, depth, DVO_MEM_HOST, p, pol, rel_poses, kind, reason, global_poses, nullptr, nullptr);
 }
 
 int dvo_run_sequences_mem(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem, const dvo_solver_params* p,
                           const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses) {
-    return run_sequences_core(c, nseq, nframes, gray, depth, mem, p, pol, rel_poses, kind, reason, global_poses);
+    return run_sequences_core(c, nseq, nframes, gray, depth, mem, p, pol, rel_poses, kind, reason, global_poses, nullptr, nullptr);
+}
+
+int dvo_run_sequences_cov(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem, const dvo_solver_params* p,
+                          const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses, double* rel_cov,
+                          double* global_cov) {
+    if (!rel_cov) { dvo_set_error("dvo_run_sequences_cov: rel_cov is required"); return DVO_ERR_ARG; }
+    return run_sequences_core(c, nseq, nframes, gray, depth, mem, p, pol, rel_poses, kind, reason, global_poses, rel_cov, global_cov);
+}
+
+int dvo_pose_covariance(dvo_ctx* c, int first, int count, const dvo_solver_params* p, int level, double* cov36, dvo_cov_info* info, int mem) {
+    if (c) { const int jr = join_aux(c); if (jr) return jr; }
+    if (!range_ok(c, first, count) || !p || !cov36 || (mem != DVO_MEM_HOST && mem != DVO_MEM_DEVICE) || level < -1 || level >= c->geom.L ||
+        (p->residual != DVO_RESIDUAL_DT_FLOOR && p->residual != DVO_RESIDUAL_DT_INTERP)) {
+        dvo_set_error("dvo_pose_covariance: bad argument"); return DVO_ERR_ARG;
+    }
+    if (!c->haveK) { dvo_set_error("dvo_pose_covariance: intrinsics not set"); return DVO_ERR_STATE; }
+    if (level < 0) for (int l = 0; l < c->geom.L; ++l) if (p->iters[l] > 0) { level = l; break; }
+    if (level < 0) { dvo_set_error("dvo_pose_covariance: level = -1 and no level has iterations"); return DVO_ERR_ARG; }
+    if (count == 0) return DVO_OK;
+    if (mem == DVO_MEM_DEVICE) return launch_cov(c, first, count, level, p, cov36, info, 1);
+    if (c->cov_cap < (size_t)count) {                    // device results for host outputs: one buffer per context, grown on demand
+        DVO_CUDA(cudaStreamSynchronize(c->stream));
+        cudaFree(c->cov_buf); cudaFree(c->cov_info_buf); c->cov_buf = nullptr; c->cov_info_buf = nullptr; c->cov_cap = 0;
+        int rc = dalloc(&c->cov_buf, (size_t)count * 36); if (rc) return rc;
+        rc = dalloc(&c->cov_info_buf, (size_t)count); if (rc) return rc;
+        c->cov_cap = (size_t)count;
+    }
+    const int rc = launch_cov(c, first, count, level, p, c->cov_buf, c->cov_info_buf, 1);
+    if (rc) return rc;
+    DVO_CUDA(cudaMemcpyAsync(cov36, c->cov_buf, sizeof(double) * 36 * count, cudaMemcpyDeviceToHost, c->stream));
+    if (info) DVO_CUDA(cudaMemcpyAsync(info, c->cov_info_buf, sizeof(dvo_cov_info) * count, cudaMemcpyDeviceToHost, c->stream));
+    DVO_CUDA(cudaStreamSynchronize(c->stream));
+    return DVO_OK;
 }
 
 int dvo_level_dims(dvo_ctx* c, int level, int* w, int* h) {
@@ -877,7 +930,7 @@ int dvo_gop_compose(dvo_ctx* c, int nseq, int nframes, const int* kind, const do
     if (c) { const int jr = join_aux(c); if (jr) return jr; }
     if (!c || nseq < 1 || nframes < 1 || !kind || !rel || !out) return DVO_ERR_ARG;
     const size_t n = (size_t)nseq * nframes;
-    if (mem == DVO_MEM_DEVICE) return launch_gop(c, nseq, nframes, kind, rel, out);
+    if (mem == DVO_MEM_DEVICE) return launch_gop(c, nseq, nframes, kind, rel, out, nullptr, nullptr);
     int* d_kind = nullptr; double* d_rel = nullptr; double* d_out = nullptr;
     {
         cudaError_t e = cudaMalloc((void**)&d_kind, sizeof(int) * n);
@@ -891,7 +944,7 @@ int dvo_gop_compose(dvo_ctx* c, int nseq, int nframes, const int* kind, const do
             return DVO_ERR_CUDA;
         }
     }
-    int rc = launch_gop(c, nseq, nframes, d_kind, d_rel, d_out);
+    int rc = launch_gop(c, nseq, nframes, d_kind, d_rel, d_out, nullptr, nullptr);
     if (rc == DVO_OK) {
         cudaError_t e = cudaMemcpyAsync(out, d_out, sizeof(double) * 19 * n, cudaMemcpyDeviceToHost, c->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);

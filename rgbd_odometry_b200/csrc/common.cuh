@@ -67,6 +67,9 @@ struct dvo_ctx {
     uint8_t* seq_stage_g[2]; uint16_t* seq_stage_d[2]; size_t seq_stage_slots;
     cudaEvent_t seq_ev_ready[2], seq_ev_free[2];
     double* seq_rel; int* seq_kind; int* seq_reason; double* seq_glob; size_t seq_rec_n, seq_glob_n;
+    double* seq_cov; double* seq_gcov; size_t seq_cov_n, seq_gcov_n;   // per-frame relative / global covariances (dvo_run_sequences_cov)
+    // device results of dvo_pose_covariance with host outputs, grown on demand
+    double* cov_buf; dvo_cov_info* cov_info_buf; size_t cov_cap;
     int sm_count;
     int solve_shape;         // threads per pair in solve_kernel: 512 when max_batch <= sm_count (one pair per SM at most), else 256
     size_t smem_optin;
@@ -144,7 +147,10 @@ int launch_resolve_texels(dvo_ctx* c, int slot, int level, float4* d_out);
 int launch_solve(dvo_ctx* c, int first, int count, const dvo_solver_params* p);
 int launch_eval(dvo_ctx* c, int slot, int level, const double* d_pose12, int jac, int weight, int arith, float huber_k, int residual,
                 double* d_out /* 6 + 36 + 1 + 1 doubles */, float* d_eps, float* d_w, float* d_u, float* d_v, float* d_J);
-int launch_gop(dvo_ctx* c, int nseq, int nframes, const int* d_kind, const double* d_rel, double* d_out);
+// 6x6 pose covariance of slots [first, first+count) at their current pose (c->pose); record k at d_cov + 36 * k * stride
+int launch_cov(dvo_ctx* c, int first, int count, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info, long long stride);
+// d_rel_cov / d_glob_cov: both null, or [nseq][nframes][36] covariances to propagate along the key-frame chain
+int launch_gop(dvo_ctx* c, int nseq, int nframes, const int* d_kind, const double* d_rel, double* d_out, const double* d_rel_cov, double* d_glob_cov);
 int launch_promote(dvo_ctx* c, int first, int count);
 int launch_ingest_raw(dvo_ctx* c, int frame, int first, int count, const uint8_t* d_bgr, const float* d_depth_m);
 int launch_copy_bytes(dvo_ctx* c, void* dst, const void* src, size_t n);

@@ -373,12 +373,14 @@ __device__ __forceinline__ float interpolate_dt(const TexSrc& S, const LevelCam&
 
 // Accumulator layout: [0..5] g, [6] sum eps^2, [7] sum eps, then (NEED_H) 21 upper-triangle entries of H row by row.
 template <bool NEED_H> struct AccN { static constexpr int N = NEED_H ? 29 : 8; };
+// The covariance sweep (WSQ) appends [29] sum w eps^2 to the Gauss-Newton layout.
+constexpr int COV_NACC = AccN<true>::N + 1;
 
 // Software-pipelined sweep over a thread's points: the coordinates are loaded two points ahead and the (random)
 // texel gather of the next point is in flight while the current point's Jacobian / fp64 accumulation executes.
 // (A counted loop with unconditional look-ahead loads into slack behind the arrays, unrolled by 1 / 2 / 3, was measured slower:
 // 4.51 / 4.32 / 4.84 ms per 1024 pairs against 4.01 for this guarded form -- DESIGN.md "measured and rejected".)
-template <int ARITH, int JAC, bool NEED_H, int THREADS, bool OUT, int RES, int TEX, int WMODE>
+template <int ARITH, int JAC, bool NEED_H, int THREADS, bool OUT, int RES, int TEX, int WMODE, bool WSQ = false>
 __device__ __forceinline__ void accumulate_points(const float* __restrict__ X, const float* __restrict__ Y,
                                                   const float* __restrict__ Z, int N, const PoseF& P, const LevelCam& cam,
                                                   const TexSrc& S, int weight_mode_rt, float huber_k,
@@ -417,6 +419,7 @@ __device__ __forceinline__ void accumulate_points(const float* __restrict__ X, c
             const double de = (double)e;
             acc[6] = fma(de, de, acc[6]);
             acc[7] += de;
+            if constexpr (WSQ) acc[COV_NACC - 1] = fma((double)wgt * de, de, acc[COV_NACC - 1]);   // double(w) * double(eps) is exact
             double Jw[6];
 #pragma unroll
             for (int k = 0; k < 6; ++k) { Jw[k] = (double)A::mul(Jr[k], wgt); acc[k] = fma(Jw[k], de, acc[k]); }   // :714-720, :777
@@ -839,6 +842,121 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs a) {
     }
 }
 
+// ------------------------------------------------------------------ pose covariance (dvo_pose_covariance)
+// One CTA per slot evaluates the normal equations at the slot's returned pose c->pose with the EXACT Jacobian and EXACT
+// arithmetic (the derivative of the residual wrt T <- T exp(psi), psi = (rho, omega)), the caller's weight / Huber k /
+// residual, plus sum w eps^2; thread 0 then forms Sigma = sigma^2 H^-1 from a Cholesky factor of H.  The CTA shape is
+// fixed (COV_THREADS), so a slot's result never depends on how many slots share the launch.  Reads c->pose only.
+constexpr int COV_THREADS = 256;
+struct CovArgs {
+    PyrGeom geom; Intr K;
+    const float *X, *Y, *Z; const int* npts; const float4* texel;
+    const uint2* tex8; const int32_t* d2; const unsigned* maxd2; const unsigned* nedge_now;
+    const double* pose; int first, level, weight; float huber_k;
+    double* cov;            // 36 doubles per slot, record of CTA k at cov + 36 * k * stride
+    dvo_cov_info* info;     // optional, same indexing
+    long long stride;
+};
+
+// Serial tail on thread 0: H (full symmetric, row-major, in shared memory M[0..35]) -> Sigma = s2 H^-1 into out, log det H.
+// The factor overwrites M's lower triangle, L^-1 goes to M + 36.  Returns false when H is not positive definite.
+__device__ __forceinline__ bool cov_from_normal_matrix(double* M, double s2, double* out, double* logdetH) {
+    double* Li = M + 36;
+    double ld = 0.0;
+    for (int j = 0; j < 6; ++j) {
+        double d = M[6 * j + j];
+        for (int k = 0; k < j; ++k) d -= M[6 * j + k] * M[6 * j + k];
+        if (!(d > 0.0)) return false;
+        ld += log(d);
+        const double r = sqrt(d);
+        M[6 * j + j] = r;
+        for (int i = j + 1; i < 6; ++i) {
+            double v = M[6 * i + j];
+            for (int k = 0; k < j; ++k) v -= M[6 * i + k] * M[6 * j + k];
+            M[6 * i + j] = v / r;
+        }
+    }
+    for (int j = 0; j < 6; ++j) {                         // L^-1 (lower triangular), column by column
+        for (int i = 0; i < j; ++i) Li[6 * i + j] = 0.0;
+        Li[6 * j + j] = 1.0 / M[6 * j + j];
+        for (int i = j + 1; i < 6; ++i) {
+            double v = 0.0;
+            for (int k = j; k < i; ++k) v += M[6 * i + k] * Li[6 * k + j];
+            Li[6 * i + j] = -v / M[6 * i + i];
+        }
+    }
+    for (int i = 0; i < 6; ++i)                           // H^-1 = L^-T L^-1
+        for (int j = i; j < 6; ++j) {
+            double v = 0.0;
+            for (int k = j; k < 6; ++k) v += Li[6 * k + i] * Li[6 * k + j];
+            out[6 * i + j] = s2 * v; out[6 * j + i] = s2 * v;
+        }
+    *logdetH = ld;
+    return true;
+}
+
+template <int RES, int TEX>
+__global__ void __launch_bounds__(COV_THREADS) cov_kernel(CovArgs a) {
+    extern __shared__ float s_lut[];
+    constexpr int NACC = COV_NACC;
+    constexpr int WARPS = COV_THREADS / 32;
+    __shared__ double s_scr[WARPS * ReduceScratch<NACC>::PER_WARP];
+    __shared__ double s_red[WARPS][NACC];
+    __shared__ double s_tot[NACC];
+    __shared__ int s_nv[WARPS];
+    __shared__ int s_nvtot;
+    const int b = a.first + blockIdx.x, l = a.level, L = a.geom.L;
+    const int N = a.npts[(long long)b * L + l];
+    const unsigned ne = a.nedge_now[(long long)b * L + l];
+    double* out = a.cov + 36 * (long long)blockIdx.x * a.stride;
+    dvo_cov_info* inf = a.info ? a.info + (long long)blockIdx.x * a.stride : nullptr;
+    int status = 0, nvis = 0;
+    double sigma2 = 0.0, logdet = 0.0;
+    if (N > 0 && ne != 0u) {                              // block-uniform
+        PoseF P;
+        for (int k = 0; k < 9; ++k) P.R[k] = (float)a.pose[12 * (long long)b + k];
+        for (int k = 0; k < 3; ++k) P.T[k] = (float)a.pose[12 * (long long)b + 9 + k];
+        const long long base = lvl_at(a.geom, l, b);
+        const LevelCam cam = make_level_cam(a.K, a.geom, l);
+        TexSrc src;
+        src.tex = a.texel + base; src.tex8 = a.tex8 + tex_at(a.geom, l, b); src.d2 = a.d2 + base; src.lut = s_lut; src.scale = 0.f;
+        if (TEX) {
+            const unsigned mx2 = a.maxd2[(long long)b * L + l];
+            src.scale = dtn_scale(mx2, ne);
+            build_lut<COV_THREADS>(s_lut, mx2, src.scale);
+            __syncthreads();
+        }
+        double acc[NACC];
+#pragma unroll
+        for (int k = 0; k < NACC; ++k) acc[k] = 0.0;
+        int nv = 0;
+        accumulate_points<DVO_ARITH_EXACT, DVO_JAC_EXACT, true, COV_THREADS, false, RES, TEX, -1, true>(
+            a.X + base, a.Y + base, a.Z + base, N, P, cam, src, a.weight, a.huber_k, acc, nv, nullptr, nullptr, nullptr, nullptr, nullptr);
+        block_reduce<NACC, COV_THREADS>(acc, nv, s_scr, s_red, s_nv, s_tot, &s_nvtot);
+        if (threadIdx.x != 0) return;
+        nvis = s_nvtot;
+        if (nvis < 7) status |= 2;
+        else {
+            double* M = s_scr;                            // the reduction scratch is free again
+            int idx = 8;
+            for (int r = 0; r < 6; ++r) for (int c = r; c < 6; ++c) { M[6 * r + c] = s_tot[idx]; M[6 * c + r] = s_tot[idx]; ++idx; }
+            sigma2 = s_tot[NACC - 1] / (double)(nvis - 6);
+            double ldH = 0.0;
+            if (cov_from_normal_matrix(M, sigma2, out, &ldH)) logdet = 6.0 * log(sigma2) - ldH;
+            else status |= 4;
+        }
+    } else {
+        if (threadIdx.x != 0) return;
+        status = 1;
+    }
+    if (status) {
+        const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+        for (int k = 0; k < 36; ++k) out[k] = qnan;
+        sigma2 = qnan; logdet = qnan;
+    }
+    if (inf) { inf->status = status; inf->level = l; inf->nvis = nvis; inf->sigma2 = sigma2; inf->logdet = logdet; }
+}
+
 // ------------------------------------------------------------------ packed texels -> float images (parity inspection)
 // {DTn, gx, gy, w} of every pixel of one slot / level through exactly the code path the solver uses (packed texel or
 // escaped d2 stencil, lookup table or direct evaluation), so that dvo_get_level_buffer checks that path pixel by pixel.
@@ -862,11 +980,54 @@ __global__ void __launch_bounds__(256) resolve_texels_kernel(ResolveArgs a) {
     }
 }
 
+// Sigma_g = Ad(Tr^-1) Sigma_key Ad(Tr^-1)^T + Sigma_rel for tangent psi = (rho, omega) and T <- T exp(psi):
+// T_key exp(dk) Tr exp(dr) = T_key Tr exp(Ad(Tr^-1) dk) exp(dr), Ad(R, t) = [[R, [t]x R], [0, R]], Tr^-1 = (R^T, -R^T t).
+// Sigma_key == nullptr stands for a zero key-frame covariance.
+__device__ __forceinline__ void propagate_cov(const double* r, const double* __restrict__ Skey, const double* __restrict__ Srel, double* __restrict__ Sg) {
+    double A[36];
+    const double Rt[9] = {r[0], r[3], r[6], r[1], r[4], r[7], r[2], r[5], r[8]};
+    double u[3]; m3_vec(Rt, r + 9, u);
+    u[0] = -u[0]; u[1] = -u[1]; u[2] = -u[2];
+    const double ux[9] = {0, -u[2], u[1], u[2], 0, -u[0], -u[1], u[0], 0};
+    double UR[9]; m3_mul(ux, Rt, UR);
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+            A[6 * i + j] = Rt[3 * i + j]; A[6 * i + 3 + j] = UR[3 * i + j];
+            A[6 * (i + 3) + j] = 0.0; A[6 * (i + 3) + 3 + j] = Rt[3 * i + j];
+        }
+#pragma unroll
+    for (int i = 0; i < 6; ++i) {
+        double row[6];                                    // row i of A Sigma_key
+#pragma unroll
+        for (int q = 0; q < 6; ++q) {
+            double v = 0.0;
+            if (Skey) {
+#pragma unroll
+                for (int p = 0; p < 6; ++p) v += A[6 * i + p] * Skey[6 * p + q];
+            }
+            row[q] = v;
+        }
+#pragma unroll
+        for (int j = 0; j < 6; ++j) {
+            double v = 0.0;
+#pragma unroll
+            for (int q = 0; q < 6; ++q) v += row[q] * A[6 * j + q];
+            Sg[6 * i + j] = v + Srel[6 * i + j];
+        }
+    }
+}
+
 // ------------------------------------------------------------------ GOP composition (src/GOP.cpp:138-196)
-__global__ void gop_kernel(int nseq, int nframes, const int* __restrict__ kind, const double* __restrict__ rel, double* __restrict__ out) {
+// With rel_cov / glob_cov (both or neither) the covariance of every global pose is propagated alongside; the pose arithmetic is
+// the same instructions either way, so the composed poses do not depend on whether covariances are requested.
+__global__ void gop_kernel(int nseq, int nframes, const int* __restrict__ kind, const double* __restrict__ rel, double* __restrict__ out,
+                           const double* __restrict__ rel_cov, double* glob_cov) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= nseq) return;
     double kR[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, kT[3] = {0, 0, 0};
+    long long key = -1;                                                            // record holding Sigma_key (-1: zero)
     for (int f = 0; f < nframes; ++f) {
         const long long i = (long long)s * nframes + f;
         const double* r = rel + 12 * i;
@@ -878,7 +1039,11 @@ __global__ void gop_kernel(int nseq, int nframes, const int* __restrict__ kind, 
         for (int k = 0; k < 9; ++k) o[k] = gR[k];
         for (int k = 0; k < 3; ++k) { o[9 + k] = gT[k]; o[12 + k] = gT[k]; }
         rot_to_quat_dev(gR, o + 15);                                               // :103-114
-        if (kind[i] != 0) { for (int k = 0; k < 9; ++k) kR[k] = gR[k]; for (int k = 0; k < 3; ++k) kT[k] = gT[k]; }   // :184-185, :192-193
+        if (glob_cov) propagate_cov(r, key >= 0 ? glob_cov + 36 * key : nullptr, rel_cov + 36 * i, glob_cov + 36 * i);
+        if (kind[i] != 0) {                                                        // :184-185, :192-193
+            for (int k = 0; k < 9; ++k) kR[k] = gR[k]; for (int k = 0; k < 3; ++k) kT[k] = gT[k];
+            key = i;
+        }
     }
 }
 
@@ -1022,8 +1187,34 @@ int launch_resolve_texels(dvo_ctx* c, int slot, int level, float4* d_out) {
     return DVO_OK;
 }
 
-int launch_gop(dvo_ctx* c, int nseq, int nframes, const int* d_kind, const double* d_rel, double* d_out) {
-    gop_kernel<<<(nseq + 127) / 128, 128, 0, c->stream>>>(nseq, nframes, d_kind, d_rel, d_out);
+template <int RES, int TEX>
+static cudaError_t launch_cov_inst(dvo_ctx* c, const CovArgs& a, int count) {
+    if (TEX) {
+        const cudaError_t e = optin_lut_smem<CovArgs, cov_kernel<RES, TEX>>(c->cfg.device);
+        if (e != cudaSuccess) return e;
+    }
+    cov_kernel<RES, TEX><<<count, COV_THREADS, TEX ? LUT_BYTES : 0, c->stream>>>(a);
+    return cudaGetLastError();
+}
+
+int launch_cov(dvo_ctx* c, int first, int count, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info, long long stride) {
+    if (count == 0) return DVO_OK;
+    CovArgs a;
+    a.geom = c->geom; a.K = c->K; a.X = c->ptsX; a.Y = c->ptsY; a.Z = c->ptsZ; a.npts = c->npts; a.texel = c->texel;
+    a.tex8 = c->tex8; a.d2 = c->d2; a.maxd2 = c->maxd2; a.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L;
+    a.pose = c->pose; a.first = first; a.level = level; a.weight = p->weight; a.huber_k = p->huber_k;
+    a.cov = d_cov; a.info = d_info; a.stride = stride;
+    constexpr int F = DVO_RESIDUAL_DT_FLOOR, I = DVO_RESIDUAL_DT_INTERP;
+    cudaError_t e;
+    if (p->residual == I) e = c->texel_mode ? launch_cov_inst<I, 1>(c, a, count) : launch_cov_inst<I, 0>(c, a, count);
+    else e = c->texel_mode ? launch_cov_inst<F, 1>(c, a, count) : launch_cov_inst<F, 0>(c, a, count);
+    c->launches++;
+    DVO_CUDA(e);
+    return DVO_OK;
+}
+
+int launch_gop(dvo_ctx* c, int nseq, int nframes, const int* d_kind, const double* d_rel, double* d_out, const double* d_rel_cov, double* d_glob_cov) {
+    gop_kernel<<<(nseq + 127) / 128, 128, 0, c->stream>>>(nseq, nframes, d_kind, d_rel, d_out, d_rel_cov, d_glob_cov);
     c->launches++;
     DVO_CUDA(cudaGetLastError());
     return DVO_OK;
