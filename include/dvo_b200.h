@@ -177,7 +177,9 @@ int dvo_run_sequences(dvo_ctx* ctx, int nseq, int nframes, const uint8_t* gray, 
  * number of reprojected points of the finest level decide whether the PREVIOUS frame becomes the new reference (pose
  * reset, re-solve; :2192-2233).  The reference ships with the three quality gates commented out (:2129-2151) and only
  * the periodic rule (:2155-2160); use_quality_gates = 1 evaluates them as designed, in source order, OR-ed with the
- * periodic rule.  Reasons as the reference numbers them: 2 laplacian b, 3 visible ratio, 4 too few points, 5 periodic. */
+ * periodic rule.  Reasons as the reference numbers them: 2 laplacian b, 3 visible ratio, 4 too few points, 5 periodic.
+ * Reason 6 (not the reference's) is the entropy ratio of dvo_run_sequences_entropy.  The gates are evaluated in the order
+ * 2, 3, 4, 6, 5, and the last one that fires names the reason. */
 typedef struct dvo_keyframe_policy {
     int keyframe_every;           /* 5 (:2156); <= 0 disables the periodic rule                 */
     int use_quality_gates;        /* 0 = as shipped                                             */
@@ -239,6 +241,25 @@ int dvo_pose_covariance(dvo_ctx* ctx, int first, int count, const dvo_solver_par
 int dvo_run_sequences_cov(dvo_ctx* ctx, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem,
                           const dvo_solver_params* params, const dvo_keyframe_policy* policy, double* rel_poses, int* kind,
                           int* reason, double* global_poses, double* rel_cov, double* global_cov);
+
+/* dvo_run_sequences_cov plus the entropy-ratio key-frame rule of DVO-SLAM (Kerl, Sturm, Cremers, IROS 2013), decided per
+ * sequence on the device.
+ *   h(Sigma) = 3 (1 + ln 2 pi) + logdet(Sigma) / 2   (nats; logdet as dvo_cov_info.logdet)
+ *   h_ref    = h of the final covariance of frame lastRef + 1, the first frame solved against the current key frame
+ *              (NaN when that covariance is degenerate)
+ *   alpha_t  = h(Sigma_t) / h_ref, Sigma_t the covariance of frame t's first solve against the current key frame (finest level
+ *              with iterations; weight, huber_k and residual from params), evaluated where a switch is allowed (lastRef != t - 1).
+ * The gate fires (reason 6) iff alpha_t is finite, h_ref < 0 and alpha_t < entropy_ratio_thresh: with h_ref < 0, alpha < 1
+ * means "less certain than right after the key frame"; with h_ref >= 0 the ratio has no meaning and the gate stays silent.
+ * It combines with the policy's quality gates and periodic rule (order above).  entropy_ratio [nseq][nframes] receives the
+ * alpha each decision saw (for a switched frame: against the outgoing key frame), NaN where the gate was not evaluated
+ * (frame 0, frames t = lastRef + 1) or a covariance was degenerate.  entropy_ratio_thresh <= 0 disables the gate: the call
+ * is then dvo_run_sequences_cov exactly, and entropy_ratio is all NaN.  NaN is rejected.  reason, global_poses, rel_cov,
+ * global_cov and entropy_ratio may be NULL (the covariances are computed in any case). */
+int dvo_run_sequences_entropy(dvo_ctx* ctx, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem,
+                              const dvo_solver_params* params, const dvo_keyframe_policy* policy, double entropy_ratio_thresh,
+                              double* rel_poses, int* kind, int* reason, double* global_poses, double* rel_cov,
+                              double* global_cov, double* entropy_ratio);
 
 /* ---- inspection (parity tests; not on the hot path) ---- */
 int dvo_level_dims(dvo_ctx* ctx, int level, int* w, int* h);

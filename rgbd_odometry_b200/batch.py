@@ -206,6 +206,23 @@ class BatchAligner:
                                              _ptr(rel_cov), _ptr(glob_cov)), "dvo_run_sequences_cov")
         return rel, kind, reason, glob, rel_cov, glob_cov
 
+    def run_sequences_entropy(self, gray, depth, nseq, nframes, params, policy, entropy_ratio_thresh, device=False, want_global=True):
+        """dvo_run_sequences_entropy: run_sequences_cov with the entropy-ratio key-frame rule of DVO-SLAM added to `policy` (reason 6).
+        Returns run_sequences_cov's six records plus entropy_ratio (nseq, nframes): the ratio each decision saw, NaN where the gate
+        was not evaluated.  entropy_ratio_thresh <= 0 disables the gate (the result is then run_sequences_cov's)."""
+        rel = np.empty((nseq, nframes, 12), np.float64)
+        kind = np.empty((nseq, nframes), np.int32)
+        reason = np.empty((nseq, nframes), np.int32)
+        glob = np.empty((nseq, nframes, 19), np.float64) if want_global else None
+        rel_cov = np.empty((nseq, nframes, 6, 6), np.float64)
+        glob_cov = np.empty((nseq, nframes, 6, 6), np.float64) if want_global else None
+        ratio = np.empty((nseq, nframes), np.float64)
+        check(self.lib.dvo_run_sequences_entropy(self.h, nseq, nframes, _ptr(gray), _ptr(depth), MEM_DEVICE if device else MEM_HOST,
+                                                 C.byref(params), C.byref(policy), float(entropy_ratio_thresh), _ptr(rel), _ptr(kind),
+                                                 _ptr(reason), _ptr(glob), _ptr(rel_cov), _ptr(glob_cov), _ptr(ratio)),
+              "dvo_run_sequences_entropy")
+        return rel, kind, reason, glob, rel_cov, glob_cov, ratio
+
     def pose_covariance(self, count, params, first=0, level=-1):
         """6x6 covariance of the pose the last solve left in slots [first, first+count), evaluated on the resident frames
         (dvo_pose_covariance): returns (cov (count, 6, 6), info array of CovInfo).  level = -1: finest level with iterations."""

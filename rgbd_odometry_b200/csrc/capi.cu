@@ -170,7 +170,7 @@ int dvo_destroy(dvo_ctx* c) {
     cudaFree(c->gcol); cudaFree(c->d2); cudaFree(c->texel); cudaFree(c->tex8); cudaFree(c->ptsX); cudaFree(c->ptsY); cudaFree(c->ptsZ); cudaFree(c->ptsPix);
     cudaFree(c->npts); cudaFree(c->solve_order); cudaFree(c->seq_mask); cudaFree(c->seq_state); cudaFree(c->nedge); cudaFree(c->maxd2); cudaFree(c->pose0); cudaFree(c->pose); cudaFree(c->info);
     cudaFree(c->seq_rel); cudaFree(c->seq_kind); cudaFree(c->seq_reason); cudaFree(c->seq_glob); cudaFree(c->seq_cov); cudaFree(c->seq_gcov);
-    cudaFree(c->cov_buf); cudaFree(c->cov_info_buf);
+    cudaFree(c->seq_cov_info); cudaFree(c->seq_ent); cudaFree(c->cov_buf); cudaFree(c->cov_info_buf);
     for (int k = 0; k < 2; ++k) {
         cudaFree(c->seq_stage_g[k]); cudaFree(c->seq_stage_d[k]);
         if (c->seq_ev_ready[k]) cudaEventDestroy(c->seq_ev_ready[k]);
@@ -462,20 +462,33 @@ int dvo_align_batch(dvo_ctx* c, int count, const uint8_t* ref_gray, const uint16
 }  // extern "C"
 
 namespace {
+// h(Sigma) = 3 (1 + ln 2 pi) + logdet(Sigma) / 2: differential entropy of a 6-D Gaussian pose estimate, in nats
+__device__ __forceinline__ double pose_entropy(double logdet) { return 3.0 * (1.0 + log(2.0 * 3.14159265358979323846)) + 0.5 * logdet; }
+
+// cinfo (entropy gate on, else null): per-frame dvo_cov_info [nseq][nframes], frame t holding the covariance of its first solve;
+// frames before t hold their final covariance.  ent [nseq][nframes] receives the ratio at every frame the gate evaluates.
 __global__ void seq_gate_kernel(int nseq, int nframes, int t, dvo_keyframe_policy pol, int finest, const dvo_pair_info* __restrict__ info,
                                 const double* __restrict__ pose, double* __restrict__ pose0, int* __restrict__ lastRef,
-                                unsigned char* __restrict__ mask, double* __restrict__ rel, int* __restrict__ kind, int* __restrict__ reason) {
+                                unsigned char* __restrict__ mask, double* __restrict__ rel, int* __restrict__ kind, int* __restrict__ reason,
+                                const dvo_cov_info* __restrict__ cinfo, double ent_thr, double* __restrict__ ent) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= nseq) return;
     const dvo_pair_info& I = info[s];
+    const long long cur = (long long)s * nframes + t;
     int signal = 0, why = 0;
     if (pol.use_quality_gates) {                                                             // :2129-2151, in source order
         if (I.laplacian_b > pol.laplacian_thresh) { signal = 1; why = 2; }
         if (I.visible_ratio[finest] < pol.visible_ratio_thresh) { signal = 1; why = 3; }
         if (I.npts[finest] < pol.min_reprojections) { signal = 1; why = 4; }
     }
+    if (cinfo && lastRef[s] != t - 1) {                                                      // entropy ratio (DVO-SLAM, Kerl et al. 2013)
+        // h_ref: the final covariance of frame lastRef + 1, the first frame solved against the current key frame
+        const double h_ref = pose_entropy(cinfo[(long long)s * nframes + lastRef[s] + 1].logdet);
+        const double alpha = pose_entropy(cinfo[cur].logdet) / h_ref;                        // NaN when either covariance is degenerate
+        ent[cur] = alpha;
+        if (isfinite(alpha) && h_ref < 0.0 && alpha < ent_thr) { signal = 1; why = 6; }     // h_ref >= 0: the ratio means nothing
+    }
     if (pol.keyframe_every > 0 && (t - lastRef[s]) == pol.keyframe_every) { signal = 1; why = 5; }   // :2155-2160
-    const long long cur = (long long)s * nframes + t;
     if (signal && lastRef[s] != t - 1) {                                                     // :2192
         mask[s] = 1; lastRef[s] = t - 1;
         kind[cur - 1] = 2; reason[cur - 1] = why;                                            // gop.updateMostRecentToKeyFrame(reasonForChange)
@@ -517,16 +530,23 @@ __global__ void seq_init_kernel(int nseq, int nframes, double* __restrict__ pose
 // (:2210-2227), is skipped.  With the quality gates the decision depends on that solve, so it runs and every frame from t = 2
 // on is followed by the masked pass (its kernels return at once for unflagged slots).
 //
-// rel_cov / global_cov (optional, dvo_run_sequences_cov): after each frame's final solve one cov_kernel launch evaluates every
-// slot at its final relative pose, on the reference it was finally solved against, into the device record at frame t.
-int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem, const dvo_solver_params* p,
-                       const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses,
-                       double* rel_cov, double* global_cov) {
-    const char* who = rel_cov ? "dvo_run_sequences_cov" : "dvo_run_sequences";
+// Covariances (cov: dvo_run_sequences_cov / _entropy): after each frame's final solve one cov_kernel launch evaluates every slot at
+// its final relative pose, on the reference it was finally solved against, into the device record at frame t.
+//
+// Entropy gate (ent_thr > 0, dvo_run_sequences_entropy): the decision depends on the first solve's covariance, so the loop runs like
+// the quality-gate loop, and the covariance launch moves before the gate: first solve, cov_kernel over every slot (record and
+// dvo_cov_info of frame t), gate, masked switch pass, masked cov_kernel for the re-solved slots only.  The other slots' first-solve
+// records already are their final ones.
+int run_sequences_core(dvo_ctx* c, const char* who, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem,
+                       const dvo_solver_params* p, const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason,
+                       double* global_poses, bool cov, double* rel_cov, double* global_cov, double ent_thr = 0.0,
+                       double* entropy_ratio = nullptr) {
     if (c) { const int jr = join_aux(c); if (jr) return jr; }
-    if (!c || nseq < 1 || nseq > c->cfg.max_batch || nframes < 1 || !gray || !depth || !p || !pol || !rel_poses || !kind || (global_cov && !rel_cov)) {
+    if (!c || nseq < 1 || nseq > c->cfg.max_batch || nframes < 1 || !gray || !depth || !p || !pol || !rel_poses || !kind || (global_cov && !cov) ||
+        isnan(ent_thr)) {
         dvo_set_error("%s: bad argument", who); return DVO_ERR_ARG;
     }
+    const bool entropy_on = ent_thr > 0.0;
     if (!c->prev_gray) { dvo_set_error("%s: create the context with keep_now_depth = 1", who); return DVO_ERR_STATE; }
     if (!c->haveK) { dvo_set_error("%s: intrinsics not set", who); return DVO_ERR_STATE; }
     int finest = -1;
@@ -553,9 +573,14 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
         }
         if (rc == DVO_OK) c->seq_stage_slots = (size_t)nseq;
     }
-    if (rel_cov && c->seq_cov_n < n) {
-        cudaFree(c->seq_cov); c->seq_cov = nullptr; c->seq_cov_n = 0;
-        if (!fail(cudaMalloc((void**)&c->seq_cov, sizeof(double) * 36 * n))) c->seq_cov_n = n;
+    if (cov && c->seq_cov_n < n) {
+        cudaFree(c->seq_cov); cudaFree(c->seq_cov_info); c->seq_cov = nullptr; c->seq_cov_info = nullptr; c->seq_cov_n = 0;
+        fail(cudaMalloc((void**)&c->seq_cov, sizeof(double) * 36 * n)); fail(cudaMalloc((void**)&c->seq_cov_info, sizeof(dvo_cov_info) * n));
+        if (rc == DVO_OK) c->seq_cov_n = n;
+    }
+    if (entropy_on && c->seq_ent_n < n) {
+        cudaFree(c->seq_ent); c->seq_ent = nullptr; c->seq_ent_n = 0;
+        if (!fail(cudaMalloc((void**)&c->seq_ent, sizeof(double) * n))) c->seq_ent_n = n;
     }
     if (rc != DVO_OK) return rc;
     double* d_rel = c->seq_rel; int* d_kind = c->seq_kind; int* d_reason = c->seq_reason; double* d_glob = nullptr;
@@ -564,7 +589,8 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
     fail(cudaMemsetAsync(d_rel, 0, sizeof(double) * 12 * n, c->stream));
     fail(cudaMemsetAsync(d_kind, 0, sizeof(int) * n, c->stream));
     fail(cudaMemsetAsync(d_reason, 0, sizeof(int) * n, c->stream));
-    if (rel_cov) fail(cudaMemsetAsync(c->seq_cov, 0, sizeof(double) * 36 * n, c->stream));          // frame 0 anchors the chain: zeros
+    if (cov) fail(cudaMemsetAsync(c->seq_cov, 0, sizeof(double) * 36 * n, c->stream));              // frame 0 anchors the chain: zeros
+    if (entropy_on) fail(cudaMemsetAsync(c->seq_ent, 0xff, sizeof(double) * n, c->stream));      // all-ones: NaN where the gate is not evaluated
     if (host_in) { fail(cudaEventRecord(c->ev_entry, c->stream)); fail(cudaStreamWaitEvent(c->copy_stream, c->ev_entry, 0)); }
 
     // frame t of every sequence: host -> staging buffer t & 1 on the copy stream
@@ -617,12 +643,16 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
         if ((rc = dvo_build_pyramids(c, 0, nseq, 2))) break;
         if ((rc = dvo_prepare(c, 0, nseq, 2))) break;
         bool switch_pass = t >= 2, first_solve = true;                                       // a previous now frame exists from t = 2 on
-        if (!pol->use_quality_gates) {
+        if (!pol->use_quality_gates && !entropy_on) {
             switch_pass = t >= 2 && pol->keyframe_every > 0 && (t - host_last_ref) == pol->keyframe_every && host_last_ref != t - 1;
             if (switch_pass) { host_last_ref = t - 1; first_solve = false; }
         }
         if (first_solve && (rc = dvo_run(c, 0, nseq, p))) break;                             // warm start: pose0 holds the previous frame's pose (:1931-1932)
-        seq_gate_kernel<<<blk, 128, 0, c->stream>>>(nseq, nframes, t, *pol, finest, c->info, c->pose, c->pose0, c->seq_state, c->seq_mask, d_rel, d_kind, d_reason);
+        double* const cov_t = cov ? c->seq_cov + 36 * (size_t)t : nullptr;
+        dvo_cov_info* const cinfo_t = entropy_on ? c->seq_cov_info + t : nullptr;
+        if (entropy_on && (rc = launch_cov(c, 0, nseq, finest, p, cov_t, cinfo_t, nframes))) break;
+        seq_gate_kernel<<<blk, 128, 0, c->stream>>>(nseq, nframes, t, *pol, finest, c->info, c->pose, c->pose0, c->seq_state, c->seq_mask, d_rel, d_kind, d_reason,
+                                                    entropy_on ? c->seq_cov_info : nullptr, ent_thr, c->seq_ent);
         c->launches++;
         if (fail(cudaGetLastError())) break;
         if (switch_pass) {
@@ -631,6 +661,7 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
             if (rc == DVO_OK) rc = dvo_build_pyramids(c, 0, nseq, 1);
             if (rc == DVO_OK) rc = dvo_prepare(c, 0, nseq, 1);                               // computeDistTransfrmOfRef + preProcessRefFrame (:2197)
             if (rc == DVO_OK) rc = dvo_run(c, 0, nseq, p);                                   // re-run from identity (:2213-2220)
+            if (rc == DVO_OK && entropy_on) rc = launch_cov(c, 0, nseq, finest, p, cov_t, cinfo_t, nframes);
             c->active = nullptr;
             if (rc != DVO_OK) break;
             seq_finish_kernel<<<blk, 128, 0, c->stream>>>(nseq, nframes, t, c->seq_mask, c->pose, c->pose0, d_rel, d_kind, d_reason);
@@ -638,7 +669,7 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
             if (fail(cudaGetLastError())) break;
         }
         // c->pose of every slot is now frame t's final relative pose, and its frames are the pair it was finally solved on
-        if (rel_cov && (rc = launch_cov(c, 0, nseq, finest, p, c->seq_cov + 36 * (size_t)t, nullptr, nframes))) break;
+        if (cov && !entropy_on && (rc = launch_cov(c, 0, nseq, finest, p, cov_t, nullptr, nframes))) break;
     }
     c->active = nullptr;
     c->timing = timing;
@@ -663,6 +694,8 @@ int run_sequences_core(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, c
         fail(cudaMemcpyAsync(kind, d_kind, sizeof(int) * n, cudaMemcpyDeviceToHost, c->stream));
         if (reason) fail(cudaMemcpyAsync(reason, d_reason, sizeof(int) * n, cudaMemcpyDeviceToHost, c->stream));
         if (rel_cov) fail(cudaMemcpyAsync(rel_cov, c->seq_cov, sizeof(double) * 36 * n, cudaMemcpyDeviceToHost, c->stream));
+        if (entropy_ratio && entropy_on) fail(cudaMemcpyAsync(entropy_ratio, c->seq_ent, sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream));
+        if (entropy_ratio && !entropy_on) std::fill(entropy_ratio, entropy_ratio + n, (double)NAN);
     }
     cudaStreamSynchronize(c->copy_stream);
     if (cudaStreamSynchronize(c->stream) != cudaSuccess && rc == DVO_OK) { dvo_set_error("%s: %s", who, cudaGetErrorString(cudaGetLastError())); rc = DVO_ERR_CUDA; }
@@ -676,24 +709,35 @@ int dvo_run_sequences(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, co
                       int keyframe_every, double* rel_poses, int* kind, double* global_poses) {
     dvo_keyframe_policy pol; memset(&pol, 0, sizeof(pol));
     pol.keyframe_every = keyframe_every; pol.use_quality_gates = 0; pol.laplacian_thresh = 3.0f; pol.visible_ratio_thresh = 0.8f; pol.min_reprojections = 50;
-    return run_sequences_core(c, nseq, nframes, gray, depth, DVO_MEM_HOST, p, &pol, rel_poses, kind, nullptr, global_poses, nullptr, nullptr);
+    return run_sequences_core(c, "dvo_run_sequences", nseq, nframes, gray, depth, DVO_MEM_HOST, p, &pol, rel_poses, kind, nullptr, global_poses, false,
+                              nullptr, nullptr);
 }
 
 int dvo_run_sequences_gated(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, const dvo_solver_params* p,
                             const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses) {
-    return run_sequences_core(c, nseq, nframes, gray, depth, DVO_MEM_HOST, p, pol, rel_poses, kind, reason, global_poses, nullptr, nullptr);
+    return run_sequences_core(c, "dvo_run_sequences", nseq, nframes, gray, depth, DVO_MEM_HOST, p, pol, rel_poses, kind, reason, global_poses, false,
+                              nullptr, nullptr);
 }
 
 int dvo_run_sequences_mem(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem, const dvo_solver_params* p,
                           const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses) {
-    return run_sequences_core(c, nseq, nframes, gray, depth, mem, p, pol, rel_poses, kind, reason, global_poses, nullptr, nullptr);
+    return run_sequences_core(c, "dvo_run_sequences", nseq, nframes, gray, depth, mem, p, pol, rel_poses, kind, reason, global_poses, false, nullptr,
+                              nullptr);
 }
 
 int dvo_run_sequences_cov(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem, const dvo_solver_params* p,
                           const dvo_keyframe_policy* pol, double* rel_poses, int* kind, int* reason, double* global_poses, double* rel_cov,
                           double* global_cov) {
     if (!rel_cov) { dvo_set_error("dvo_run_sequences_cov: rel_cov is required"); return DVO_ERR_ARG; }
-    return run_sequences_core(c, nseq, nframes, gray, depth, mem, p, pol, rel_poses, kind, reason, global_poses, rel_cov, global_cov);
+    return run_sequences_core(c, "dvo_run_sequences_cov", nseq, nframes, gray, depth, mem, p, pol, rel_poses, kind, reason, global_poses, true,
+                              rel_cov, global_cov);
+}
+
+int dvo_run_sequences_entropy(dvo_ctx* c, int nseq, int nframes, const uint8_t* gray, const uint16_t* depth, int mem, const dvo_solver_params* p,
+                              const dvo_keyframe_policy* pol, double entropy_ratio_thresh, double* rel_poses, int* kind, int* reason,
+                              double* global_poses, double* rel_cov, double* global_cov, double* entropy_ratio) {
+    return run_sequences_core(c, "dvo_run_sequences_entropy", nseq, nframes, gray, depth, mem, p, pol, rel_poses, kind, reason, global_poses, true,
+                              rel_cov, global_cov, entropy_ratio_thresh, entropy_ratio);
 }
 
 int dvo_pose_covariance(dvo_ctx* c, int first, int count, const dvo_solver_params* p, int level, double* cov36, dvo_cov_info* info, int mem) {

@@ -68,6 +68,8 @@ struct dvo_ctx {
     cudaEvent_t seq_ev_ready[2], seq_ev_free[2];
     double* seq_rel; int* seq_kind; int* seq_reason; double* seq_glob; size_t seq_rec_n, seq_glob_n;
     double* seq_cov; double* seq_gcov; size_t seq_cov_n, seq_gcov_n;   // per-frame relative / global covariances (dvo_run_sequences_cov)
+    dvo_cov_info* seq_cov_info;    // per-frame dvo_cov_info of seq_cov (same size); written by the entropy key-frame gate only
+    double* seq_ent; size_t seq_ent_n;   // per-frame entropy ratio the gate saw (dvo_run_sequences_entropy)
     // device results of dvo_pose_covariance with host outputs, grown on demand
     double* cov_buf; dvo_cov_info* cov_info_buf; size_t cov_cap;
     int sm_count;
@@ -147,7 +149,8 @@ int launch_resolve_texels(dvo_ctx* c, int slot, int level, float4* d_out);
 int launch_solve(dvo_ctx* c, int first, int count, const dvo_solver_params* p);
 int launch_eval(dvo_ctx* c, int slot, int level, const double* d_pose12, int jac, int weight, int arith, float huber_k, int residual,
                 double* d_out /* 6 + 36 + 1 + 1 doubles */, float* d_eps, float* d_w, float* d_u, float* d_v, float* d_J);
-// 6x6 pose covariance of slots [first, first+count) at their current pose (c->pose); record k at d_cov + 36 * k * stride
+// 6x6 pose covariance of slots [first, first+count) at their current pose (c->pose); record k at d_cov + 36 * k * stride.
+// With c->active set, slots whose flag is 0 are skipped and keep their records.
 int launch_cov(dvo_ctx* c, int first, int count, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info, long long stride);
 // d_rel_cov / d_glob_cov: both null, or [nseq][nframes][36] covariances to propagate along the key-frame chain
 int launch_gop(dvo_ctx* c, int nseq, int nframes, const int* d_kind, const double* d_rel, double* d_out, const double* d_rel_cov, double* d_glob_cov);

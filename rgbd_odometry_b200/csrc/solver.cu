@@ -856,6 +856,7 @@ struct CovArgs {
     double* cov;            // 36 doubles per slot, record of CTA k at cov + 36 * k * stride
     dvo_cov_info* info;     // optional, same indexing
     long long stride;
+    const unsigned char* active;   // optional per-slot mask: a slot whose flag is 0 keeps its record as it is
 };
 
 // Serial tail on thread 0: H (full symmetric, row-major, in shared memory M[0..35]) -> Sigma = s2 H^-1 into out, log det H.
@@ -906,6 +907,7 @@ __global__ void __launch_bounds__(COV_THREADS) cov_kernel(CovArgs a) {
     __shared__ int s_nv[WARPS];
     __shared__ int s_nvtot;
     const int b = a.first + blockIdx.x, l = a.level, L = a.geom.L;
+    if (a.active && !a.active[b]) return;                 // masked pass (key-frame switch): the slot's record stays as it is
     const int N = a.npts[(long long)b * L + l];
     const unsigned ne = a.nedge_now[(long long)b * L + l];
     double* out = a.cov + 36 * (long long)blockIdx.x * a.stride;
@@ -1203,7 +1205,7 @@ int launch_cov(dvo_ctx* c, int first, int count, int level, const dvo_solver_par
     a.geom = c->geom; a.K = c->K; a.X = c->ptsX; a.Y = c->ptsY; a.Z = c->ptsZ; a.npts = c->npts; a.texel = c->texel;
     a.tex8 = c->tex8; a.d2 = c->d2; a.maxd2 = c->maxd2; a.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L;
     a.pose = c->pose; a.first = first; a.level = level; a.weight = p->weight; a.huber_k = p->huber_k;
-    a.cov = d_cov; a.info = d_info; a.stride = stride;
+    a.cov = d_cov; a.info = d_info; a.stride = stride; a.active = c->active;
     constexpr int F = DVO_RESIDUAL_DT_FLOOR, I = DVO_RESIDUAL_DT_INTERP;
     cudaError_t e;
     if (p->residual == I) e = c->texel_mode ? launch_cov_inst<I, 1>(c, a, count) : launch_cov_inst<I, 0>(c, a, count);

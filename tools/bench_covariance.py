@@ -3,7 +3,12 @@
   config 2  1024 pairs 640x480x4, GN 10 it/level: a dvo_process step with and without a following dvo_pose_covariance (device
             output), alternated in one run, plus the covariance pass alone on the solved batch;
   config 4  148 sequences x 8 frames of 1280x720, 5 levels, SUBGRAD_REF 50 it/level: dvo_run_sequences_mem against
-            dvo_run_sequences_cov (device-resident inputs), alternated.
+            dvo_run_sequences_cov (device-resident inputs), alternated;
+  entropy   the same config 4 workload: dvo_run_sequences_cov, dvo_run_sequences_entropy with the gate disabled and with a
+            threshold at which some sequences switch (the median of the ratios an enabled, never-firing gate reports),
+            alternated.
+
+--configs picks the arms (default: 2,4).
 
 CUDA events on the context's stream, warm-up first.  The card name and power limit are read in the same run.  Writes one JSON
 file (--out) and prints it.  Needs a CUDA device.
@@ -129,6 +134,45 @@ def config4(args, stream):
             "run_ms_rounds": plain, "run_cov_ms_rounds": withcov, "records_bit_identical": bool(same)}
 
 
+def entropy(args, stream):
+    W, H, L, K = 1280, 720, 5, O.K1280
+    nseq, nframes = args.sequences, args.seq_frames
+    with ThreadPoolExecutor(os.cpu_count() or 1) as ex:
+        seqs = list(ex.map(lambda s: O.synth_sequence(700000 + s, nframes, W, H, K, max_angle_deg=0.4, max_trans_m=0.008), range(nseq)))
+    gray = torch.from_numpy(np.stack([s[0] for s in seqs])).cuda()
+    depth = torch.from_numpy(np.stack([s[1] for s in seqs]).view(np.int16)).cuda()
+    al = dvo.BatchAligner(W, H, L, max_batch=nseq, keep_now_depth=True, intrinsics=K)
+    al.set_stream(stream.cuda_stream)
+    prm = dvo.solver_params(iters=(50,) * L)
+    pol = dvo.keyframe_policy()
+    ent = lambda thr: al.run_sequences_entropy(gray.data_ptr(), depth.data_ptr(), nseq, nframes, prm, pol, thr, device=True)
+    probe = ent(1e-300)                                              # enabled, never fires: the ratios of the shipped schedule
+    thr = float(np.median(probe[6][np.isfinite(probe[6])]))
+    run_cov = lambda: al.run_sequences_cov(gray.data_ptr(), depth.data_ptr(), nseq, nframes, prm, pol, device=True)
+    run_off = lambda: ent(0.0)
+    run_on = lambda: ent(thr)
+    a, b, c = run_cov(), run_off(), run_on()
+    off_same = all(np.array_equal(x.view(np.uint8), y.view(np.uint8)) for x, y in zip(a, b[:6])) and bool(np.isnan(b[6]).all())
+    kind, reason = c[1], c[2]
+    n0 = al.launch_count(); run_cov(); n1 = al.launch_count(); run_off(); n2 = al.launch_count(); run_on(); n3 = al.launch_count()
+    t_cov, t_off, t_on = [], [], []
+    for _ in range(args.rounds):                                     # alternated: cov, off, on, cov, off, on, ...
+        t_cov.append(timed(stream, run_cov, 1))
+        t_off.append(timed(stream, run_off, 1))
+        t_on.append(timed(stream, run_on, 1))
+    al.close()
+    med = lambda v: float(np.median(v))
+    return {"workload": f"{nseq} synthetic sequences x {nframes} frames 1280x720, 5 levels, SUBGRAD_REF 50 it/level, key frame every 5, "
+                        "device-resident inputs", "entropy_ratio_thresh": thr,
+            "sequences_switched_by_entropy": int(((kind == 2) & (reason == 6)).any(axis=1).sum()),
+            "entropy_switches": int(((kind == 2) & (reason == 6)).sum()), "periodic_switches": int(((kind == 2) & (reason == 5)).sum()),
+            "run_cov_ms_median": med(t_cov), "run_entropy_off_ms_median": med(t_off), "run_entropy_on_ms_median": med(t_on),
+            "entropy_on_overhead_ms": med(t_on) - med(t_cov), "entropy_on_overhead_frac": (med(t_on) - med(t_cov)) / med(t_cov),
+            "launches_cov": n1 - n0, "launches_entropy_off": n2 - n1, "launches_entropy_on": n3 - n2,
+            "run_cov_ms_rounds": t_cov, "run_entropy_off_ms_rounds": t_off, "run_entropy_on_ms_rounds": t_on,
+            "disabled_records_bit_identical_to_cov": bool(off_same)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--pairs", type=int, default=1024)
@@ -137,6 +181,7 @@ def main():
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--sequences", type=int, default=148)
     ap.add_argument("--seq-frames", type=int, default=8)
+    ap.add_argument("--configs", default="2,4", help="comma-separated arms: 2, 4, entropy")
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_bench_covariance.json"))
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -144,7 +189,11 @@ def main():
     stream = torch.cuda.Stream()
     torch.cuda.set_stream(stream)
     t0 = time.time()
-    res = {"card": card(), "config2": config2(args, stream), "config4": config4(args, stream), "seconds": None}
+    arms = {"2": ("config2", config2), "4": ("config4", config4), "entropy": ("entropy", entropy)}
+    res = {"card": card()}
+    for a in args.configs.split(","):
+        name, fn = arms[a.strip()]
+        res[name] = fn(args, stream)
     res["seconds"] = time.time() - t0
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
