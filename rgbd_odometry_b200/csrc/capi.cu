@@ -84,7 +84,6 @@ int dvo_create(const dvo_config* cfg, dvo_ctx** out) {
     }
     if (cfg->device < 0 || cfg->device >= ndev) { dvo_set_error("dvo_create: device %d out of range (%d devices)", cfg->device, ndev); return DVO_ERR_ARG; }
     DVO_CUDA(cudaSetDevice(cfg->device));
-    if (const char* e = getenv("DVO_L2_FETCH")) { cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(e)); cudaGetLastError(); }   // experiment knob
     dvo_ctx* c = new (std::nothrow) dvo_ctx();
     if (!c) return DVO_ERR_NOMEM;
     memset(c, 0, sizeof(*c));
@@ -110,11 +109,6 @@ int dvo_create(const dvo_config* cfg, dvo_ctx** out) {
     c->sm_count = prop.multiProcessorCount;
     c->smem_optin = prop.sharedMemPerBlockOptin;
     c->solve_shape = (cfg->max_batch <= c->sm_count) ? 512 : 256;
-    if (const char* e = getenv("DVO_SOLVE_SHAPE")) { const int v = atoi(e); if (v == 256 || v == 512) c->solve_shape = v; }   // experiment knob
-    c->texel_mode = 1;
-    c->edt_band = 0;
-    if (const char* e = getenv("DVO_EDT_BAND")) c->edt_band = atoi(e);                                                       // experiment knob
-    if (const char* e = getenv("DVO_TEXEL_MODE")) c->texel_mode = atoi(e) ? 1 : 0;                                           // experiment knob (A/B)
     CREATE_CUDA(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
     c->stream = c->own_stream;
     CREATE_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
@@ -126,8 +120,6 @@ int dvo_create(const dvo_config* cfg, dvo_ctx** out) {
         CREATE_CUDA(cudaEventCreateWithFlags(&c->ev_aux_done[k], cudaEventDisableTiming));
     }
     CREATE_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
-    c->e2e_chunk = 128;      // 8 pipeline stages per 1024 pairs: 25.7 ms per pass against 27.2 (256), 30.2 (512), 33.3 (64)
-    if (const char* e = getenv("DVO_E2E_CHUNK")) { const int v = atoi(e); if (v > 0) c->e2e_chunk = v; }
     CREATE_CUDA(cudaEventCreate(&c->ev_a));
     CREATE_CUDA(cudaEventCreate(&c->ev_b));
 
@@ -139,7 +131,7 @@ int dvo_create(const dvo_config* cfg, dvo_ctx** out) {
     if (cfg->keep_now_depth) { A(dalloc(&c->depth[1], T)); A(dalloc(&c->prev_gray, B * (size_t)g.P[0])); A(dalloc(&c->prev_depth, B * (size_t)g.P[0])); }
     c->now_valid = (unsigned char*)calloc(B, 1); c->prev_valid = (unsigned char*)calloc(B, 1);
     A(dalloc(&c->gcol, T)); A(dalloc(&c->d2, T));
-    if (c->texel_mode) A(dalloc(&c->tex8, (size_t)g.total_t)); else A(dalloc(&c->texel, T));
+    A(dalloc(&c->tex8, (size_t)g.total_t));
     A(dalloc(&c->ptsX, T)); A(dalloc(&c->ptsY, T)); A(dalloc(&c->ptsZ, T)); A(dalloc(&c->ptsPix, T));
     A(dalloc(&c->npts, B * g.L)); A(dalloc(&c->solve_order, B)); A(dalloc(&c->seq_mask, B)); A(dalloc(&c->seq_state, B)); A(dalloc(&c->nedge, 2 * B * g.L)); A(dalloc(&c->maxd2, B * g.L));
     A(dalloc(&c->pose0, B * 12)); A(dalloc(&c->pose, B * 12)); A(dalloc(&c->info, B));
@@ -167,7 +159,7 @@ int dvo_destroy(dvo_ctx* c) {
     cudaSetDevice(c->cfg.device);
     if (c->own_stream) cudaStreamSynchronize(c->own_stream);
     for (int f = 0; f < 2; ++f) { cudaFree(c->gray[f]); cudaFree(c->depth[f]); cudaFree(c->edge[f]); }
-    cudaFree(c->gcol); cudaFree(c->d2); cudaFree(c->texel); cudaFree(c->tex8); cudaFree(c->ptsX); cudaFree(c->ptsY); cudaFree(c->ptsZ); cudaFree(c->ptsPix);
+    cudaFree(c->gcol); cudaFree(c->d2); cudaFree(c->tex8); cudaFree(c->ptsX); cudaFree(c->ptsY); cudaFree(c->ptsZ); cudaFree(c->ptsPix);
     cudaFree(c->npts); cudaFree(c->solve_order); cudaFree(c->seq_mask); cudaFree(c->seq_state); cudaFree(c->nedge); cudaFree(c->maxd2); cudaFree(c->pose0); cudaFree(c->pose); cudaFree(c->info);
     cudaFree(c->seq_rel); cudaFree(c->seq_kind); cudaFree(c->seq_reason); cudaFree(c->seq_glob); cudaFree(c->seq_cov); cudaFree(c->seq_gcov);
     cudaFree(c->seq_cov_info); cudaFree(c->seq_ent); cudaFree(c->cov_buf); cudaFree(c->cov_info_buf);
@@ -299,13 +291,8 @@ int dvo_prepare(dvo_ctx* c, int first, int count, int frames_mask) {
     if (count == 0) return DVO_OK;
     int rc;
     { StageTimer t(c, DVO_STAGE_CANNY); rc = launch_canny(c, first, count, frames_mask); if (rc) return rc; }
-    if (frames_mask & 2) {
-        if (c->texel_mode && c->edt_band >= 0) {       // fused: the stage slot of the row pass times both
-            StageTimer t(c, DVO_STAGE_EDT_ROWS); rc = launch_edt_pack(c, first, count); if (rc) return rc;
-        } else {
-            { StageTimer t(c, DVO_STAGE_EDT_ROWS); rc = launch_edt_rows(c, first, count); if (rc) return rc; }
-            { StageTimer t(c, DVO_STAGE_NORMGRAD); rc = c->texel_mode ? launch_pack(c, first, count) : launch_normgrad(c, first, count); if (rc) return rc; }
-        }
+    if (frames_mask & 2) {       // EDT rows + texels: the stage slot of the row pass times both (DVO_STAGE_NORMGRAD stays 0)
+        StageTimer t(c, DVO_STAGE_EDT_ROWS); rc = launch_edt_pack(c, first, count); if (rc) return rc;
     }
     return DVO_OK;
 }
@@ -335,16 +322,12 @@ int dvo_run(dvo_ctx* c, int first, int count, const dvo_solver_params* p) {
     return launch_solve(c, first, count, p);
 }
 
-// pyramids + Canny / EDT / normalise + solve of one slot range on the CURRENT c->stream, no stage timers, no join
+// pyramids + Canny / EDT + texels + solve of one slot range on the CURRENT c->stream, no stage timers, no join
 static int process_range(dvo_ctx* c, int first, int count, const dvo_solver_params* p, cudaEvent_t pre_done) {
     int rc;
     if ((rc = launch_pyramid(c, first, count, 3))) return rc;
     if ((rc = launch_canny(c, first, count, 3))) return rc;
-    if (c->texel_mode && c->edt_band >= 0) { if ((rc = launch_edt_pack(c, first, count))) return rc; }
-    else {
-        if ((rc = launch_edt_rows(c, first, count))) return rc;
-        if ((rc = c->texel_mode ? launch_pack(c, first, count) : launch_normgrad(c, first, count))) return rc;
-    }
+    if ((rc = launch_edt_pack(c, first, count))) return rc;
     if (pre_done) DVO_CUDA(cudaEventRecord(pre_done, c->stream));
     return launch_solve(c, first, count, p);
 }
@@ -413,6 +396,10 @@ int dvo_get_poses(dvo_ctx* c, int first, int count, double* R9T3, dvo_pair_info*
     return DVO_OK;
 }
 
+// frame pairs per upload/compute pipeline stage in dvo_align_batch: 8 stages per 1024 pairs, 25.7 ms per pass against
+// 27.2 (256), 30.2 (512), 33.3 (64)
+constexpr int E2E_CHUNK = 128;
+
 int dvo_align_batch(dvo_ctx* c, int count, const uint8_t* ref_gray, const uint16_t* ref_depth, const uint8_t* now_gray,
                     const uint16_t* now_depth, const dvo_solver_params* p, double* R9T3, dvo_pair_info* info) {
     if (c) { const int jr = join_aux(c); if (jr) return jr; }
@@ -431,7 +418,7 @@ int dvo_align_batch(dvo_ctx* c, int count, const uint8_t* ref_gray, const uint16
         cudaError_t e = cudaEventRecord(c->ev_entry, c->stream);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(c->copy_stream, c->ev_entry, 0);
         if (e != cudaSuccess) { dvo_set_error("dvo_align_batch: %s", cudaGetErrorString(e)); rc = DVO_ERR_CUDA; break; }
-        int nchunks = (n + c->e2e_chunk - 1) / c->e2e_chunk;
+        int nchunks = (n + E2E_CHUNK - 1) / E2E_CHUNK;
         if (nchunks > 16) nchunks = 16;
         const int chunk = (n + nchunks - 1) / nchunks;
         int k = 0;
@@ -783,12 +770,12 @@ int dvo_get_level_buffer(dvo_ctx* c, int slot, int frame, int level, int which, 
         case DVO_BUF_GRAY: src = c->gray[frame] + o; es = 1; break;
         case DVO_BUF_DEPTH: if (!c->depth[frame]) { dvo_set_error("depth not stored for this frame"); return DVO_ERR_STATE; } src = c->depth[frame] + o; es = 2; break;
         case DVO_BUF_EDGE: src = c->edge[frame] + o; es = 1; break;
-        case DVO_BUF_D2: if (frame != DVO_FRAME_NOW) { dvo_set_error("d2 exists for the now frame only"); return DVO_ERR_ARG; } src = c->d2 + o; es = 4; break;
+        case DVO_BUF_D2: if (frame != DVO_FRAME_NOW) { dvo_set_error("d2 exists for the now frame only"); return DVO_ERR_ARG; } break;
         case DVO_BUF_DTN: case DVO_BUF_GX: case DVO_BUF_GY:
-            if (frame != DVO_FRAME_NOW) { dvo_set_error("DT exists for the now frame only"); return DVO_ERR_ARG; } src = c->texel ? c->texel + o : nullptr; es = 16; break;
+            if (frame != DVO_FRAME_NOW) { dvo_set_error("DT exists for the now frame only"); return DVO_ERR_ARG; } break;
         default: dvo_set_error("dvo_get_level_buffer: unknown buffer %d", which); return DVO_ERR_ARG;
     }
-    if (which == DVO_BUF_D2 && c->texel_mode && c->edt_band >= 0) {      // fused EDT + texel kernel: the 32-bit image is sparse, rebuild the dense one
+    if (which == DVO_BUF_D2) {      // the fused EDT + texel kernel leaves the 32-bit image sparse: rebuild the dense one from the texels
         if (bytes < P * 4) { dvo_set_error("dvo_get_level_buffer: destination too small"); return DVO_ERR_ARG; }
         int32_t* d_tmp = nullptr;
         DVO_CUDA(cudaMalloc((void**)&d_tmp, P * 4));
@@ -800,17 +787,14 @@ int dvo_get_level_buffer(dvo_ctx* c, int slot, int frame, int level, int which, 
         DVO_CUDA(ce);
         return DVO_OK;
     }
-    if (which >= DVO_BUF_DTN) {
+    if (which >= DVO_BUF_DTN) {      // no float images are kept: evaluate them from the packed texels for this slot / level on demand
         if (bytes < P * 4) { dvo_set_error("dvo_get_level_buffer: destination too small"); return DVO_ERR_ARG; }
         std::vector<float> tmp(P * 4);
         float4* d_tmp = nullptr;
-        if (!src) {      // packed-texel contexts keep no float images: evaluate them for this slot / level on demand
-            DVO_CUDA(cudaMalloc((void**)&d_tmp, P * 16));
-            const int rc = c->texel_mode ? launch_resolve_texels(c, slot, level, d_tmp) : launch_normgrad_into(c, slot, level, d_tmp);
-            if (rc) { cudaFree(d_tmp); return rc; }
-            src = d_tmp;
-        }
-        cudaError_t ce = cudaMemcpyAsync(tmp.data(), src, P * 16, cudaMemcpyDeviceToHost, c->stream);
+        DVO_CUDA(cudaMalloc((void**)&d_tmp, P * 16));
+        const int rc = launch_resolve_texels(c, slot, level, d_tmp);
+        if (rc) { cudaFree(d_tmp); return rc; }
+        cudaError_t ce = cudaMemcpyAsync(tmp.data(), d_tmp, P * 16, cudaMemcpyDeviceToHost, c->stream);
         if (ce == cudaSuccess) ce = cudaStreamSynchronize(c->stream);
         cudaFree(d_tmp);
         DVO_CUDA(ce);

@@ -61,7 +61,6 @@ struct dvo_ctx {
     cudaEvent_t ev_fork, ev_pre[2], ev_aux_done[2];
     bool aux_pending;               // work is in flight on aux[] that the context stream has not joined yet
     int proc_first, proc_count;     // slot range of the dvo_process call that left that work in flight
-    int e2e_chunk;           // frame pairs per upload/compute pipeline stage in dvo_align_batch
     // sequence mode (run_sequences_core): staging for the pipelined uploads and the device record of a run, kept across calls
     // (cudaMalloc / cudaFree of ~0.8 GB per call made the end-to-end sequence rate vary 8x between runs)
     uint8_t* seq_stage_g[2]; uint16_t* seq_stage_d[2]; size_t seq_stage_slots;
@@ -85,10 +84,7 @@ struct dvo_ctx {
     uint8_t* edge[2];        // [frame] Canny edge maps 0/255
     uint16_t* gcol;          // now: EDT phase-1 column distances
     int32_t* d2;             // now: exact squared distance
-    float4* texel;           // now: {DTn, gx, gy, getWeightOf(DTn)} -- legacy 16-byte texels (texel_mode 0 only)
-    uint2* tex8;             // now: packed 8-byte texels (texel_mode 1, the default)
-    int edt_band;            // experiment knob: band height of the fused EDT + texel kernel (0 = automatic); -1 = unfused kernels
-    int texel_mode;          // 1: packed texels + in-kernel lookup tables; 0: legacy float4 texels written by normgrad_kernel
+    uint2* tex8;             // now: packed 8-byte texels
     float *ptsX, *ptsY, *ptsZ;   // ref: back-projected edge points (row-major pixel order), capacity P[l] per slot and level
     int* ptsPix;                 // ref: pixel index y*w+x of every point (restores the reference's column-major order)
     int* npts;               // [Bmax][L]
@@ -137,14 +133,12 @@ void dvo_set_error(const char* fmt, ...);
 int launch_pyramid(dvo_ctx* c, int first, int count, int frames_mask);
 int launch_canny(dvo_ctx* c, int first, int count, int frames_mask);
 void canny_scratch_layout(const PyrGeom& g, long long* bm_off, int* bm_words, size_t* words_per_image);
-int launch_edt_rows(dvo_ctx* c, int first, int count);
-int launch_normgrad(dvo_ctx* c, int first, int count);
-int launch_pack(dvo_ctx* c, int first, int count);
+// EDT row pass + packed texels of the now frame (fused up to 800 pixels wide, the row kernels + pack_texel_kernel above that)
 int launch_edt_pack(dvo_ctx* c, int first, int count);
-int launch_d2_from_texels(dvo_ctx* c, int slot, int level, int32_t* d_out);      // EDT rows + packed texels fused (texel_mode 1)
-// inspection: {DTn, gx, gy, w} of one slot / level into a caller-provided device buffer of P[level] float4
-int launch_normgrad_into(dvo_ctx* c, int slot, int level, float4* d_out);
-// same images, resolved from the packed texels through the solver's own lookup path (texel_mode 1)
+// inspection: the dense d2 image of one slot / level into a caller-provided device buffer of P[level] int32
+int launch_d2_from_texels(dvo_ctx* c, int slot, int level, int32_t* d_out);
+// inspection: {DTn, gx, gy, w} of one slot / level into a caller-provided device buffer of P[level] float4, resolved from the
+// packed texels through the solver's own lookup path
 int launch_resolve_texels(dvo_ctx* c, int slot, int level, float4* d_out);
 int launch_solve(dvo_ctx* c, int first, int count, const dvo_solver_params* p);
 int launch_eval(dvo_ctx* c, int slot, int level, const double* d_pose12, int jac, int weight, int arith, float huber_k, int residual,

@@ -1,4 +1,4 @@
-"""Quick solve-stage timing at the bench workload (1024 pairs) for the current DVO_SOLVE_THREADS."""
+"""Quick solve-stage timing at the bench workload (1024 pairs, or the batch size given as the first argument)."""
 import sys, os
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -20,4 +20,4 @@ out = []
 for name, solver, it in (("gn10", dvo.GN, 10), ("subgrad50", dvo.SUBGRAD_REF, 50), ("gn10_L3only", dvo.GN, -1)):
     iters = (it,) * 4 if it > 0 else (0, 0, 0, 50)
     out.append(f"{name}={timed(dvo.solver_params(solver=solver, iters=iters)):.3f}ms")
-print(os.environ.get("DVO_SOLVE_THREADS", "256"), " ".join(out))
+print(B, " ".join(out))
