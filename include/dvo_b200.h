@@ -91,7 +91,8 @@ typedef struct dvo_solver_params {
 /* per pair result record (what runIterations returns besides the pose, src/SolveDVO.cpp:997-1005, plus the
  * quiet-path residual statistic of processResidueHistogram :1398-1483) */
 typedef struct dvo_pair_info {
-    int status;                          /* 0 ok; bit0: a level had no reference points or no now edges   */
+    int status;                          /* 0 ok; bit0: a level had no reference points or no now edges;
+                                            bit1: slot index out of range (dvo_align_pairs with device indices) */
     int npts[DVO_MAX_LEVELS];            /* selected reference edge points per level                      */
     int best_index[DVO_MAX_LEVELS];      /* bestEnergyIndex per level                                     */
     int iterations_run[DVO_MAX_LEVELS];  /* iterations actually executed per level                        */
@@ -231,6 +232,25 @@ typedef struct dvo_cov_info {
  * After dvo_align_batch with count > max_batch only the last chunk's frames and poses are resident. */
 int dvo_pose_covariance(dvo_ctx* ctx, int first, int count, const dvo_solver_params* params, int level,
                         double* cov36, dvo_cov_info* info, int mem);
+
+/* Align npairs (reference, now) pairs of frames that are already prepared in this context. Pair k solves the REFERENCE-frame
+ * data of slot ref_slot[k] (edge points, npts) against the NOW-frame data of slot now_slot[k] (texels, d2, max d2, edge counts).
+ * Both slots must lie in [0, max_batch). A frame serves in both roles once it has been loaded into both roles of a slot
+ * (dvo_set_frames REF and NOW with the same images) and built and prepared with frames_mask = 3. npairs may exceed max_batch.
+ * pose0: npairs x 12 initial poses (NULL = identity). poses: npairs x 12. info: optional. cov36 / cov_info: optional, the
+ * dvo_pose_covariance of each pair at its returned pose (level -1 rule as there). mem applies to every array argument.
+ * The slots' own pose, info, energies and trace are not touched.
+ *   - One solve launch over all pairs with the kernel configuration dvo_run would choose for these params on this context
+ *     (same thread count per pair), so a pair's pose and info equal what dvo_run gives for a slot holding the same two frames,
+ *     and do not depend on npairs or on the pair's position in the list.  DT_INTERP with FAST arithmetic is rejected, as there.
+ *   - No energies or trace are recorded for pairs: dvo_get_energies / dvo_get_trace keep describing the last dvo_run.
+ *   - DVO_MEM_HOST: indices outside [0, max_batch) return DVO_ERR_ARG; the call returns when the outputs are filled.
+ *     DVO_MEM_DEVICE: indices are checked on the device; such a pair gets dvo_pair_info.status bit 1, 12 NaNs as its pose and a
+ *     NaN covariance with dvo_cov_info.status bit 0; the call is asynchronous on the context stream.
+ *   - A slot that was never prepared has no points or edges: status bit 0, as in dvo_run. */
+int dvo_align_pairs(dvo_ctx* ctx, int npairs, const int* ref_slot, const int* now_slot, const double* pose0,
+                    const dvo_solver_params* params, double* poses, dvo_pair_info* info,
+                    double* cov36, dvo_cov_info* cov_info, int mem);
 
 /* dvo_run_sequences_mem plus per-frame covariances: rel_cov [nseq][nframes][36] of rel_poses (frame 0: zeros, it anchors
  * the chain), global_cov [nseq][nframes][36] (may be NULL) of global_poses, first-order propagated along the key-frame chain:

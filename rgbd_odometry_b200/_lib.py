@@ -68,7 +68,7 @@ SYMBOLS = [
     "dvo_set_initial_pose", "dvo_run", "dvo_process", "dvo_join", "dvo_join_stream", "dvo_get_poses", "dvo_align_batch", "dvo_level_dims", "dvo_get_level_buffer",
     "dvo_get_points", "dvo_eval_normal_equations", "dvo_eval_normal_equations_ex", "dvo_get_trace", "dvo_get_energies", "dvo_enable_timing", "dvo_get_stage_ms",
     "dvo_launch_count", "dvo_gop_compose", "dvo_run_sequences", "dvo_run_sequences_gated", "dvo_run_sequences_mem",
-    "dvo_pose_covariance", "dvo_run_sequences_cov", "dvo_run_sequences_entropy",
+    "dvo_pose_covariance", "dvo_run_sequences_cov", "dvo_run_sequences_entropy", "dvo_align_pairs",
     "dvo_photo_create", "dvo_photo_destroy", "dvo_photo_set_stream", "dvo_photo_synchronize", "dvo_photo_launch_count",
     "dvo_photo_set_intrinsics", "dvo_photo_set_frames", "dvo_photo_prepare_ref", "dvo_photo_set_pose", "dvo_photo_estimate",
     "dvo_photo_get_poses", "dvo_photo_get_level", "dvo_photo_get_A", "dvo_photo_eval", "dvo_photo_put_level",
@@ -135,6 +135,8 @@ def load(build_if_missing=True):
     lib.dvo_run_sequences_mem.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(SolverParams),
                                           C.POINTER(KeyframePolicy), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.dvo_pose_covariance.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(SolverParams), C.c_int, C.c_void_p, C.c_void_p, C.c_int]
+    lib.dvo_align_pairs.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(SolverParams), C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.c_void_p, C.c_int]
     lib.dvo_run_sequences_cov.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(SolverParams),
                                           C.POINTER(KeyframePolicy), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.dvo_run_sequences_entropy.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(SolverParams),

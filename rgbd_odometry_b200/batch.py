@@ -45,6 +45,11 @@ def undistort(img, K, D):
     return out
 
 
+def records(raw, cls):
+    """ctypes array of `cls` (PairInfo, CovInfo) from the raw records align_pairs(device=True) returns as a uint8 CUDA tensor."""
+    return (cls * raw.shape[0]).from_buffer_copy(raw.cpu().numpy().tobytes())
+
+
 def _ptr(a):
     if a is None:
         return None
@@ -237,6 +242,55 @@ class BatchAligner:
         the context stream."""
         check(self.lib.dvo_pose_covariance(self.h, first, count, C.byref(params), level, C.c_void_p(cov_ptr),
                                            C.c_void_p(info_ptr) if info_ptr else None, MEM_DEVICE), "dvo_pose_covariance")
+
+    def load_frames(self, gray, depth, first=0, device=False, count=None):
+        """Load n frames into BOTH roles of slots [first, first+n) -- reference and now get the same images -- then build_pyramids(3)
+        and prepare(3), so that every one of these slots can serve as either side of align_pairs.  gray (n, H, W) u8 and depth
+        (n, H, W) u16 numpy arrays, or with device=True raw device pointers and `count`."""
+        if not device:
+            gray = np.ascontiguousarray(gray, np.uint8)
+            depth = np.ascontiguousarray(depth, np.uint16)
+            count = gray.shape[0]
+        for frame in (FRAME_REF, FRAME_NOW):
+            self.set_frames(frame, gray, depth, first=first, count=count, device=device)
+        self.build_pyramids(count, first=first, frames_mask=3)
+        self.prepare(count, first=first, frames_mask=3)
+
+    def align_pairs(self, ref_slots, now_slots, params, pose0=None, covariance=False, device=False):
+        """dvo_align_pairs: pair k aligns the reference data of slot ref_slots[k] against the now data of slot now_slots[k], both
+        already prepared (see load_frames).  Returns (poses (n, 12), info), plus (cov (n, 6, 6), cov_info) when covariance=True.
+        Host (device=False): index sequences and pose0 ((n, 12) or None = identity) on the host; numpy poses / cov and ctypes
+        arrays of PairInfo / CovInfo.  device=True: int32 CUDA tensors of indices and a float64 CUDA tensor pose0; the results are
+        CUDA tensors -- poses, cov, and the raw info / cov_info records as uint8 (n, record size), see `records` -- written
+        asynchronously on the context stream (synchronize() before reading them).  Out-of-range device indices give info status
+        bit 1 and NaN poses; on the host they raise."""
+        if device:
+            import torch
+            n = int(ref_slots.shape[0])
+            dev = ref_slots.device
+            poses = torch.empty((n, 12), dtype=torch.float64, device=dev)
+            info = torch.empty((n, C.sizeof(PairInfo)), dtype=torch.uint8, device=dev)
+            cov = torch.empty((n, 6, 6), dtype=torch.float64, device=dev) if covariance else None
+            cinfo = torch.empty((n, C.sizeof(CovInfo)), dtype=torch.uint8, device=dev) if covariance else None
+            ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+            check(self.lib.dvo_align_pairs(self.h, n, ptr(ref_slots), ptr(now_slots), ptr(pose0), C.byref(params), ptr(poses), ptr(info),
+                                           ptr(cov), ptr(cinfo), MEM_DEVICE), "dvo_align_pairs")
+        else:
+            ref_slots = np.ascontiguousarray(ref_slots, np.int32)
+            now_slots = np.ascontiguousarray(now_slots, np.int32)
+            n = ref_slots.shape[0]
+            if now_slots.shape[0] != n:
+                raise ValueError("ref_slots and now_slots differ in length")
+            if pose0 is not None:
+                pose0 = np.ascontiguousarray(pose0, np.float64).reshape(n, 12)
+            poses = np.empty((n, 12), np.float64)
+            info = (PairInfo * max(n, 1))()
+            cov = np.empty((n, 6, 6), np.float64) if covariance else None
+            cinfo = (CovInfo * max(n, 1))() if covariance else None
+            check(self.lib.dvo_align_pairs(self.h, n, _ptr(ref_slots), _ptr(now_slots), _ptr(pose0), C.byref(params), _ptr(poses),
+                                           C.cast(info, C.c_void_p), _ptr(cov), C.cast(cinfo, C.c_void_p) if covariance else None,
+                                           MEM_HOST), "dvo_align_pairs")
+        return (poses, info, cov, cinfo) if covariance else (poses, info)
 
     def level_dims(self, level):
         w, h = C.c_int(), C.c_int()

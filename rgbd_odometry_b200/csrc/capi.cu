@@ -163,6 +163,7 @@ int dvo_destroy(dvo_ctx* c) {
     cudaFree(c->npts); cudaFree(c->solve_order); cudaFree(c->seq_mask); cudaFree(c->seq_state); cudaFree(c->nedge); cudaFree(c->maxd2); cudaFree(c->pose0); cudaFree(c->pose); cudaFree(c->info);
     cudaFree(c->seq_rel); cudaFree(c->seq_kind); cudaFree(c->seq_reason); cudaFree(c->seq_glob); cudaFree(c->seq_cov); cudaFree(c->seq_gcov);
     cudaFree(c->seq_cov_info); cudaFree(c->seq_ent); cudaFree(c->cov_buf); cudaFree(c->cov_info_buf);
+    cudaFree(c->pair_ref); cudaFree(c->pair_now); cudaFree(c->pair_order); cudaFree(c->pair_pose0); cudaFree(c->pair_pose); cudaFree(c->pair_info);
     for (int k = 0; k < 2; ++k) {
         cudaFree(c->seq_stage_g[k]); cudaFree(c->seq_stage_d[k]);
         if (c->seq_ev_ready[k]) cudaEventDestroy(c->seq_ev_ready[k]);
@@ -727,6 +728,21 @@ int dvo_run_sequences_entropy(dvo_ctx* c, int nseq, int nframes, const uint8_t* 
                               rel_cov, global_cov, entropy_ratio_thresh, entropy_ratio);
 }
 
+}  // extern "C"
+
+// device results of a covariance call with host outputs: one buffer per context, grown on demand
+static int reserve_cov_buf(dvo_ctx* c, size_t n) {
+    if (c->cov_cap >= n) return DVO_OK;
+    DVO_CUDA(cudaStreamSynchronize(c->stream));
+    cudaFree(c->cov_buf); cudaFree(c->cov_info_buf); c->cov_buf = nullptr; c->cov_info_buf = nullptr; c->cov_cap = 0;
+    int rc = dalloc(&c->cov_buf, n * 36); if (rc) return rc;
+    rc = dalloc(&c->cov_info_buf, n); if (rc) return rc;
+    c->cov_cap = n;
+    return DVO_OK;
+}
+
+extern "C" {
+
 int dvo_pose_covariance(dvo_ctx* c, int first, int count, const dvo_solver_params* p, int level, double* cov36, dvo_cov_info* info, int mem) {
     if (c) { const int jr = join_aux(c); if (jr) return jr; }
     if (!range_ok(c, first, count) || !p || !cov36 || (mem != DVO_MEM_HOST && mem != DVO_MEM_DEVICE) || level < -1 || level >= c->geom.L ||
@@ -738,18 +754,74 @@ int dvo_pose_covariance(dvo_ctx* c, int first, int count, const dvo_solver_param
     if (level < 0) { dvo_set_error("dvo_pose_covariance: level = -1 and no level has iterations"); return DVO_ERR_ARG; }
     if (count == 0) return DVO_OK;
     if (mem == DVO_MEM_DEVICE) return launch_cov(c, first, count, level, p, cov36, info, 1);
-    if (c->cov_cap < (size_t)count) {                    // device results for host outputs: one buffer per context, grown on demand
-        DVO_CUDA(cudaStreamSynchronize(c->stream));
-        cudaFree(c->cov_buf); cudaFree(c->cov_info_buf); c->cov_buf = nullptr; c->cov_info_buf = nullptr; c->cov_cap = 0;
-        int rc = dalloc(&c->cov_buf, (size_t)count * 36); if (rc) return rc;
-        rc = dalloc(&c->cov_info_buf, (size_t)count); if (rc) return rc;
-        c->cov_cap = (size_t)count;
-    }
+    { const int rc = reserve_cov_buf(c, (size_t)count); if (rc) return rc; }
     const int rc = launch_cov(c, first, count, level, p, c->cov_buf, c->cov_info_buf, 1);
     if (rc) return rc;
     DVO_CUDA(cudaMemcpyAsync(cov36, c->cov_buf, sizeof(double) * 36 * count, cudaMemcpyDeviceToHost, c->stream));
     if (info) DVO_CUDA(cudaMemcpyAsync(info, c->cov_info_buf, sizeof(dvo_cov_info) * count, cudaMemcpyDeviceToHost, c->stream));
     DVO_CUDA(cudaStreamSynchronize(c->stream));
+    return DVO_OK;
+}
+
+int dvo_align_pairs(dvo_ctx* c, int npairs, const int* ref_slot, const int* now_slot, const double* pose0, const dvo_solver_params* p,
+                    double* poses, dvo_pair_info* info, double* cov36, dvo_cov_info* cov_info, int mem) {
+    if (c) { const int jr = join_aux(c); if (jr) return jr; }
+    if (!c || npairs < 0 || !ref_slot || !now_slot || !p || !poses || (mem != DVO_MEM_HOST && mem != DVO_MEM_DEVICE) ||
+        (cov36 && p->residual != DVO_RESIDUAL_DT_FLOOR && p->residual != DVO_RESIDUAL_DT_INTERP)) {
+        dvo_set_error("dvo_align_pairs: bad argument"); return DVO_ERR_ARG;
+    }
+    if (!c->haveK) { dvo_set_error("dvo_align_pairs: intrinsics not set"); return DVO_ERR_STATE; }
+    int level = -1;                                      // covariance level: the finest with iterations, as dvo_pose_covariance's -1
+    if (cov36) {
+        for (int l = 0; l < c->geom.L; ++l) if (p->iters[l] > 0) { level = l; break; }
+        if (level < 0) { dvo_set_error("dvo_align_pairs: covariance requested and no level has iterations"); return DVO_ERR_ARG; }
+    }
+    const int B = c->cfg.max_batch;
+    if (mem == DVO_MEM_HOST)                             // device indices are checked by the kernels (status bit 1)
+        for (int k = 0; k < npairs; ++k)
+            if (ref_slot[k] < 0 || ref_slot[k] >= B || now_slot[k] < 0 || now_slot[k] >= B) {
+                dvo_set_error("dvo_align_pairs: pair %d addresses slots (%d, %d) outside [0, %d)", k, ref_slot[k], now_slot[k], B);
+                return DVO_ERR_ARG;
+            }
+    if (npairs == 0) return DVO_OK;
+    const size_t n = (size_t)npairs;
+    if (c->pair_cap < n) {                               // per-pair state: one set of buffers per context, grown on demand
+        DVO_CUDA(cudaStreamSynchronize(c->stream));
+        cudaFree(c->pair_ref); cudaFree(c->pair_now); cudaFree(c->pair_order); cudaFree(c->pair_pose0); cudaFree(c->pair_pose); cudaFree(c->pair_info);
+        c->pair_ref = c->pair_now = c->pair_order = nullptr; c->pair_pose0 = c->pair_pose = nullptr; c->pair_info = nullptr; c->pair_cap = 0;
+        int rc = DVO_OK;
+        auto A = [&](int r) { if (rc == DVO_OK) rc = r; };
+        A(dalloc(&c->pair_ref, n)); A(dalloc(&c->pair_now, n)); A(dalloc(&c->pair_order, n));
+        A(dalloc(&c->pair_pose0, n * 12)); A(dalloc(&c->pair_pose, n * 12)); A(dalloc(&c->pair_info, n));
+        if (rc) return rc;
+        c->pair_cap = n;
+    }
+    const cudaMemcpyKind in = mem == DVO_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    const cudaMemcpyKind out = mem == DVO_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    DVO_CUDA(cudaMemcpyAsync(c->pair_ref, ref_slot, sizeof(int) * n, in, c->stream));
+    DVO_CUDA(cudaMemcpyAsync(c->pair_now, now_slot, sizeof(int) * n, in, c->stream));
+    std::vector<double> id;
+    if (pose0) DVO_CUDA(cudaMemcpyAsync(c->pair_pose0, pose0, sizeof(double) * 12 * n, in, c->stream));
+    else {
+        id.assign(12 * n, 0.0);
+        for (size_t k = 0; k < n; ++k) { id[12 * k] = 1.0; id[12 * k + 4] = 1.0; id[12 * k + 8] = 1.0; }
+        DVO_CUDA(cudaMemcpyAsync(c->pair_pose0, id.data(), sizeof(double) * 12 * n, cudaMemcpyHostToDevice, c->stream));
+    }
+    int rc = launch_solve_pairs(c, npairs, p);
+    if (rc) return rc;
+    double* d_cov = cov36; dvo_cov_info* d_cinfo = cov_info;
+    if (cov36 && mem == DVO_MEM_HOST) {
+        if ((rc = reserve_cov_buf(c, n))) return rc;
+        d_cov = c->cov_buf; d_cinfo = c->cov_info_buf;
+    }
+    if (cov36 && (rc = launch_cov_pairs(c, npairs, level, p, d_cov, d_cinfo))) return rc;
+    DVO_CUDA(cudaMemcpyAsync(poses, c->pair_pose, sizeof(double) * 12 * n, out, c->stream));
+    if (info) DVO_CUDA(cudaMemcpyAsync(info, c->pair_info, sizeof(dvo_pair_info) * n, out, c->stream));
+    if (cov36 && mem == DVO_MEM_HOST) {
+        DVO_CUDA(cudaMemcpyAsync(cov36, c->cov_buf, sizeof(double) * 36 * n, cudaMemcpyDeviceToHost, c->stream));
+        if (cov_info) DVO_CUDA(cudaMemcpyAsync(cov_info, c->cov_info_buf, sizeof(dvo_cov_info) * n, cudaMemcpyDeviceToHost, c->stream));
+    }
+    if (mem == DVO_MEM_HOST) DVO_CUDA(cudaStreamSynchronize(c->stream));
     return DVO_OK;
 }
 

@@ -71,6 +71,8 @@ struct dvo_ctx {
     double* seq_ent; size_t seq_ent_n;   // per-frame entropy ratio the gate saw (dvo_run_sequences_entropy)
     // device results of dvo_pose_covariance with host outputs, grown on demand
     double* cov_buf; dvo_cov_info* cov_info_buf; size_t cov_cap;
+    // dvo_align_pairs: per-pair slot indices, initial / returned poses, info records and launch order, grown on demand
+    int *pair_ref, *pair_now, *pair_order; double *pair_pose0, *pair_pose; dvo_pair_info* pair_info; size_t pair_cap;
     int sm_count;
     int solve_shape;         // threads per pair in solve_kernel: 512 when max_batch <= sm_count (one pair per SM at most), else 256
     size_t smem_optin;
@@ -141,11 +143,15 @@ int launch_d2_from_texels(dvo_ctx* c, int slot, int level, int32_t* d_out);
 // packed texels through the solver's own lookup path
 int launch_resolve_texels(dvo_ctx* c, int slot, int level, float4* d_out);
 int launch_solve(dvo_ctx* c, int first, int count, const dvo_solver_params* p);
+// solve of the npairs pairs (c->pair_ref[k], c->pair_now[k]) from c->pair_pose0 into c->pair_pose / c->pair_info
+int launch_solve_pairs(dvo_ctx* c, int npairs, const dvo_solver_params* p);
 int launch_eval(dvo_ctx* c, int slot, int level, const double* d_pose12, int jac, int weight, int arith, float huber_k, int residual,
                 double* d_out /* 6 + 36 + 1 + 1 doubles */, float* d_eps, float* d_w, float* d_u, float* d_v, float* d_J);
 // 6x6 pose covariance of slots [first, first+count) at their current pose (c->pose); record k at d_cov + 36 * k * stride.
 // With c->active set, slots whose flag is 0 are skipped and keep their records.
 int launch_cov(dvo_ctx* c, int first, int count, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info, long long stride);
+// the same for the pairs of the last launch_solve_pairs, at c->pair_pose; record k at d_cov + 36 * k
+int launch_cov_pairs(dvo_ctx* c, int npairs, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info);
 // d_rel_cov / d_glob_cov: both null, or [nseq][nframes][36] covariances to propagate along the key-frame chain
 int launch_gop(dvo_ctx* c, int nseq, int nframes, const int* d_kind, const double* d_rel, double* d_out, const double* d_rel_cov, double* d_glob_cov);
 int launch_promote(dvo_ctx* c, int first, int count);

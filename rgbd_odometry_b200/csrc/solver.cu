@@ -566,15 +566,20 @@ struct SolveArgs {
     const double* pose0; double* pose; dvo_pair_info* info; double* trace; int trace_iters; const int* order; const unsigned char* active;
     float* energy;
     dvo_solver_params prm; int first;
+    // pair launches (solve_pairs_kernel) only: reference / now slot of each pair.  Appended so that the parameter offsets of the
+    // slot kernels stay where they were.
+    const int* ref_slot; const int* now_slot;
 };
 
 // One iteration's serial tail (thread 0): best tracking, step computation, pose update.  Returns 1 to stop the level.
+// ENERGY: record energyAtEachIteration in energy_rec (slot launches; pair launches keep no per-iteration state).
+template <bool ENERGY>
 __device__ __forceinline__ int solver_step(SolverState& S, const double* tot, int nvis, int N, int itr, const dvo_solver_params& prm,
                                         bool need_h, dvo_pair_info* info, int level, double* trace_rec, float* energy_rec) {
     const float ratio = (float)nvis / (float)N;                                   // :457
     const float energy = (float)sqrt(tot[6]);                                      // :1310-1312
     info->iterations_run[level] = itr + 1;
-    if (itr < DVO_ENERGY_ITERS) energy_rec[itr] = energy;                          // energyAtEachIteration (:634, :690)
+    if constexpr (ENERGY) { if (itr < DVO_ENERGY_ITERS) energy_rec[itr] = energy; }   // energyAtEachIteration (:634, :690)
     double Hf[36];
     if (need_h) {
         int idx = 8;
@@ -645,18 +650,14 @@ __device__ __forceinline__ int solver_step(SolverState& S, const double* tot, in
 // (~1 ms), so with B / (CTAs resident) only a few "waves" the makespan is set by what the last-started CTAs still
 // have to do; starting the big pairs first leaves the short ones for the tail.  Work = sum_l iters[l] * npts[l],
 // bucketed into 256 classes by a single CTA (counting sort; the order inside a class is irrelevant to the results).
-__global__ void __launch_bounds__(1024) solve_order_kernel(const int* __restrict__ npts, int L, dvo_solver_params prm, int first, int count,
-                                                           int* __restrict__ order) {
+// work(i) is the work of launch entry i, id(i) what the order list holds for it.
+template <typename Work, typename Id>
+__device__ __forceinline__ void order_heaviest_first(int count, Work work, Id id, int* __restrict__ order) {
     __shared__ unsigned s_max, s_cnt[256], s_base[256];
     const int tid = threadIdx.x;
     if (tid == 0) s_max = 1u;
     if (tid < 256) s_cnt[tid] = 0u;
     __syncthreads();
-    auto work = [&](int i) {
-        unsigned wk = 0;
-        for (int l = 0; l < L; ++l) wk += (unsigned)max(prm.iters[l], 0) * (unsigned)npts[(long long)(first + i) * L + l];
-        return wk;
-    };
     unsigned m = 0;
     for (int i = tid; i < count; i += blockDim.x) m = max(m, work(i));
     atomicMax(&s_max, m);
@@ -668,16 +669,44 @@ __global__ void __launch_bounds__(1024) solve_order_kernel(const int* __restrict
     __syncthreads();
     for (int i = tid; i < count; i += blockDim.x) {
         const int cls = 255 - min(255, (int)((float)work(i) * scale));
-        order[atomicAdd(&s_base[cls], 1u)] = first + i;
+        order[atomicAdd(&s_base[cls], 1u)] = id(i);
     }
+}
+
+__global__ void __launch_bounds__(1024) solve_order_kernel(const int* __restrict__ npts, int L, dvo_solver_params prm, int first, int count,
+                                                           int* __restrict__ order) {
+    auto work = [&](int i) {
+        unsigned wk = 0;
+        for (int l = 0; l < L; ++l) wk += (unsigned)max(prm.iters[l], 0) * (unsigned)npts[(long long)(first + i) * L + l];
+        return wk;
+    };
+    order_heaviest_first(count, work, [&](int i) { return first + i; }, order);
+}
+
+// Pairs: the work of pair k is that of its reference slot (out-of-range slots weigh nothing); the list holds pair indices.
+__global__ void __launch_bounds__(1024) pair_order_kernel(const int* __restrict__ npts, int L, dvo_solver_params prm, int Bmax, int count,
+                                                          const int* __restrict__ ref_slot, int* __restrict__ order) {
+    auto work = [&](int k) {
+        const int s = ref_slot[k];
+        unsigned wk = 0;
+        if (s < 0 || s >= Bmax) return wk;
+        for (int l = 0; l < L; ++l) wk += (unsigned)max(prm.iters[l], 0) * (unsigned)npts[(long long)s * L + l];
+        return wk;
+    };
+    order_heaviest_first(count, work, [](int k) { return k; }, order);
 }
 
 // One CTA owns a frame pair for the whole coarse-to-fine schedule.  (A thread-block-cluster variant that striped a
 // pair's points over 2/4/8 CTAs and combined partial sums through distributed shared memory was measured slower --
 // 4.29 ms -> 4.58 / 5.53 / 8.62 ms per 1024 pairs -- and removed; so was a cp.async shared-memory ring that kept 2..8
 // texel gathers in flight per thread: 4.56 .. 4.72 ms.  See DESIGN.md "measured and rejected".)
-template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, int PIPE>
-__global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768) / THREADS) solve_kernel(SolveArgs a) {
+//
+// PAIRS (solve_pairs_kernel, dvo_align_pairs): the order list holds pair indices b; the reference data (edge points, npts) come
+// from slot a.ref_slot[b], the now data (texels, d2, max d2, edge counts) from slot a.now_slot[b]; pose0 / pose / info are indexed
+// by pair, and no trace or energies are written.  Otherwise b is a slot and both slots are b.  The flag is a template parameter
+// so that the slot kernels compile exactly as they would without it.
+template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, int PIPE, bool PAIRS>
+__device__ __forceinline__ void solve_body(const SolveArgs& a) {
     extern __shared__ float s_lut[];          // 2 * LUT_N floats, then the sweep's ring (PIPE > 0)
     constexpr int NACC = AccN<NEED_H>::N;
     constexpr int SOLVE_WARPS = THREADS / 32;
@@ -691,15 +720,32 @@ __global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768
     __shared__ dvo_pair_info s_info;
 
     const int b = a.order[blockIdx.x];
-    if (a.active && !a.active[b]) return;                 // masked pass (gated key-frame switch): pose / info of the slot stay as they are
+    if (!PAIRS && a.active && !a.active[b]) return;       // masked pass (gated key-frame switch): pose / info of the slot stay as they are
     const int L = a.geom.L;
     const bool lead = (threadIdx.x == 0);
+    int rb = b, nb = b;                                   // slot of the reference data, slot of the now data
+    if constexpr (PAIRS) {
+        rb = a.ref_slot[b]; nb = a.now_slot[b];
+        if (rb < 0 || rb >= a.geom.Bmax || nb < 0 || nb >= a.geom.Bmax) {                     // status bit 1, NaN pose
+            if (lead) {
+                const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+                for (int k = 0; k < 12; ++k) a.pose[12 * (long long)b + k] = qnan;
+                dvo_pair_info inf;
+                inf.status = 2; inf.laplacian_b = 0.f;
+                for (int l = 0; l < DVO_MAX_LEVELS; ++l) {
+                    inf.npts[l] = 0; inf.best_index[l] = -1; inf.iterations_run[l] = 0; inf.best_energy[l] = 0.f; inf.visible_ratio[l] = 0.f;
+                }
+                a.info[b] = inf;
+            }
+            return;
+        }
+    }
     if (lead) {
         for (int k = 0; k < 9; ++k) S.cR[k] = a.pose0[12 * (long long)b + k];
         for (int k = 0; k < 3; ++k) S.cT[k] = a.pose0[12 * (long long)b + 9 + k];
         s_info.status = 0; s_info.laplacian_b = 0.f;
         for (int l = 0; l < DVO_MAX_LEVELS; ++l) {
-            s_info.npts[l] = (l < L) ? a.npts[(long long)b * L + l] : 0; s_info.best_index[l] = -1; s_info.iterations_run[l] = 0;
+            s_info.npts[l] = (l < L) ? a.npts[(long long)rb * L + l] : 0; s_info.best_index[l] = -1; s_info.iterations_run[l] = 0;
             s_info.best_energy[l] = 0.f; s_info.visible_ratio[l] = 0.f;
         }
     }
@@ -708,15 +754,17 @@ __global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768
     for (int l = L - 1; l >= 0; --l) {
         const int iters = a.prm.iters[l];
         if (iters <= 0) continue;
-        const int N = a.npts[(long long)b * L + l];
-        const unsigned ne = a.nedge_now[(long long)b * L + l];
+        const int N = a.npts[(long long)rb * L + l];
+        const unsigned ne = a.nedge_now[(long long)nb * L + l];
         if (N <= 0 || ne == 0u) { if (lead) s_info.status |= 1; continue; }                  // reference asserts (:282)
-        const long long base = lvl_at(a.geom, l, b);
+        const long long base = lvl_at(a.geom, l, rb);
         const float* X = a.X + base; const float* Y = a.Y + base; const float* Z = a.Z + base;
         const LevelCam cam = make_level_cam(a.K, a.geom, l);
         TexSrc src;
-        src.tex8 = a.tex8 + tex_at(a.geom, l, b); src.d2 = a.d2 + base; src.lut = s_lut;
-        const unsigned mx2 = a.maxd2[(long long)b * L + l];
+        src.tex8 = a.tex8 + tex_at(a.geom, l, nb); src.lut = s_lut;
+        if constexpr (PAIRS) src.d2 = a.d2 + lvl_at(a.geom, l, nb);
+        else src.d2 = a.d2 + base;
+        const unsigned mx2 = a.maxd2[(long long)nb * L + l];
         src.scale = dtn_scale(mx2, ne);
         build_lut<THREADS>(s_lut, mx2, src.scale);           // visible after the barrier below
         if (lead) {
@@ -744,9 +792,9 @@ __global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768
             block_reduce<NACC, THREADS>(acc, nvis, s_scr, s_red, s_nv, s_tot, &s_nvtot);
             if (lead) {
                 double* tr = nullptr;
-                if (a.trace && itr < a.trace_iters)
+                if (!PAIRS && a.trace && itr < a.trace_iters)
                     tr = a.trace + (((long long)b * L + l) * a.trace_iters + itr) * DVO_TRACE_DOUBLES;
-                s_stop = solver_step(S, s_tot, s_nvtot, N, itr, a.prm, NEED_H, &s_info, l, tr, a.energy + ((long long)b * L + l) * DVO_ENERGY_ITERS);
+                s_stop = solver_step<!PAIRS>(S, s_tot, s_nvtot, N, itr, a.prm, NEED_H, &s_info, l, tr, a.energy + ((long long)b * L + l) * DVO_ENERGY_ITERS);
                 for (int k = 0; k < 9; ++k) s_pose.R[k] = (float)S.cR[k];                      // pose of the next iteration (:673-674)
                 for (int k = 0; k < 3; ++k) s_pose.T[k] = (float)S.cT[k];
             }
@@ -767,6 +815,15 @@ __global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768
         for (int k = 0; k < 3; ++k) a.pose[12 * (long long)b + 9 + k] = S.cT[k];
         a.info[b] = s_info;
     }
+}
+
+template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, int PIPE>
+__global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768) / THREADS) solve_kernel(SolveArgs a) {
+    solve_body<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE, false>(a);
+}
+template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, int PIPE>
+__global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768) / THREADS) solve_pairs_kernel(SolveArgs a) {
+    solve_body<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE, true>(a);
 }
 
 // ------------------------------------------------------------------ single evaluation (parity inspection)
@@ -832,6 +889,8 @@ struct CovArgs {
     dvo_cov_info* info;     // optional, same indexing
     long long stride;
     const unsigned char* active;   // optional per-slot mask: a slot whose flag is 0 keeps its record as it is
+    // pair launches (cov_pairs_kernel) only, appended as in SolveArgs: reference / now slot of each pair
+    const int* ref_slot; const int* now_slot;
 };
 
 // Serial tail on thread 0: H (full symmetric, row-major, in shared memory M[0..35]) -> Sigma = s2 H^-1 into out, log det H.
@@ -871,8 +930,10 @@ __device__ __forceinline__ bool cov_from_normal_matrix(double* M, double s2, dou
     return true;
 }
 
-template <int RES>
-__global__ void __launch_bounds__(COV_THREADS) cov_kernel(CovArgs a) {
+// PAIRS: CTA k evaluates pair k (a.first = 0) at its pose a.pose[k] on reference slot a.ref_slot[k] and now slot
+// a.now_slot[k]; a pair with a slot outside [0, Bmax) gets status bit 0.  As solve_body, a template flag.
+template <int RES, bool PAIRS>
+__device__ __forceinline__ void cov_body(const CovArgs& a) {
     extern __shared__ float s_lut[];
     constexpr int NACC = COV_NACC;
     constexpr int WARPS = COV_THREADS / 32;
@@ -882,9 +943,15 @@ __global__ void __launch_bounds__(COV_THREADS) cov_kernel(CovArgs a) {
     __shared__ int s_nv[WARPS];
     __shared__ int s_nvtot;
     const int b = a.first + blockIdx.x, l = a.level, L = a.geom.L;
-    if (a.active && !a.active[b]) return;                 // masked pass (key-frame switch): the slot's record stays as it is
-    const int N = a.npts[(long long)b * L + l];
-    const unsigned ne = a.nedge_now[(long long)b * L + l];
+    if (!PAIRS && a.active && !a.active[b]) return;       // masked pass (key-frame switch): the slot's record stays as it is
+    int rb = b, nb = b;                                   // slot of the reference data, slot of the now data
+    bool in_range = true;
+    if constexpr (PAIRS) {
+        rb = a.ref_slot[b]; nb = a.now_slot[b];
+        in_range = rb >= 0 && rb < a.geom.Bmax && nb >= 0 && nb < a.geom.Bmax;
+    }
+    const int N = in_range ? a.npts[(long long)rb * L + l] : 0;
+    const unsigned ne = in_range ? a.nedge_now[(long long)nb * L + l] : 0u;
     double* out = a.cov + 36 * (long long)blockIdx.x * a.stride;
     dvo_cov_info* inf = a.info ? a.info + (long long)blockIdx.x * a.stride : nullptr;
     int status = 0, nvis = 0;
@@ -893,11 +960,13 @@ __global__ void __launch_bounds__(COV_THREADS) cov_kernel(CovArgs a) {
         PoseF P;
         for (int k = 0; k < 9; ++k) P.R[k] = (float)a.pose[12 * (long long)b + k];
         for (int k = 0; k < 3; ++k) P.T[k] = (float)a.pose[12 * (long long)b + 9 + k];
-        const long long base = lvl_at(a.geom, l, b);
+        const long long base = lvl_at(a.geom, l, rb);
         const LevelCam cam = make_level_cam(a.K, a.geom, l);
         TexSrc src;
-        src.tex8 = a.tex8 + tex_at(a.geom, l, b); src.d2 = a.d2 + base; src.lut = s_lut;
-        const unsigned mx2 = a.maxd2[(long long)b * L + l];
+        src.tex8 = a.tex8 + tex_at(a.geom, l, nb); src.lut = s_lut;
+        if constexpr (PAIRS) src.d2 = a.d2 + lvl_at(a.geom, l, nb);
+        else src.d2 = a.d2 + base;
+        const unsigned mx2 = a.maxd2[(long long)nb * L + l];
         src.scale = dtn_scale(mx2, ne);
         build_lut<COV_THREADS>(s_lut, mx2, src.scale);
         __syncthreads();
@@ -931,6 +1000,11 @@ __global__ void __launch_bounds__(COV_THREADS) cov_kernel(CovArgs a) {
     }
     if (inf) { inf->status = status; inf->level = l; inf->nvis = nvis; inf->sigma2 = sigma2; inf->logdet = logdet; }
 }
+
+template <int RES>
+__global__ void __launch_bounds__(COV_THREADS) cov_kernel(CovArgs a) { cov_body<RES, false>(a); }
+template <int RES>
+__global__ void __launch_bounds__(COV_THREADS) cov_pairs_kernel(CovArgs a) { cov_body<RES, true>(a); }
 
 // ------------------------------------------------------------------ packed texels -> float images (parity inspection)
 // {DTn, gx, gy, w} of every pixel of one slot / level through exactly the code path the solver uses (packed texel or
@@ -1036,34 +1110,36 @@ static cudaError_t optin_lut_smem(int device, int bytes = LUT_BYTES) {
     return e;
 }
 
-template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE>
+// PAIRS selects solve_pairs_kernel, the same configuration launched over pairs (dvo_align_pairs)
+template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, bool PAIRS>
 static cudaError_t launch_solve_w(dvo_ctx* c, const SolveArgs& a, int count) {
     // the shipped configuration (reference Jacobian, getWeightOf weights) takes the ring sweep
     constexpr int PIPE = (WMODE == DVO_WEIGHT_REF_CAUCHY && JAC == DVO_JAC_REFERENCE) ? (NEED_H ? DVO_SOLVE_PIPE_GN : DVO_SOLVE_PIPE_SG) : 0;
     constexpr int SMEM = LUT_BYTES + PIPE * THREADS * 32;
-    const cudaError_t e = optin_lut_smem<SolveArgs, solve_kernel<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE>>(c->cfg.device, SMEM);
+    constexpr auto kern = PAIRS ? solve_pairs_kernel<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE> : solve_kernel<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE>;
+    const cudaError_t e = optin_lut_smem<SolveArgs, kern>(c->cfg.device, SMEM);
     if (e != cudaSuccess) return e;
-    solve_kernel<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE><<<count, THREADS, SMEM, c->stream>>>(a);
+    kern<<<count, THREADS, SMEM, c->stream>>>(a);
     return cudaGetLastError();
 }
 
 // the shipped weight (getWeightOf, REF_CAUCHY) on the shipped residual gets its own instantiation with the weight mode fixed at
 // compile time; every other combination takes the generic kernel that branches on the run-time value
-template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES>
+template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, bool PAIRS>
 static cudaError_t launch_solve_inst(dvo_ctx* c, const SolveArgs& a, int count) {
     if (DVO_WMODE_SPECIALIZE && ARITH == DVO_ARITH_EXACT && RES == DVO_RESIDUAL_DT_FLOOR && a.prm.weight == DVO_WEIGHT_REF_CAUCHY)
-        return launch_solve_w<ARITH, JAC, NEED_H, THREADS, RES, (ARITH == DVO_ARITH_EXACT && RES == DVO_RESIDUAL_DT_FLOOR) ? DVO_WEIGHT_REF_CAUCHY : -1>(c, a, count);
-    return launch_solve_w<ARITH, JAC, NEED_H, THREADS, RES, -1>(c, a, count);
+        return launch_solve_w<ARITH, JAC, NEED_H, THREADS, RES, (ARITH == DVO_ARITH_EXACT && RES == DVO_RESIDUAL_DT_FLOOR) ? DVO_WEIGHT_REF_CAUCHY : -1, PAIRS>(c, a, count);
+    return launch_solve_w<ARITH, JAC, NEED_H, THREADS, RES, -1, PAIRS>(c, a, count);
 }
 
-template <int ARITH, int JAC>
+template <int ARITH, int JAC, bool PAIRS>
 static cudaError_t launch_solve_t(dvo_ctx* c, const SolveArgs& a, int count, bool need_h) {
     constexpr int THREADS = 256;
     constexpr int F = DVO_RESIDUAL_DT_FLOOR, I = DVO_RESIDUAL_DT_INTERP;
     if (a.prm.residual == I) {
         if (ARITH != DVO_ARITH_EXACT) return cudaErrorNotSupported;      // the interpolated variant is built for EXACT arithmetic only
-        if (need_h) return launch_solve_inst<DVO_ARITH_EXACT, JAC, true, THREADS, I>(c, a, count);
-        return launch_solve_inst<DVO_ARITH_EXACT, JAC, false, THREADS, I>(c, a, count);
+        if (need_h) return launch_solve_inst<DVO_ARITH_EXACT, JAC, true, THREADS, I, PAIRS>(c, a, count);
+        return launch_solve_inst<DVO_ARITH_EXACT, JAC, false, THREADS, I, PAIRS>(c, a, count);
     }
     // Up to one pair per SM there is nothing to overlap a CTA with, so a pair gets 512 threads: the sweeps run twice as
     // wide and a pair's latency drops by a third (148 pairs, GN: 0.91 -> 0.62 ms).  At full load the two shapes tie
@@ -1071,35 +1147,58 @@ static cudaError_t launch_solve_t(dvo_ctx* c, const SolveArgs& a, int count, boo
     // The shape is fixed per context (dvo_create: max_batch <= SM count -> 512), never per launch: the two shapes group the
     // fp64 partial sums differently, and a pair's pose must not depend on how many pairs happen to share a launch.
     const bool wide = (ARITH == DVO_ARITH_EXACT) && c->solve_shape == 512;
-    if (wide && need_h) return launch_solve_inst<DVO_ARITH_EXACT, JAC, true, 512, F>(c, a, count);
-    if (wide) return launch_solve_inst<DVO_ARITH_EXACT, JAC, false, 512, F>(c, a, count);
-    if (need_h) return launch_solve_inst<ARITH, JAC, true, THREADS, F>(c, a, count);
-    return launch_solve_inst<ARITH, JAC, false, THREADS, F>(c, a, count);
+    if (wide && need_h) return launch_solve_inst<DVO_ARITH_EXACT, JAC, true, 512, F, PAIRS>(c, a, count);
+    if (wide) return launch_solve_inst<DVO_ARITH_EXACT, JAC, false, 512, F, PAIRS>(c, a, count);
+    if (need_h) return launch_solve_inst<ARITH, JAC, true, THREADS, F, PAIRS>(c, a, count);
+    return launch_solve_inst<ARITH, JAC, false, THREADS, F, PAIRS>(c, a, count);
 }
 
-int launch_solve(dvo_ctx* c, int first, int count, const dvo_solver_params* p) {
+// The kernel choice of every solve launch, slots (dvo_run) and pairs (dvo_align_pairs) alike.
+template <bool PAIRS>
+static cudaError_t dispatch_solve(dvo_ctx* c, const SolveArgs& a, int count, const dvo_solver_params* p) {
+    // H is needed by GN / LM, and by SUBGRAD_REF only when a trace is kept (parity tests on J^T W J).  Pair launches keep no trace
+    // but follow the same rule: H selects the reduction, and with it how the partial sums of g are grouped.
+    const bool need_h = (p->solver != DVO_SOLVER_SUBGRAD_REF) || (c->trace != nullptr);
+    const bool ex = p->arithmetic != DVO_ARITH_FAST, rj = p->jacobian != DVO_JAC_EXACT;
+    if (ex && rj) return launch_solve_t<DVO_ARITH_EXACT, DVO_JAC_REFERENCE, PAIRS>(c, a, count, need_h);
+    if (ex) return launch_solve_t<DVO_ARITH_EXACT, DVO_JAC_EXACT, PAIRS>(c, a, count, need_h);
+    if (rj) return launch_solve_t<DVO_ARITH_FAST, DVO_JAC_REFERENCE, PAIRS>(c, a, count, need_h);
+    return launch_solve_t<DVO_ARITH_FAST, DVO_JAC_EXACT, PAIRS>(c, a, count, need_h);
+}
+
+static SolveArgs solve_args(dvo_ctx* c, const dvo_solver_params* p) {
     SolveArgs a;
+    memset(&a, 0, sizeof(a));
     a.geom = c->geom; a.K = c->K; a.X = c->ptsX; a.Y = c->ptsY; a.Z = c->ptsZ; a.npts = c->npts;
     a.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L;
     a.tex8 = c->tex8; a.d2 = c->d2; a.maxd2 = c->maxd2;
+    a.prm = *p;
+    return a;
+}
+
+int launch_solve(dvo_ctx* c, int first, int count, const dvo_solver_params* p) {
+    SolveArgs a = solve_args(c, p);
     a.pose0 = c->pose0; a.pose = c->pose; a.info = c->info; a.trace = c->trace; a.trace_iters = c->cfg.trace_iters; a.energy = c->energy;
-    a.prm = *p; a.first = first;
-    // H is needed by GN / LM, and by SUBGRAD_REF only when a trace is kept (parity tests on J^T W J)
-    const bool need_h = (p->solver != DVO_SOLVER_SUBGRAD_REF) || (c->trace != nullptr);
+    a.first = first;
     if (c->trace) DVO_CUDA(cudaMemsetAsync(c->trace + (size_t)first * c->geom.L * c->cfg.trace_iters * DVO_TRACE_DOUBLES, 0,
                                            sizeof(double) * (size_t)count * c->geom.L * c->cfg.trace_iters * DVO_TRACE_DOUBLES, c->stream));
     // the order list of slots [first, first + count) lives at solve_order + first, so launches on disjoint ranges never share it
     solve_order_kernel<<<1, 1024, 0, c->stream>>>(c->npts, c->geom.L, *p, first, count, c->solve_order + first);
     a.order = c->solve_order + first; a.active = c->active;
-    const bool ex = p->arithmetic != DVO_ARITH_FAST, rj = p->jacobian != DVO_JAC_EXACT;
-    cudaError_t e;
-    if (ex && rj) e = launch_solve_t<DVO_ARITH_EXACT, DVO_JAC_REFERENCE>(c, a, count, need_h);
-    else if (ex) e = launch_solve_t<DVO_ARITH_EXACT, DVO_JAC_EXACT>(c, a, count, need_h);
-    else if (rj) e = launch_solve_t<DVO_ARITH_FAST, DVO_JAC_REFERENCE>(c, a, count, need_h);
-    else e = launch_solve_t<DVO_ARITH_FAST, DVO_JAC_EXACT>(c, a, count, need_h);
-    DVO_CUDA(e);
+    DVO_CUDA(dispatch_solve<false>(c, a, count, p));
     c->launches++;
     c->launches++;
+    return DVO_OK;
+}
+
+int launch_solve_pairs(dvo_ctx* c, int npairs, const dvo_solver_params* p) {
+    SolveArgs a = solve_args(c, p);
+    a.pose0 = c->pair_pose0; a.pose = c->pair_pose; a.info = c->pair_info;
+    a.ref_slot = c->pair_ref; a.now_slot = c->pair_now;
+    pair_order_kernel<<<1, 1024, 0, c->stream>>>(c->npts, c->geom.L, *p, c->geom.Bmax, npairs, c->pair_ref, c->pair_order);
+    a.order = c->pair_order;
+    DVO_CUDA(dispatch_solve<true>(c, a, npairs, p));
+    c->launches += 2;
     return DVO_OK;
 }
 
@@ -1145,26 +1244,39 @@ int launch_resolve_texels(dvo_ctx* c, int slot, int level, float4* d_out) {
     return DVO_OK;
 }
 
-template <int RES>
+template <int RES, bool PAIRS>
 static cudaError_t launch_cov_inst(dvo_ctx* c, const CovArgs& a, int count) {
-    const cudaError_t e = optin_lut_smem<CovArgs, cov_kernel<RES>>(c->cfg.device);
+    constexpr auto kern = PAIRS ? cov_pairs_kernel<RES> : cov_kernel<RES>;
+    const cudaError_t e = optin_lut_smem<CovArgs, kern>(c->cfg.device);
     if (e != cudaSuccess) return e;
-    cov_kernel<RES><<<count, COV_THREADS, LUT_BYTES, c->stream>>>(a);
+    kern<<<count, COV_THREADS, LUT_BYTES, c->stream>>>(a);
     return cudaGetLastError();
 }
 
-int launch_cov(dvo_ctx* c, int first, int count, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info, long long stride) {
+template <bool PAIRS>
+static int launch_cov_t(dvo_ctx* c, int first, int count, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info, long long stride) {
     if (count == 0) return DVO_OK;
     CovArgs a;
+    memset(&a, 0, sizeof(a));
     a.geom = c->geom; a.K = c->K; a.X = c->ptsX; a.Y = c->ptsY; a.Z = c->ptsZ; a.npts = c->npts;
     a.tex8 = c->tex8; a.d2 = c->d2; a.maxd2 = c->maxd2; a.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L;
     a.pose = c->pose; a.first = first; a.level = level; a.weight = p->weight; a.huber_k = p->huber_k;
-    a.cov = d_cov; a.info = d_info; a.stride = stride; a.active = c->active;
-    const cudaError_t e = p->residual == DVO_RESIDUAL_DT_INTERP ? launch_cov_inst<DVO_RESIDUAL_DT_INTERP>(c, a, count)
-                                                                : launch_cov_inst<DVO_RESIDUAL_DT_FLOOR>(c, a, count);
+    a.cov = d_cov; a.info = d_info; a.stride = stride;
+    if (PAIRS) { a.pose = c->pair_pose; a.ref_slot = c->pair_ref; a.now_slot = c->pair_now; }
+    else a.active = c->active;
+    const cudaError_t e = p->residual == DVO_RESIDUAL_DT_INTERP ? launch_cov_inst<DVO_RESIDUAL_DT_INTERP, PAIRS>(c, a, count)
+                                                                : launch_cov_inst<DVO_RESIDUAL_DT_FLOOR, PAIRS>(c, a, count);
     c->launches++;
     DVO_CUDA(e);
     return DVO_OK;
+}
+
+int launch_cov(dvo_ctx* c, int first, int count, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info, long long stride) {
+    return launch_cov_t<false>(c, first, count, level, p, d_cov, d_info, stride);
+}
+
+int launch_cov_pairs(dvo_ctx* c, int npairs, int level, const dvo_solver_params* p, double* d_cov, dvo_cov_info* d_info) {
+    return launch_cov_t<true>(c, 0, npairs, level, p, d_cov, d_info, 1);
 }
 
 int launch_gop(dvo_ctx* c, int nseq, int nframes, const int* d_kind, const double* d_rel, double* d_out, const double* d_rel_cov, double* d_glob_cov) {
