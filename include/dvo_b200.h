@@ -30,6 +30,9 @@ extern "C" {
 
 #define DVO_MAX_LEVELS 6
 
+/* DVO_ERR_NOMEM: an allocation failed, in whichever entry point made it (context creation, buffers grown on demand, per-call
+ * temporaries).  For device memory dvo_last_error() reads "cudaMalloc(<n> bytes) failed: ...".  Earlier versions returned
+ * DVO_ERR_CUDA for some of these failures. */
 enum { DVO_OK = 0, DVO_ERR_ARG = -1, DVO_ERR_CUDA = -2, DVO_ERR_STATE = -3, DVO_ERR_NOMEM = -4 };
 enum { DVO_MEM_HOST = 0, DVO_MEM_DEVICE = 1 };
 enum { DVO_FRAME_REF = 0, DVO_FRAME_NOW = 1 };

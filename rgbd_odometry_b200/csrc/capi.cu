@@ -30,12 +30,6 @@ struct StageTimer {
         float ms = 0.f; cudaEventElapsedTime(&ms, c->ev_a, c->ev_b); c->stage_ms[stage] += ms;
     }
 };
-template <typename T> int dalloc(T** p, size_t n) {
-    if (n == 0) { *p = nullptr; return DVO_OK; }
-    cudaError_t e = cudaMalloc((void**)p, n * sizeof(T));
-    if (e != cudaSuccess) { dvo_set_error("cudaMalloc(%zu bytes) failed: %s", n * sizeof(T), cudaGetErrorString(e)); return DVO_ERR_NOMEM; }
-    return DVO_OK;
-}
 bool range_ok(dvo_ctx* c, int first, int count) { return c && first >= 0 && count >= 0 && first + count <= c->cfg.max_batch; }
 // make the context stream wait for whatever dvo_process left running on the internal streams
 int join_aux(dvo_ctx* c) {
@@ -86,7 +80,6 @@ int dvo_create(const dvo_config* cfg, dvo_ctx** out) {
     DVO_CUDA(cudaSetDevice(cfg->device));
     dvo_ctx* c = new (std::nothrow) dvo_ctx();
     if (!c) return DVO_ERR_NOMEM;
-    memset(c, 0, sizeof(*c));
     c->cfg = *cfg;
     PyrGeom& g = c->geom;
     g.L = cfg->levels; g.Bmax = cfg->max_batch;
@@ -126,28 +119,28 @@ int dvo_create(const dvo_config* cfg, dvo_ctx** out) {
     const size_t T = (size_t)g.total, B = (size_t)g.Bmax;
     int rc = DVO_OK;
     auto A = [&](int r) { if (rc == DVO_OK) rc = r; };
-    for (int f = 0; f < 2; ++f) { A(dalloc(&c->gray[f], T)); A(dalloc(&c->edge[f], T)); }
-    A(dalloc(&c->depth[0], T));
-    if (cfg->keep_now_depth) { A(dalloc(&c->depth[1], T)); A(dalloc(&c->prev_gray, B * (size_t)g.P[0])); A(dalloc(&c->prev_depth, B * (size_t)g.P[0])); }
-    c->now_valid = (unsigned char*)calloc(B, 1); c->prev_valid = (unsigned char*)calloc(B, 1);
-    A(dalloc(&c->gcol, T)); A(dalloc(&c->d2, T));
-    A(dalloc(&c->tex8, (size_t)g.total_t));
-    A(dalloc(&c->ptsX, T)); A(dalloc(&c->ptsY, T)); A(dalloc(&c->ptsZ, T)); A(dalloc(&c->ptsPix, T));
-    A(dalloc(&c->npts, B * g.L)); A(dalloc(&c->solve_order, B)); A(dalloc(&c->seq_mask, B)); A(dalloc(&c->seq_state, B)); A(dalloc(&c->nedge, 2 * B * g.L)); A(dalloc(&c->maxd2, B * g.L));
-    A(dalloc(&c->pose0, B * 12)); A(dalloc(&c->pose, B * 12)); A(dalloc(&c->info, B));
-    if (cfg->trace_iters > 0) A(dalloc(&c->trace, B * g.L * cfg->trace_iters * DVO_TRACE_DOUBLES));
-    A(dalloc(&c->energy, B * g.L * DVO_ENERGY_ITERS));
+    for (int f = 0; f < 2; ++f) { A(c->gray[f].reserve(T)); A(c->edge[f].reserve(T)); }
+    A(c->depth[0].reserve(T));
+    if (cfg->keep_now_depth) { A(c->depth[1].reserve(T)); A(c->prev_gray.reserve(B * (size_t)g.P[0])); A(c->prev_depth.reserve(B * (size_t)g.P[0])); }
+    A(c->gcol.reserve(T)); A(c->d2.reserve(T));
+    A(c->tex8.reserve((size_t)g.total_t));
+    A(c->ptsX.reserve(T)); A(c->ptsY.reserve(T)); A(c->ptsZ.reserve(T)); A(c->ptsPix.reserve(T));
+    A(c->npts.reserve(B * g.L)); A(c->solve_order.reserve(B)); A(c->seq_mask.reserve(B)); A(c->seq_state.reserve(B)); A(c->nedge.reserve(2 * B * g.L)); A(c->maxd2.reserve(B * g.L));
+    A(c->pose0.reserve(B * 12)); A(c->pose.reserve(B * 12)); A(c->info.reserve(B));
+    if (cfg->trace_iters > 0) A(c->trace.reserve(B * g.L * cfg->trace_iters * DVO_TRACE_DOUBLES));
+    A(c->energy.reserve(B * g.L * DVO_ENERGY_ITERS));
     // candidate / edge bitmaps: sobel_nms_kernel -> canny_kernel (which keeps working in them when they do not fit in shared memory)
     canny_scratch_layout(g, c->bm_off, c->bm_words, &c->bitmap_scratch_words);
-    A(dalloc(&c->bitmap_scratch, c->bitmap_scratch_words * B * 2));
+    A(c->bitmap_scratch.reserve(c->bitmap_scratch_words * B * 2));
     if (rc != DVO_OK) { dvo_destroy(c); return rc; }
+    c->now_valid.reset(new (std::nothrow) unsigned char[B]());
+    c->prev_valid.reset(new (std::nothrow) unsigned char[B]());
+    if (!c->now_valid || !c->prev_valid) { dvo_set_error("dvo_create: out of host memory"); dvo_destroy(c); return DVO_ERR_NOMEM; }
     CREATE_CUDA(cudaMemsetAsync(c->npts, 0, sizeof(int) * B * g.L, c->stream));
     CREATE_CUDA(cudaMemsetAsync(c->bitmap_scratch, 0, sizeof(uint32_t) * c->bitmap_scratch_words * B * 2, c->stream));   // the bitmaps' zero borders are never written
     CREATE_CUDA(cudaMemsetAsync(c->nedge, 0, sizeof(unsigned) * 2 * B * g.L, c->stream));
     CREATE_CUDA(cudaMemsetAsync(c->maxd2, 0, sizeof(unsigned) * B * g.L, c->stream));
     CREATE_CUDA(cudaMemsetAsync(c->info, 0, sizeof(dvo_pair_info) * B, c->stream));
-    CREATE_CUDA(cudaMallocHost((void**)&c->h_pose, sizeof(double) * 12 * B));
-    CREATE_CUDA(cudaMallocHost((void**)&c->h_info, sizeof(dvo_pair_info) * B));
     dvo_set_initial_pose(c, 0, g.Bmax, nullptr, DVO_MEM_HOST);
     CREATE_CUDA(cudaStreamSynchronize(c->stream));
     *out = c;
@@ -158,21 +151,10 @@ int dvo_destroy(dvo_ctx* c) {
     if (!c) return DVO_OK;
     cudaSetDevice(c->cfg.device);
     if (c->own_stream) cudaStreamSynchronize(c->own_stream);
-    for (int f = 0; f < 2; ++f) { cudaFree(c->gray[f]); cudaFree(c->depth[f]); cudaFree(c->edge[f]); }
-    cudaFree(c->gcol); cudaFree(c->d2); cudaFree(c->tex8); cudaFree(c->ptsX); cudaFree(c->ptsY); cudaFree(c->ptsZ); cudaFree(c->ptsPix);
-    cudaFree(c->npts); cudaFree(c->solve_order); cudaFree(c->seq_mask); cudaFree(c->seq_state); cudaFree(c->nedge); cudaFree(c->maxd2); cudaFree(c->pose0); cudaFree(c->pose); cudaFree(c->info);
-    cudaFree(c->seq_rel); cudaFree(c->seq_kind); cudaFree(c->seq_reason); cudaFree(c->seq_glob); cudaFree(c->seq_cov); cudaFree(c->seq_gcov);
-    cudaFree(c->seq_cov_info); cudaFree(c->seq_ent); cudaFree(c->cov_buf); cudaFree(c->cov_info_buf);
-    cudaFree(c->pair_ref); cudaFree(c->pair_now); cudaFree(c->pair_order); cudaFree(c->pair_pose0); cudaFree(c->pair_pose); cudaFree(c->pair_info);
     for (int k = 0; k < 2; ++k) {
-        cudaFree(c->seq_stage_g[k]); cudaFree(c->seq_stage_d[k]);
         if (c->seq_ev_ready[k]) cudaEventDestroy(c->seq_ev_ready[k]);
         if (c->seq_ev_free[k]) cudaEventDestroy(c->seq_ev_free[k]);
     }
-    cudaFree(c->trace); cudaFree(c->energy); cudaFree(c->bitmap_scratch); cudaFree(c->prev_gray); cudaFree(c->prev_depth); cudaFree(c->raw_bgr); cudaFree(c->raw_depth);
-    free(c->now_valid); free(c->prev_valid);
-    if (c->h_pose) cudaFreeHost(c->h_pose);
-    if (c->h_info) cudaFreeHost(c->h_info);
     if (c->ev_a) cudaEventDestroy(c->ev_a);
     if (c->ev_b) cudaEventDestroy(c->ev_b);
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
@@ -185,7 +167,7 @@ int dvo_destroy(dvo_ctx* c) {
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     for (int i = 0; i < 16; ++i) if (c->ev_chunk[i]) cudaEventDestroy(c->ev_chunk[i]);
     if (c->ev_entry) cudaEventDestroy(c->ev_entry);
-    delete c;
+    delete c;                                            // the buffers free themselves
     return DVO_OK;
 }
 
@@ -257,16 +239,14 @@ int dvo_set_frames_raw(dvo_ctx* c, int frame, int first, int count, const uint8_
     const size_t P0 = c->geom.P[0];
     const uint8_t* d_bgr = bgr; const float* d_dm = depth_m;
     if (mem != DVO_MEM_DEVICE) {
-        if (c->raw_capacity < (size_t)count) {           // staging sized for the largest range seen so far
-            DVO_CUDA(cudaStreamSynchronize(c->stream));
-            cudaFree(c->raw_bgr); cudaFree(c->raw_depth); c->raw_bgr = nullptr; c->raw_depth = nullptr; c->raw_capacity = 0;
-            int rc = dalloc(&c->raw_bgr, (size_t)count * P0 * 3); if (rc) return rc;
-            rc = dalloc(&c->raw_depth, (size_t)count * P0); if (rc) return rc;
-            c->raw_capacity = (size_t)count;
-        }
+        // staging sized for the largest range seen so far; a copy still in flight may read the buffers a growth replaces
+        if (c->raw_bgr.n < (size_t)count * P0 * 3) DVO_CUDA(cudaStreamSynchronize(c->stream));
+        int rc = c->raw_bgr.reserve((size_t)count * P0 * 3);
+        if (rc == DVO_OK) rc = c->raw_depth.reserve((size_t)count * P0);
+        if (rc) return rc;
         DVO_CUDA(cudaMemcpyAsync(c->raw_bgr, bgr, P0 * count * 3, cudaMemcpyHostToDevice, c->stream));
         if (depth_m) DVO_CUDA(cudaMemcpyAsync(c->raw_depth, depth_m, P0 * count * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-        d_bgr = c->raw_bgr; d_dm = depth_m ? c->raw_depth : nullptr;
+        d_bgr = c->raw_bgr; d_dm = depth_m ? c->raw_depth.get() : nullptr;
     }
     return launch_ingest_raw(c, frame, first, count, d_bgr, d_dm);
 }
@@ -546,30 +526,16 @@ int run_sequences_core(dvo_ctx* c, const char* who, int nseq, int nframes, const
     auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == DVO_OK) { dvo_set_error("%s: %s", who, cudaGetErrorString(e)); rc = DVO_ERR_CUDA; } return rc != DVO_OK; };
 
     // ---- buffers: record of the run (device), staging for the uploads -- owned by the context, grown on demand, reused across calls
-    if (c->seq_rec_n < n) {
-        cudaFree(c->seq_rel); cudaFree(c->seq_kind); cudaFree(c->seq_reason); c->seq_rel = nullptr; c->seq_kind = nullptr; c->seq_reason = nullptr; c->seq_rec_n = 0;
-        fail(cudaMalloc((void**)&c->seq_rel, sizeof(double) * 12 * n)); fail(cudaMalloc((void**)&c->seq_kind, sizeof(int) * n)); fail(cudaMalloc((void**)&c->seq_reason, sizeof(int) * n));
-        if (rc == DVO_OK) c->seq_rec_n = n;
-    }
-    if (host_in && c->seq_stage_slots < (size_t)nseq) {
-        for (int k = 0; k < 2; ++k) { cudaFree(c->seq_stage_g[k]); cudaFree(c->seq_stage_d[k]); c->seq_stage_g[k] = nullptr; c->seq_stage_d[k] = nullptr; }
-        c->seq_stage_slots = 0;
+    auto A = [&](int r) { if (rc == DVO_OK) rc = r; };
+    A(c->seq_rel.reserve(12 * n)); A(c->seq_kind.reserve(n)); A(c->seq_reason.reserve(n));
+    if (host_in)
         for (int k = 0; k < 2 && rc == DVO_OK; ++k) {
-            fail(cudaMalloc((void**)&c->seq_stage_g[k], P0 * nseq)); fail(cudaMalloc((void**)&c->seq_stage_d[k], P0 * nseq * sizeof(uint16_t)));
+            A(c->seq_stage_g[k].reserve(P0 * nseq)); A(c->seq_stage_d[k].reserve(P0 * nseq));
             if (!c->seq_ev_ready[k]) fail(cudaEventCreateWithFlags(&c->seq_ev_ready[k], cudaEventDisableTiming));
             if (!c->seq_ev_free[k]) fail(cudaEventCreateWithFlags(&c->seq_ev_free[k], cudaEventDisableTiming));
         }
-        if (rc == DVO_OK) c->seq_stage_slots = (size_t)nseq;
-    }
-    if (cov && c->seq_cov_n < n) {
-        cudaFree(c->seq_cov); cudaFree(c->seq_cov_info); c->seq_cov = nullptr; c->seq_cov_info = nullptr; c->seq_cov_n = 0;
-        fail(cudaMalloc((void**)&c->seq_cov, sizeof(double) * 36 * n)); fail(cudaMalloc((void**)&c->seq_cov_info, sizeof(dvo_cov_info) * n));
-        if (rc == DVO_OK) c->seq_cov_n = n;
-    }
-    if (entropy_on && c->seq_ent_n < n) {
-        cudaFree(c->seq_ent); c->seq_ent = nullptr; c->seq_ent_n = 0;
-        if (!fail(cudaMalloc((void**)&c->seq_ent, sizeof(double) * n))) c->seq_ent_n = n;
-    }
+    if (cov) { A(c->seq_cov.reserve(36 * n)); A(c->seq_cov_info.reserve(n)); }
+    if (entropy_on) A(c->seq_ent.reserve(n));
     if (rc != DVO_OK) return rc;
     double* d_rel = c->seq_rel; int* d_kind = c->seq_kind; int* d_reason = c->seq_reason; double* d_glob = nullptr;
     uint8_t* stage_g[2] = {c->seq_stage_g[0], c->seq_stage_g[1]}; uint16_t* stage_d[2] = {c->seq_stage_d[0], c->seq_stage_d[1]};
@@ -640,7 +606,7 @@ int run_sequences_core(dvo_ctx* c, const char* who, int nseq, int nframes, const
         dvo_cov_info* const cinfo_t = entropy_on ? c->seq_cov_info + t : nullptr;
         if (entropy_on && (rc = launch_cov(c, 0, nseq, finest, p, cov_t, cinfo_t, nframes))) break;
         seq_gate_kernel<<<blk, 128, 0, c->stream>>>(nseq, nframes, t, *pol, finest, c->info, c->pose, c->pose0, c->seq_state, c->seq_mask, d_rel, d_kind, d_reason,
-                                                    entropy_on ? c->seq_cov_info : nullptr, ent_thr, c->seq_ent);
+                                                    entropy_on ? c->seq_cov_info.get() : nullptr, ent_thr, c->seq_ent);
         c->launches++;
         if (fail(cudaGetLastError())) break;
         if (switch_pass) {
@@ -662,17 +628,11 @@ int run_sequences_core(dvo_ctx* c, const char* who, int nseq, int nframes, const
     c->active = nullptr;
     c->timing = timing;
     if (rc == DVO_OK && (global_poses || global_cov)) {
-        if (c->seq_glob_n < n) {
-            cudaFree(c->seq_glob); c->seq_glob = nullptr; c->seq_glob_n = 0;
-            if (!fail(cudaMalloc((void**)&c->seq_glob, sizeof(double) * 19 * n))) c->seq_glob_n = n;
-        }
-        if (global_cov && rc == DVO_OK && c->seq_gcov_n < n) {
-            cudaFree(c->seq_gcov); c->seq_gcov = nullptr; c->seq_gcov_n = 0;
-            if (!fail(cudaMalloc((void**)&c->seq_gcov, sizeof(double) * 36 * n))) c->seq_gcov_n = n;
-        }
+        A(c->seq_glob.reserve(19 * n));
+        if (global_cov && rc == DVO_OK) A(c->seq_gcov.reserve(36 * n));
         d_glob = c->seq_glob;
         if (rc == DVO_OK) {
-            rc = launch_gop(c, nseq, nframes, d_kind, d_rel, d_glob, global_cov ? c->seq_cov : nullptr, global_cov ? c->seq_gcov : nullptr);
+            rc = launch_gop(c, nseq, nframes, d_kind, d_rel, d_glob, global_cov ? c->seq_cov.get() : nullptr, global_cov ? c->seq_gcov.get() : nullptr);
             if (rc == DVO_OK && global_poses) fail(cudaMemcpyAsync(global_poses, d_glob, sizeof(double) * 19 * n, cudaMemcpyDeviceToHost, c->stream));
             if (rc == DVO_OK && global_cov) fail(cudaMemcpyAsync(global_cov, c->seq_gcov, sizeof(double) * 36 * n, cudaMemcpyDeviceToHost, c->stream));
         }
@@ -730,17 +690,6 @@ int dvo_run_sequences_entropy(dvo_ctx* c, int nseq, int nframes, const uint8_t* 
 
 }  // extern "C"
 
-// device results of a covariance call with host outputs: one buffer per context, grown on demand
-static int reserve_cov_buf(dvo_ctx* c, size_t n) {
-    if (c->cov_cap >= n) return DVO_OK;
-    DVO_CUDA(cudaStreamSynchronize(c->stream));
-    cudaFree(c->cov_buf); cudaFree(c->cov_info_buf); c->cov_buf = nullptr; c->cov_info_buf = nullptr; c->cov_cap = 0;
-    int rc = dalloc(&c->cov_buf, n * 36); if (rc) return rc;
-    rc = dalloc(&c->cov_info_buf, n); if (rc) return rc;
-    c->cov_cap = n;
-    return DVO_OK;
-}
-
 extern "C" {
 
 int dvo_pose_covariance(dvo_ctx* c, int first, int count, const dvo_solver_params* p, int level, double* cov36, dvo_cov_info* info, int mem) {
@@ -754,9 +703,10 @@ int dvo_pose_covariance(dvo_ctx* c, int first, int count, const dvo_solver_param
     if (level < 0) { dvo_set_error("dvo_pose_covariance: level = -1 and no level has iterations"); return DVO_ERR_ARG; }
     if (count == 0) return DVO_OK;
     if (mem == DVO_MEM_DEVICE) return launch_cov(c, first, count, level, p, cov36, info, 1);
-    { const int rc = reserve_cov_buf(c, (size_t)count); if (rc) return rc; }
-    const int rc = launch_cov(c, first, count, level, p, c->cov_buf, c->cov_info_buf, 1);
-    if (rc) return rc;
+    if (c->cov_buf.n < 36 * (size_t)count) DVO_CUDA(cudaStreamSynchronize(c->stream));   // growth replaces buffers work in flight may use
+    int rc;
+    if ((rc = c->cov_buf.reserve(36 * (size_t)count)) || (rc = c->cov_info_buf.reserve(count))) return rc;
+    if ((rc = launch_cov(c, first, count, level, p, c->cov_buf, c->cov_info_buf, 1))) return rc;
     DVO_CUDA(cudaMemcpyAsync(cov36, c->cov_buf, sizeof(double) * 36 * count, cudaMemcpyDeviceToHost, c->stream));
     if (info) DVO_CUDA(cudaMemcpyAsync(info, c->cov_info_buf, sizeof(dvo_cov_info) * count, cudaMemcpyDeviceToHost, c->stream));
     DVO_CUDA(cudaStreamSynchronize(c->stream));
@@ -785,17 +735,13 @@ int dvo_align_pairs(dvo_ctx* c, int npairs, const int* ref_slot, const int* now_
             }
     if (npairs == 0) return DVO_OK;
     const size_t n = (size_t)npairs;
-    if (c->pair_cap < n) {                               // per-pair state: one set of buffers per context, grown on demand
-        DVO_CUDA(cudaStreamSynchronize(c->stream));
-        cudaFree(c->pair_ref); cudaFree(c->pair_now); cudaFree(c->pair_order); cudaFree(c->pair_pose0); cudaFree(c->pair_pose); cudaFree(c->pair_info);
-        c->pair_ref = c->pair_now = c->pair_order = nullptr; c->pair_pose0 = c->pair_pose = nullptr; c->pair_info = nullptr; c->pair_cap = 0;
-        int rc = DVO_OK;
-        auto A = [&](int r) { if (rc == DVO_OK) rc = r; };
-        A(dalloc(&c->pair_ref, n)); A(dalloc(&c->pair_now, n)); A(dalloc(&c->pair_order, n));
-        A(dalloc(&c->pair_pose0, n * 12)); A(dalloc(&c->pair_pose, n * 12)); A(dalloc(&c->pair_info, n));
-        if (rc) return rc;
-        c->pair_cap = n;
-    }
+    // per-pair state: one set of buffers per context, grown on demand; growth replaces buffers work in flight may use
+    if (c->pair_ref.n < n) DVO_CUDA(cudaStreamSynchronize(c->stream));
+    int rc = DVO_OK;
+    auto A = [&](int r) { if (rc == DVO_OK) rc = r; };
+    A(c->pair_ref.reserve(n)); A(c->pair_now.reserve(n)); A(c->pair_order.reserve(n));
+    A(c->pair_pose0.reserve(n * 12)); A(c->pair_pose.reserve(n * 12)); A(c->pair_info.reserve(n));
+    if (rc) return rc;
     const cudaMemcpyKind in = mem == DVO_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     const cudaMemcpyKind out = mem == DVO_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
     DVO_CUDA(cudaMemcpyAsync(c->pair_ref, ref_slot, sizeof(int) * n, in, c->stream));
@@ -807,11 +753,11 @@ int dvo_align_pairs(dvo_ctx* c, int npairs, const int* ref_slot, const int* now_
         for (size_t k = 0; k < n; ++k) { id[12 * k] = 1.0; id[12 * k + 4] = 1.0; id[12 * k + 8] = 1.0; }
         DVO_CUDA(cudaMemcpyAsync(c->pair_pose0, id.data(), sizeof(double) * 12 * n, cudaMemcpyHostToDevice, c->stream));
     }
-    int rc = launch_solve_pairs(c, npairs, p);
-    if (rc) return rc;
+    if ((rc = launch_solve_pairs(c, npairs, p))) return rc;
     double* d_cov = cov36; dvo_cov_info* d_cinfo = cov_info;
     if (cov36 && mem == DVO_MEM_HOST) {
-        if ((rc = reserve_cov_buf(c, n))) return rc;
+        if (c->cov_buf.n < 36 * n) DVO_CUDA(cudaStreamSynchronize(c->stream));   // as in dvo_pose_covariance
+        if ((rc = c->cov_buf.reserve(36 * n)) || (rc = c->cov_info_buf.reserve(n))) return rc;
         d_cov = c->cov_buf; d_cinfo = c->cov_info_buf;
     }
     if (cov36 && (rc = launch_cov_pairs(c, npairs, level, p, d_cov, d_cinfo))) return rc;
@@ -849,27 +795,21 @@ int dvo_get_level_buffer(dvo_ctx* c, int slot, int frame, int level, int which, 
     }
     if (which == DVO_BUF_D2) {      // the fused EDT + texel kernel leaves the 32-bit image sparse: rebuild the dense one from the texels
         if (bytes < P * 4) { dvo_set_error("dvo_get_level_buffer: destination too small"); return DVO_ERR_ARG; }
-        int32_t* d_tmp = nullptr;
-        DVO_CUDA(cudaMalloc((void**)&d_tmp, P * 4));
-        const int rc = launch_d2_from_texels(c, slot, level, d_tmp);
-        cudaError_t ce = rc ? cudaSuccess : cudaMemcpyAsync(dst, d_tmp, P * 4, cudaMemcpyDeviceToHost, c->stream);
-        if (ce == cudaSuccess) ce = cudaStreamSynchronize(c->stream);
-        cudaFree(d_tmp);
-        if (rc) return rc;
-        DVO_CUDA(ce);
+        DevBuf<int32_t> d_tmp;
+        int rc;
+        if ((rc = d_tmp.reserve(P)) || (rc = launch_d2_from_texels(c, slot, level, d_tmp))) return rc;
+        DVO_CUDA(cudaMemcpyAsync(dst, d_tmp, P * 4, cudaMemcpyDeviceToHost, c->stream));
+        DVO_CUDA(cudaStreamSynchronize(c->stream));
         return DVO_OK;
     }
     if (which >= DVO_BUF_DTN) {      // no float images are kept: evaluate them from the packed texels for this slot / level on demand
         if (bytes < P * 4) { dvo_set_error("dvo_get_level_buffer: destination too small"); return DVO_ERR_ARG; }
         std::vector<float> tmp(P * 4);
-        float4* d_tmp = nullptr;
-        DVO_CUDA(cudaMalloc((void**)&d_tmp, P * 16));
-        const int rc = launch_resolve_texels(c, slot, level, d_tmp);
-        if (rc) { cudaFree(d_tmp); return rc; }
-        cudaError_t ce = cudaMemcpyAsync(tmp.data(), d_tmp, P * 16, cudaMemcpyDeviceToHost, c->stream);
-        if (ce == cudaSuccess) ce = cudaStreamSynchronize(c->stream);
-        cudaFree(d_tmp);
-        DVO_CUDA(ce);
+        DevBuf<float4> d_tmp;
+        int rc;
+        if ((rc = d_tmp.reserve(P)) || (rc = launch_resolve_texels(c, slot, level, d_tmp))) return rc;
+        DVO_CUDA(cudaMemcpyAsync(tmp.data(), d_tmp, P * 16, cudaMemcpyDeviceToHost, c->stream));
+        DVO_CUDA(cudaStreamSynchronize(c->stream));
         const int comp = which - DVO_BUF_DTN;
         float* d = (float*)dst;
         for (size_t i = 0; i < P; ++i) d[i] = tmp[4 * i + comp];
@@ -943,52 +883,38 @@ int dvo_eval_normal_equations_ex(dvo_ctx* c, int slot, int level, const double* 
     int N = 0;
     DVO_CUDA(cudaMemcpyAsync(&N, c->npts + (size_t)slot * c->geom.L + level, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     DVO_CUDA(cudaStreamSynchronize(c->stream));
-    double* d_pose = nullptr; double* d_out = nullptr; float* d_pp = nullptr;
+    DevBuf<double> d_pose, d_out; DevBuf<float> d_pp;
     const bool pp = eps || w || u || v || J;
     const size_t n1 = (size_t)(N > 0 ? N : 1);
-    {   // temporaries: released on every path
-        cudaError_t e = cudaMalloc((void**)&d_pose, sizeof(double) * 12);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&d_out, sizeof(double) * 44);
-        if (e == cudaSuccess && pp) e = cudaMalloc((void**)&d_pp, sizeof(float) * n1 * 10);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d_pose, R9T3, sizeof(double) * 12, cudaMemcpyHostToDevice, c->stream);
-        if (e != cudaSuccess) {
-            dvo_set_error("dvo_eval_normal_equations: %s", cudaGetErrorString(e));
-            cudaFree(d_pose); cudaFree(d_out); cudaFree(d_pp);
-            return DVO_ERR_CUDA;
-        }
-    }
+    int rc;
+    if ((rc = d_pose.reserve(12)) || (rc = d_out.reserve(44)) || (pp && (rc = d_pp.reserve(n1 * 10)))) return rc;
+    DVO_CUDA(cudaMemcpyAsync(d_pose, R9T3, sizeof(double) * 12, cudaMemcpyHostToDevice, c->stream));
     float *de = nullptr, *dw = nullptr, *du = nullptr, *dv = nullptr, *dJ = nullptr;
     if (pp) { de = d_pp; dw = d_pp + n1; du = d_pp + 2 * n1; dv = d_pp + 3 * n1; dJ = d_pp + 4 * n1; }
-    int rc = launch_eval(c, slot, level, d_pose, prm->jacobian, prm->weight, prm->arithmetic, prm->huber_k, prm->residual, d_out, de, dw, du, dv, dJ);
-    if (rc == DVO_OK) {
-        double out[44];
-        std::vector<float> host(pp ? n1 * 10 : 0);
-        cudaError_t e = cudaMemcpyAsync(out, d_out, sizeof(out), cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess && pp && N > 0) e = cudaMemcpyAsync(host.data(), d_pp, sizeof(float) * n1 * 10, cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        if (e != cudaSuccess) { dvo_set_error("dvo_eval_normal_equations: %s", cudaGetErrorString(e)); rc = DVO_ERR_CUDA; }
-        else {
-            if (g6) memcpy(g6, out, sizeof(double) * 6);
-            if (H36) memcpy(H36, out + 6, sizeof(double) * 36);
-            if (sumsq) *sumsq = out[42];
-            if (nvis) *nvis = (int)out[43];
-            if (pp && N > 0) {                       // per-point arrays are returned in the reference's (column-major) order
-                std::vector<int> perm;
-                rc = reference_order(c, slot, level, N, perm);
-                if (rc == DVO_OK)
-                    for (int k = 0; k < N; ++k) {
-                        const size_t i = (size_t)perm[k];
-                        if (eps) eps[k] = host[i];
-                        if (w) w[k] = host[n1 + i];
-                        if (u) u[k] = host[2 * n1 + i];
-                        if (v) v[k] = host[3 * n1 + i];
-                        if (J) for (int q = 0; q < 6; ++q) J[6 * (size_t)k + q] = host[4 * n1 + 6 * i + q];
-                    }
-            }
+    if ((rc = launch_eval(c, slot, level, d_pose, prm->jacobian, prm->weight, prm->arithmetic, prm->huber_k, prm->residual, d_out, de, dw, du, dv, dJ)))
+        return rc;
+    double out[44];
+    std::vector<float> host(pp ? n1 * 10 : 0);
+    DVO_CUDA(cudaMemcpyAsync(out, d_out, sizeof(out), cudaMemcpyDeviceToHost, c->stream));
+    if (pp && N > 0) DVO_CUDA(cudaMemcpyAsync(host.data(), d_pp, sizeof(float) * n1 * 10, cudaMemcpyDeviceToHost, c->stream));
+    DVO_CUDA(cudaStreamSynchronize(c->stream));
+    if (g6) memcpy(g6, out, sizeof(double) * 6);
+    if (H36) memcpy(H36, out + 6, sizeof(double) * 36);
+    if (sumsq) *sumsq = out[42];
+    if (nvis) *nvis = (int)out[43];
+    if (pp && N > 0) {                               // per-point arrays are returned in the reference's (column-major) order
+        std::vector<int> perm;
+        if ((rc = reference_order(c, slot, level, N, perm))) return rc;
+        for (int k = 0; k < N; ++k) {
+            const size_t i = (size_t)perm[k];
+            if (eps) eps[k] = host[i];
+            if (w) w[k] = host[n1 + i];
+            if (u) u[k] = host[2 * n1 + i];
+            if (v) v[k] = host[3 * n1 + i];
+            if (J) for (int q = 0; q < 6; ++q) J[6 * (size_t)k + q] = host[4 * n1 + 6 * i + q];
         }
     }
-    cudaFree(d_pose); cudaFree(d_out); cudaFree(d_pp);
-    return rc;
+    return DVO_OK;
 }
 
 int dvo_get_trace(dvo_ctx* c, int slot, int level, double* trace) {
@@ -1031,31 +957,19 @@ int dvo_gop_compose(dvo_ctx* c, int nseq, int nframes, const int* kind, const do
     if (!c || nseq < 1 || nframes < 1 || !kind || !rel || !out) return DVO_ERR_ARG;
     const size_t n = (size_t)nseq * nframes;
     if (mem == DVO_MEM_DEVICE) return launch_gop(c, nseq, nframes, kind, rel, out, nullptr, nullptr);
-    int* d_kind = nullptr; double* d_rel = nullptr; double* d_out = nullptr;
-    {
-        cudaError_t e = cudaMalloc((void**)&d_kind, sizeof(int) * n);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&d_rel, sizeof(double) * 12 * n);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&d_out, sizeof(double) * 19 * n);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d_kind, kind, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d_rel, rel, sizeof(double) * 12 * n, cudaMemcpyHostToDevice, c->stream);
-        if (e != cudaSuccess) {
-            dvo_set_error("dvo_gop_compose: %s", cudaGetErrorString(e));
-            cudaFree(d_kind); cudaFree(d_rel); cudaFree(d_out);
-            return DVO_ERR_CUDA;
-        }
-    }
-    int rc = launch_gop(c, nseq, nframes, d_kind, d_rel, d_out, nullptr, nullptr);
-    if (rc == DVO_OK) {
-        cudaError_t e = cudaMemcpyAsync(out, d_out, sizeof(double) * 19 * n, cudaMemcpyDeviceToHost, c->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        if (e != cudaSuccess) { dvo_set_error("dvo_gop_compose: %s", cudaGetErrorString(e)); rc = DVO_ERR_CUDA; }
-    }
-    cudaFree(d_kind); cudaFree(d_rel); cudaFree(d_out);
-    return rc;
+    DevBuf<int> d_kind; DevBuf<double> d_rel, d_out;
+    int rc;
+    if ((rc = d_kind.reserve(n)) || (rc = d_rel.reserve(12 * n)) || (rc = d_out.reserve(19 * n))) return rc;
+    DVO_CUDA(cudaMemcpyAsync(d_kind, kind, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
+    DVO_CUDA(cudaMemcpyAsync(d_rel, rel, sizeof(double) * 12 * n, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = launch_gop(c, nseq, nframes, d_kind, d_rel, d_out, nullptr, nullptr))) return rc;
+    DVO_CUDA(cudaMemcpyAsync(out, d_out, sizeof(double) * 19 * n, cudaMemcpyDeviceToHost, c->stream));
+    DVO_CUDA(cudaStreamSynchronize(c->stream));
+    return DVO_OK;
 }
 
 // ---- device-resident storage blobs (PyramidalStorageStruct keeps caller-provided level arrays on the device) ----
-struct dvo_blob { void* d; size_t bytes; int device; };
+struct dvo_blob { DevBuf<unsigned char> d; size_t bytes; int device; };
 
 int dvo_blob_create(size_t bytes, int device, dvo_blob** out) {
     if (!out || bytes == 0) { dvo_set_error("dvo_blob_create: bad argument"); return DVO_ERR_ARG; }
@@ -1065,8 +979,8 @@ int dvo_blob_create(size_t bytes, int device, dvo_blob** out) {
     DVO_CUDA(cudaSetDevice(device));
     dvo_blob* b = new (std::nothrow) dvo_blob();
     if (!b) return DVO_ERR_NOMEM;
-    b->bytes = bytes; b->device = device; b->d = nullptr;
-    if (cudaMalloc(&b->d, bytes) != cudaSuccess) { cudaGetLastError(); delete b; dvo_set_error("dvo_blob_create: cudaMalloc(%zu) failed", bytes); return DVO_ERR_NOMEM; }
+    b->bytes = bytes; b->device = device;
+    if (const int rc = b->d.reserve(bytes)) { cudaGetLastError(); delete b; return rc; }
     *out = b;
     return DVO_OK;
 }
@@ -1082,12 +996,11 @@ int dvo_blob_download(dvo_blob* b, void* host_dst, size_t bytes) {
     DVO_CUDA(cudaMemcpy(host_dst, b->d, bytes, cudaMemcpyDeviceToHost));
     return DVO_OK;
 }
-void* dvo_blob_device_ptr(dvo_blob* b) { return b ? b->d : nullptr; }
+void* dvo_blob_device_ptr(dvo_blob* b) { return b ? b->d.get() : nullptr; }
 size_t dvo_blob_bytes(dvo_blob* b) { return b ? b->bytes : 0; }
 int dvo_blob_destroy(dvo_blob* b) {
     if (!b) return DVO_OK;
     cudaSetDevice(b->device);
-    cudaFree(b->d);
     delete b;
     return DVO_OK;
 }

@@ -61,11 +61,11 @@ extern "C" int dvo_undistort(const void* src, void* dst, int width, int height, 
     const size_t bytes = (size_t)width * height * a.cn * (type == DVO_IMG_U16C1 ? 2 : 1) * count;
     const cudaStream_t s = (cudaStream_t)cuda_stream;
     const void* d_src = src; void* d_dst = dst;
-    void *t_src = nullptr, *t_dst = nullptr;
+    DevBuf<uint8_t> t_src, t_dst;
     if (mem != DVO_MEM_DEVICE) {
-        DVO_CUDA(cudaMalloc(&t_src, bytes));
-        if (cudaMalloc(&t_dst, bytes) != cudaSuccess) { cudaFree(t_src); dvo_set_error("dvo_undistort: out of device memory"); return DVO_ERR_NOMEM; }
-        cudaMemcpyAsync(t_src, src, bytes, cudaMemcpyHostToDevice, s);
+        int rc;
+        if ((rc = t_src.reserve(bytes)) || (rc = t_dst.reserve(bytes))) return rc;
+        DVO_CUDA(cudaMemcpyAsync(t_src, src, bytes, cudaMemcpyHostToDevice, s));
         d_src = t_src; d_dst = t_dst;
     }
     dim3 grid((unsigned)(((size_t)width * height + 255) / 256), (unsigned)count);
@@ -75,7 +75,6 @@ extern "C" int dvo_undistort(const void* src, void* dst, int width, int height, 
     if (mem != DVO_MEM_DEVICE) {
         if (e == cudaSuccess) e = cudaMemcpyAsync(dst, t_dst, bytes, cudaMemcpyDeviceToHost, s);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        cudaFree(t_src); cudaFree(t_dst);
     }
     if (e != cudaSuccess) { dvo_set_error("dvo_undistort: %s", cudaGetErrorString(e)); return DVO_ERR_CUDA; }
     return DVO_OK;

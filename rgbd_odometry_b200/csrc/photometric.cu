@@ -40,13 +40,13 @@ struct PhState {
 struct dvo_photo_ctx {
     dvo_photo_config cfg; PhGeom g; PhCam K; bool haveK;
     cudaStream_t own_stream, stream;
-    uint8_t* bgr[2];      // full resolution, [Bmax][H][W][3]
-    uint8_t* gray[2];     // AREA pyramid of the full-resolution gray
-    uint16_t* depth[2];   // AREA pyramid of depth (now: stored for API completeness)
-    int* winner;          // [Bmax][P0]: per target cell the winning source pixel as (column << 16) | row, -1 = hole
-    double* partial;      // [Bmax][maxblk][PH_NACC]
-    double* A;            // [Bmax][L][36]   J^T J of the reference frame
-    PhState* st;          // [Bmax]
+    DevBuf<uint8_t> bgr[2];      // full resolution, [Bmax][H][W][3]
+    DevBuf<uint8_t> gray[2];     // AREA pyramid of the full-resolution gray
+    DevBuf<uint16_t> depth[2];   // AREA pyramid of depth (now: stored for API completeness)
+    DevBuf<int> winner;          // [Bmax][P0]: per target cell the winning source pixel as (column << 16) | row, -1 = hole
+    DevBuf<double> partial;      // [Bmax][maxblk][PH_NACC]
+    DevBuf<double> A;            // [Bmax][L][36]   J^T J of the reference frame
+    DevBuf<PhState> st;          // [Bmax]
     int maxblk;
     long long launches;
 };
@@ -506,11 +506,6 @@ PhArgs ph_args(dvo_photo_ctx* c, int level, int first, int compat, double huber_
     a.nblk = nblk; a.maxblk = c->maxblk; a.huber_k = huber_k; a.lambda0 = lambda0; a.reset_winner = 0;
     return a;
 }
-template <typename T> int ph_alloc(T** p, size_t n) {
-    cudaError_t e = cudaMalloc((void**)p, (n ? n : 1) * sizeof(T));
-    if (e != cudaSuccess) { dvo_set_error("cudaMalloc(%zu bytes) failed: %s", n * sizeof(T), cudaGetErrorString(e)); return DVO_ERR_NOMEM; }
-    return DVO_OK;
-}
 }  // namespace
 
 extern "C" {
@@ -544,7 +539,6 @@ int dvo_photo_create(const dvo_photo_config* cfg, dvo_photo_ctx** out) {
     DVO_CUDA(cudaSetDevice(cfg->device));
     dvo_photo_ctx* c = new (std::nothrow) dvo_photo_ctx();
     if (!c) return DVO_ERR_NOMEM;
-    memset(c, 0, sizeof(*c));
     c->cfg = *cfg;
     PhGeom& g = c->g; g.L = cfg->levels; g.Bmax = cfg->max_batch; g.W = cfg->width; g.H = cfg->height;
     long long acc = 0;
@@ -556,8 +550,8 @@ int dvo_photo_create(const dvo_photo_config* cfg, dvo_photo_ctx** out) {
     const size_t B = g.Bmax, P0 = g.P[0];
     int rc = DVO_OK;
     auto A = [&](int r) { if (rc == DVO_OK) rc = r; };
-    for (int f = 0; f < 2; ++f) { A(ph_alloc(&c->bgr[f], B * P0 * 3)); A(ph_alloc(&c->gray[f], (size_t)g.total)); A(ph_alloc(&c->depth[f], (size_t)g.total)); }
-    A(ph_alloc(&c->winner, B * P0)); A(ph_alloc(&c->partial, B * c->maxblk * PH_NACC)); A(ph_alloc(&c->A, B * g.L * 36)); A(ph_alloc(&c->st, B));
+    for (int f = 0; f < 2; ++f) { A(c->bgr[f].reserve(B * P0 * 3)); A(c->gray[f].reserve((size_t)g.total)); A(c->depth[f].reserve((size_t)g.total)); }
+    A(c->winner.reserve(B * P0)); A(c->partial.reserve(B * c->maxblk * PH_NACC)); A(c->A.reserve(B * g.L * 36)); A(c->st.reserve(B));
     if (rc != DVO_OK) { dvo_photo_destroy(c); return rc; }
     PH_CREATE_CUDA(cudaMemsetAsync(c->st, 0, sizeof(PhState) * B, c->stream));
     PH_CREATE_CUDA(cudaMemsetAsync(c->A, 0, sizeof(double) * B * g.L * 36, c->stream));
@@ -571,8 +565,6 @@ int dvo_photo_destroy(dvo_photo_ctx* c) {
     if (!c) return DVO_OK;
     cudaSetDevice(c->cfg.device);
     if (c->own_stream) cudaStreamSynchronize(c->own_stream);
-    for (int f = 0; f < 2; ++f) { cudaFree(c->bgr[f]); cudaFree(c->gray[f]); cudaFree(c->depth[f]); }
-    cudaFree(c->winner); cudaFree(c->partial); cudaFree(c->A); cudaFree(c->st);
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
     delete c;
     return DVO_OK;
@@ -638,17 +630,13 @@ int dvo_photo_set_pose(dvo_photo_ctx* c, int first, int count, const double* R9T
         DVO_CUDA(cudaGetLastError());
         return DVO_OK;
     }
-    double* d = nullptr;
-    DVO_CUDA(cudaMalloc((void**)&d, sizeof(double) * 12 * count));
-    cudaError_t e = cudaMemcpyAsync(d, R9T3, sizeof(double) * 12 * count, cudaMemcpyHostToDevice, c->stream);
-    if (e == cudaSuccess) {
-        ph_init_state_kernel<<<(count + 127) / 128, 128, 0, c->stream>>>(c->st, first, count, d, 0.0);
-        c->launches++;
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(d);                                   // released on every path
-    DVO_CUDA(e);
+    DevBuf<double> d;
+    if (const int rc = d.reserve(12 * (size_t)count)) return rc;
+    DVO_CUDA(cudaMemcpyAsync(d, R9T3, sizeof(double) * 12 * count, cudaMemcpyHostToDevice, c->stream));
+    ph_init_state_kernel<<<(count + 127) / 128, 128, 0, c->stream>>>(c->st, first, count, d, 0.0);
+    c->launches++;
+    DVO_CUDA(cudaGetLastError());
+    DVO_CUDA(cudaStreamSynchronize(c->stream));
     return DVO_OK;
 }
 
@@ -707,34 +695,31 @@ int dvo_photo_get_level(dvo_photo_ctx* c, int slot, int frame, int level, int wh
         return DVO_OK;
     }
     // colour level (im_r_color): INTER_AREA of the full-resolution BGR, built on demand
-    uint8_t* d_bgr = nullptr;
+    DevBuf<uint8_t> d_bgr;
     const bool need_bgr = (which == DVO_PHOTO_BGR || which == DVO_PHOTO_BLUEVALS || which == DVO_PHOTO_GREENVALS || which == DVO_PHOTO_REDVALS);
     if (need_bgr) {
-        DVO_CUDA(cudaMalloc((void**)&d_bgr, P * 3));
+        if (const int rc = d_bgr.reserve(P * 3)) return rc;
         const uint8_t* src = c->bgr[frame] + (size_t)slot * g.P[0] * 3;
         if (level == 0) DVO_CUDA(cudaMemcpyAsync(d_bgr, src, P * 3, cudaMemcpyDeviceToDevice, c->stream));
         else { ph_area_kernel<uint8_t, 3><<<dim3((unsigned)((P + 255) / 256), 1), 256, 0, c->stream>>>(src, d_bgr, g.W, g.H, level, 0, 0); c->launches++; }
         if (which == DVO_PHOTO_BGR) {
-            int rc = DVO_OK;
-            if (bytes < P * 3) { dvo_set_error("dvo_photo_get_level: destination too small"); rc = DVO_ERR_ARG; }
-            else { cudaMemcpyAsync(dst, d_bgr, P * 3, cudaMemcpyDeviceToHost, c->stream); if (cudaStreamSynchronize(c->stream) != cudaSuccess) rc = DVO_ERR_CUDA; }
-            cudaFree(d_bgr);
-            return rc;
+            if (bytes < P * 3) { dvo_set_error("dvo_photo_get_level: destination too small"); return DVO_ERR_ARG; }
+            DVO_CUDA(cudaMemcpyAsync(dst, d_bgr, P * 3, cudaMemcpyDeviceToHost, c->stream));
+            DVO_CUDA(cudaStreamSynchronize(c->stream));
+            return DVO_OK;
         }
     }
-    if (!c->haveK) { cudaFree(d_bgr); dvo_set_error("dvo_photo_get_level: intrinsics not set"); return DVO_ERR_STATE; }
-    if (frame != DVO_FRAME_REF) { cudaFree(d_bgr); dvo_set_error("dvo_photo_get_level: X/Y/Z/J/colour arrays exist for the reference frame only"); return DVO_ERR_ARG; }
+    if (!c->haveK) { dvo_set_error("dvo_photo_get_level: intrinsics not set"); return DVO_ERR_STATE; }
+    if (frame != DVO_FRAME_REF) { dvo_set_error("dvo_photo_get_level: X/Y/Z/J/colour arrays exist for the reference frame only"); return DVO_ERR_ARG; }
     const size_t n = (which == DVO_PHOTO_J) ? P * 6 : P;
-    if (bytes < n * sizeof(double)) { cudaFree(d_bgr); dvo_set_error("dvo_photo_get_level: destination too small"); return DVO_ERR_ARG; }
-    double* d_out = nullptr;
-    DVO_CUDA(cudaMalloc((void**)&d_out, n * sizeof(double)));
+    if (bytes < n * sizeof(double)) { dvo_set_error("dvo_photo_get_level: destination too small"); return DVO_ERR_ARG; }
+    DevBuf<double> d_out;
+    if (const int rc = d_out.reserve(n)) return rc;
     PhArgs a = ph_args(c, level, slot, compat, 0.0, 0.0);
     ph_materialize_kernel<<<(unsigned)((P + 255) / 256), 256, 0, c->stream>>>(a, which, d_bgr, d_out);
     c->launches++;
-    cudaError_t e = cudaMemcpyAsync(dst, d_out, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(d_out); cudaFree(d_bgr);
-    if (e != cudaSuccess) { dvo_set_error("dvo_photo_get_level: %s", cudaGetErrorString(e)); return DVO_ERR_CUDA; }
+    DVO_CUDA(cudaMemcpyAsync(dst, d_out, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    DVO_CUDA(cudaStreamSynchronize(c->stream));
     return DVO_OK;
 }
 
@@ -780,15 +765,14 @@ int dvo_photo_eval(dvo_photo_ctx* c, int slot, int level, const double* R9T3, in
     DVO_CUDA(cudaMemcpyAsync(part.data(), c->partial + (size_t)slot * c->maxblk * PH_NACC, sizeof(double) * part.size(), cudaMemcpyDeviceToHost, c->stream));
     PhState st;
     DVO_CUDA(cudaMemcpyAsync(&st, c->st + slot, sizeof(PhState), cudaMemcpyDeviceToHost, c->stream));
-    double* d_cv = nullptr;
+    DevBuf<double> d_cv;
     if (canvas) {
-        DVO_CUDA(cudaMalloc((void**)&d_cv, sizeof(double) * a.P));
+        if ((rc = d_cv.reserve(a.P))) return rc;
         ph_canvas_kernel<<<(a.P + 255) / 256, 256, 0, c->stream>>>(a, d_cv);
         c->launches++;
         DVO_CUDA(cudaMemcpyAsync(canvas, d_cv, sizeof(double) * a.P, cudaMemcpyDeviceToHost, c->stream));
     }
     DVO_CUDA(cudaStreamSynchronize(c->stream));
-    cudaFree(d_cv);
     double tot[PH_NACC];
     for (int k = 0; k < PH_NACC; ++k) { double v = 0.0; for (int j = 0; j < a.nblk; ++j) v += part[(size_t)j * PH_NACC + k]; tot[k] = v; }
     if (b6) memcpy(b6, tot, sizeof(double) * 6);

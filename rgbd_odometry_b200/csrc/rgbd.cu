@@ -33,14 +33,14 @@ struct RgState { double T[16]; dvo_rgbd_info info; };
 struct dvo_rgbd_ctx {
     dvo_rgbd_config cfg; RgGeom g; RgCam K; bool haveK;
     cudaStream_t own_stream, stream;
-    uint8_t* bgr;         // staging: one frame set, [Bmax][H][W][3]
-    uint16_t* depth_in;   // staging: [Bmax][H][W]
-    uint8_t* gray[2];     // NEAREST pyramid of BGR2GRAY(full), level-major
-    uint16_t* depth[2];
-    double* A;            // [Bmax][L][36]
-    int* npts;            // [Bmax][L]
-    RgState* st;          // [Bmax]
-    double* pose_stage;   // [Bmax][16] device staging for dvo_rgbd_set_pose
+    DevBuf<uint8_t> bgr;         // staging: one frame set, [Bmax][H][W][3]
+    DevBuf<uint16_t> depth_in;   // staging: [Bmax][H][W]
+    DevBuf<uint8_t> gray[2];     // NEAREST pyramid of BGR2GRAY(full), level-major
+    DevBuf<uint16_t> depth[2];
+    DevBuf<double> A;            // [Bmax][L][36]
+    DevBuf<int> npts;            // [Bmax][L]
+    DevBuf<RgState> st;          // [Bmax]
+    DevBuf<double> pose_stage;   // [Bmax][16] device staging for dvo_rgbd_set_pose
     long long launches;
 };
 
@@ -337,7 +337,6 @@ __global__ void rg_set_pose_kernel(RgState* st, int first, int count, const doub
 // ------------------------------------------------------------------------------------------------------
 namespace {
 bool rg_range_ok(dvo_rgbd_ctx* c, int first, int count) { return c && first >= 0 && count >= 0 && first + count <= c->cfg.max_batch; }
-template <typename T> cudaError_t rg_alloc(T** p, size_t n) { return cudaMalloc((void**)p, sizeof(T) * (n ? n : 1)); }
 int rg_level_dim(int dim, int level) { return (int)nearbyint((double)dim * ldexp(1.0, -level)); }     // cv::resize: cvRound(dim * scale)
 }  // namespace
 
@@ -351,8 +350,7 @@ int dvo_rgbd_create(const dvo_rgbd_config* cfg, dvo_rgbd_ctx** out) {
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { dvo_set_error("dvo_rgbd_create: no usable CUDA device (there is no CPU fallback)"); return DVO_ERR_CUDA; }
     DVO_CUDA(cudaSetDevice(cfg->device));
     dvo_rgbd_ctx* c = new (std::nothrow) dvo_rgbd_ctx();
-    if (!c) return DVO_ERR_ARG;
-    memset(c, 0, sizeof(*c));
+    if (!c) return DVO_ERR_NOMEM;
     c->cfg = *cfg;
     RgGeom& g = c->g;
     g.L = cfg->levels; g.Bmax = cfg->max_batch; g.W = cfg->width; g.H = cfg->height;
@@ -362,13 +360,14 @@ int dvo_rgbd_create(const dvo_rgbd_config* cfg, dvo_rgbd_ctx** out) {
     cudaError_t e = cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking);
     c->stream = c->own_stream;
     const size_t B = (size_t)g.Bmax, P0 = (size_t)g.P[0];
-    if (e == cudaSuccess) e = rg_alloc(&c->bgr, B * P0 * 3);
-    if (e == cudaSuccess) e = rg_alloc(&c->depth_in, B * P0);
-    for (int f = 0; f < 2 && e == cudaSuccess; ++f) { e = rg_alloc(&c->gray[f], (size_t)g.total); if (e == cudaSuccess) e = rg_alloc(&c->depth[f], (size_t)g.total); }
-    if (e == cudaSuccess) e = rg_alloc(&c->A, B * g.L * 36);
-    if (e == cudaSuccess) e = rg_alloc(&c->npts, B * g.L);
-    if (e == cudaSuccess) e = rg_alloc(&c->st, B);
-    if (e == cudaSuccess) e = rg_alloc(&c->pose_stage, B * 16);
+    int rc = DVO_OK;
+    auto A = [&](int r) { if (rc == DVO_OK) rc = r; };
+    if (e == cudaSuccess) {
+        A(c->bgr.reserve(B * P0 * 3)); A(c->depth_in.reserve(B * P0));
+        for (int f = 0; f < 2; ++f) { A(c->gray[f].reserve((size_t)g.total)); A(c->depth[f].reserve((size_t)g.total)); }
+        A(c->A.reserve(B * g.L * 36)); A(c->npts.reserve(B * g.L)); A(c->st.reserve(B)); A(c->pose_stage.reserve(B * 16));
+        if (rc) { dvo_rgbd_destroy(c); return rc; }
+    }
     if (e == cudaSuccess) e = cudaMemsetAsync(c->npts, 0, sizeof(int) * B * g.L, c->stream);
     if (e == cudaSuccess) e = cudaMemsetAsync(c->st, 0, sizeof(RgState) * B, c->stream);
     if (e == cudaSuccess) e = cudaMemsetAsync(c->A, 0, sizeof(double) * B * g.L * 36, c->stream);
@@ -379,9 +378,6 @@ int dvo_rgbd_create(const dvo_rgbd_config* cfg, dvo_rgbd_ctx** out) {
 
 int dvo_rgbd_destroy(dvo_rgbd_ctx* c) {
     if (!c) return DVO_OK;
-    cudaFree(c->bgr); cudaFree(c->depth_in);
-    for (int f = 0; f < 2; ++f) { cudaFree(c->gray[f]); cudaFree(c->depth[f]); }
-    cudaFree(c->A); cudaFree(c->npts); cudaFree(c->st); cudaFree(c->pose_stage);
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
     delete c;
     return DVO_OK;
@@ -499,13 +495,10 @@ int dvo_rgbd_eval(dvo_rgbd_ctx* c, int slot, int level, const double* T16, int g
     if (!c->haveK) { dvo_set_error("dvo_rgbd_eval: intrinsics not set"); return DVO_ERR_STATE; }
     const int rows = c->g.h[level], cols = c->g.w[level];
     const size_t P = (size_t)rows * cols;
-    uint8_t* d_sel = nullptr; double* d_J = nullptr; double* d_eps = nullptr; int* d_uv = nullptr; double* d_T = nullptr;
-    cudaError_t e = cudaMalloc((void**)&d_sel, P);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_J, sizeof(double) * 6 * P);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_eps, sizeof(double) * P);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_uv, sizeof(int) * 2 * P);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_T, sizeof(double) * 16);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_T, T16, sizeof(double) * 16, cudaMemcpyHostToDevice, c->stream);
+    DevBuf<uint8_t> d_sel; DevBuf<double> d_J, d_eps, d_T; DevBuf<int> d_uv;
+    int rc;
+    if ((rc = d_sel.reserve(P)) || (rc = d_J.reserve(6 * P)) || (rc = d_eps.reserve(P)) || (rc = d_uv.reserve(2 * P)) || (rc = d_T.reserve(16))) return rc;
+    cudaError_t e = cudaMemcpyAsync(d_T, T16, sizeof(double) * 16, cudaMemcpyHostToDevice, c->stream);
     std::vector<uint8_t> h_sel(P); std::vector<double> h_J(6 * P), h_eps(P); std::vector<int> h_uv(2 * P);
     if (e == cudaSuccess) {
         rg_eval_kernel<<<(unsigned)((P + 255) / 256), 256, 0, c->stream>>>(c->g, c->K, c->gray[0], c->depth[0], c->gray[1], slot, level, d_T, gradient_threshold,
@@ -518,7 +511,6 @@ int dvo_rgbd_eval(dvo_rgbd_ctx* c, int slot, int level, const double* T16, int g
     if (e == cudaSuccess) e = cudaMemcpyAsync(h_eps.data(), d_eps, sizeof(double) * P, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(h_uv.data(), d_uv, sizeof(int) * 2 * P, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(d_sel); cudaFree(d_J); cudaFree(d_eps); cudaFree(d_uv); cudaFree(d_T);
     if (e != cudaSuccess) { dvo_set_error("dvo_rgbd_eval: %s", cudaGetErrorString(e)); return DVO_ERR_CUDA; }
     int k = 0, seen = 0; double ss = 0.0, b[6] = {0, 0, 0, 0, 0, 0};
     for (int j = 0; j < cols; ++j)
