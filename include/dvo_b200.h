@@ -284,6 +284,47 @@ int dvo_run_sequences_entropy(dvo_ctx* ctx, int nseq, int nframes, const uint8_t
                               double* rel_poses, int* kind, int* reason, double* global_poses, double* rel_cov,
                               double* global_cov, double* entropy_ratio);
 
+/* ---- windowed pose-graph optimisation (the back end DVO-SLAM puts behind this front end; Kerl, Sturm, Cremers, IROS 2013) ----
+ * ngraphs independent graphs of the same shape: nnodes nodes and nedges edges each.  Node i has a global pose G_i (12-double
+ * record; composition as dvo_gop_compose: G_a G_b = (R_a R_b, T_a + R_a T_b)); node 0 is held at its input pose (the gauge).
+ * Edge e = (a, b, Z, Sigma): Z the relative pose of the pair (reference a, now b) as dvo_align_pairs returns it (noise-free:
+ * G_b = G_a Z), Sigma its 6x6 covariance as cov36 (tangent (rho, omega), T <- T exp(psi)), information Omega = Sigma^-1.
+ *   r_e = log(Z^-1 G_a^-1 G_b) (se3 log, (rho, omega)),  F = 1/2 sum_e r_e^T Omega_e r_e,
+ *   right perturbations G <- G exp(d):  dr/dd_b = Jinv(r),  dr/dd_a = -Jinv(r) Ad(G_b^-1 G_a),
+ *   Jinv(r) = I + 1/2 ad(r), ad(rho, omega) = [[omega x, rho x], [0, omega x]], Ad(R, t) = [[R, [t]x R], [0, R]] (first-order
+ *   inverse Jacobian: it changes the path of the iteration; at a zero-residual optimum it changes nothing).
+ * Every edge needs 1 <= |a - b| <= max_lag <= DVO_PGO_MAX_LAG: windowed odometry, forward and backward pairs; loop closures
+ * are out of scope.  An edge whose Sigma has a non-finite entry or is not positive definite (its lower triangle is factored)
+ * is skipped, so pairs dvo_align_pairs flagged (NaN covariance) drop out on their own.
+ * Levenberg-Marquardt with Marquardt damping H + lambda diag(H): an iteration is one damped solve and one cost evaluation; a
+ * step is accepted iff the cost decreases (then lambda /= 10, else lambda *= 10).  The loop stops after max_iterations, after
+ * an accepted step whose relative decrease (F - F') / F is below rel_tol, or when lambda exceeds DVO_PGO_LAMBDA_MAX.
+ * node_cov36 (optional): the 6x6 diagonal blocks of H^-1 with lambda = 0 at the returned poses, same tangent and convention as
+ * global_cov of dvo_run_sequences_cov; node 0 gets zeros (it anchors the graph).
+ * mem = DVO_MEM_HOST: a bad edge index returns DVO_ERR_ARG before anything is launched; returns when the outputs are filled.
+ * DVO_MEM_DEVICE: the device checks the indices (status bit 0); asynchronous on the context stream.  A graph with status bit
+ * 0 or 1 keeps its input poses and gets NaN marginals.  Reads no frame data: works on any context.  One kernel launch; a
+ * graph's results are bit-identical whatever ngraphs, its position in the batch and mem. */
+#define DVO_PGO_MAX_LAG 8
+#define DVO_PGO_LAMBDA_MAX 1e16
+typedef struct dvo_pgo_params {
+    int max_iterations;   /* damped solves, accepted or not (e.g. 100)          */
+    double lambda0;       /* initial Marquardt damping (e.g. 1e-4), > 0           */
+    double rel_tol;       /* stop after an accepted step with (F - F') / F < rel_tol (e.g. 1e-10) */
+} dvo_pgo_params;
+typedef struct dvo_pgo_info {
+    int status;       /* bit0 an edge index is out of range, a == b or |a-b| > max_lag (device indices); bit1 a node is not
+                         connected to node 0 through valid edges; bit2 H not positive definite at the returned poses (marginals NaN) */
+    int iterations, accepted, edges_used;
+    double cost_initial, cost_final;   /* F at the input and at the returned poses; NaN when status bit 0 or 1 is set */
+} dvo_pgo_info;
+int dvo_pose_graph_optimize(dvo_ctx* ctx, int ngraphs, int nnodes, int nedges, int max_lag,
+                            const int* edge_ref, const int* edge_now,     /* [ngraphs][nedges]       */
+                            const double* meas12, const double* cov36,    /* [ngraphs][nedges][12/36] */
+                            double* poses12,                              /* [ngraphs][nnodes][12], in: initial, out: optimised */
+                            const dvo_pgo_params* prm, double* node_cov36 /* optional [ngraphs][nnodes][36] */,
+                            dvo_pgo_info* info /* optional [ngraphs] */, int mem);
+
 /* ---- inspection (parity tests; not on the hot path) ---- */
 int dvo_level_dims(dvo_ctx* ctx, int level, int* w, int* h);
 int dvo_get_level_buffer(dvo_ctx* ctx, int slot, int frame, int level, int which, void* host_dst, size_t bytes);

@@ -43,6 +43,19 @@ class KeyframePolicy(C.Structure):
                 ("visible_ratio_thresh", C.c_float), ("min_reprojections", C.c_int)]
 
 
+class PgoParams(C.Structure):
+    """dvo_pgo_params: LM iteration cap (damped solves), initial Marquardt damping, relative-decrease stop."""
+    _fields_ = [("max_iterations", C.c_int), ("lambda0", C.c_double), ("rel_tol", C.c_double)]
+
+
+class PgoInfo(C.Structure):
+    """dvo_pgo_info: status bits (0 bad edge index, 1 not connected to node 0, 2 H not positive definite), counts, costs."""
+    _fields_ = [("status", C.c_int), ("iterations", C.c_int), ("accepted", C.c_int), ("edges_used", C.c_int),
+                ("cost_initial", C.c_double), ("cost_final", C.c_double)]
+
+
+PGO_MAX_LAG = 8
+
 RGBD_MAX_LEVELS = 5
 
 
@@ -68,7 +81,7 @@ SYMBOLS = [
     "dvo_set_initial_pose", "dvo_run", "dvo_process", "dvo_join", "dvo_join_stream", "dvo_get_poses", "dvo_align_batch", "dvo_level_dims", "dvo_get_level_buffer",
     "dvo_get_points", "dvo_eval_normal_equations", "dvo_eval_normal_equations_ex", "dvo_get_trace", "dvo_get_energies", "dvo_enable_timing", "dvo_get_stage_ms",
     "dvo_launch_count", "dvo_gop_compose", "dvo_run_sequences", "dvo_run_sequences_gated", "dvo_run_sequences_mem",
-    "dvo_pose_covariance", "dvo_run_sequences_cov", "dvo_run_sequences_entropy", "dvo_align_pairs",
+    "dvo_pose_covariance", "dvo_run_sequences_cov", "dvo_run_sequences_entropy", "dvo_align_pairs", "dvo_pose_graph_optimize",
     "dvo_photo_create", "dvo_photo_destroy", "dvo_photo_set_stream", "dvo_photo_synchronize", "dvo_photo_launch_count",
     "dvo_photo_set_intrinsics", "dvo_photo_set_frames", "dvo_photo_prepare_ref", "dvo_photo_set_pose", "dvo_photo_estimate",
     "dvo_photo_get_poses", "dvo_photo_get_level", "dvo_photo_get_A", "dvo_photo_eval", "dvo_photo_put_level",
@@ -142,6 +155,8 @@ def load(build_if_missing=True):
     lib.dvo_run_sequences_entropy.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(SolverParams),
                                               C.POINTER(KeyframePolicy), C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.dvo_pose_graph_optimize.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.POINTER(PgoParams), C.c_void_p, C.c_void_p, C.c_int]
     lib.dvo_photo_create.argtypes = [C.POINTER(PhotoConfig), C.POINTER(C.c_void_p)]
     lib.dvo_photo_destroy.argtypes = [C.c_void_p]
     lib.dvo_photo_set_stream.argtypes = [C.c_void_p, C.c_void_p]

@@ -4,7 +4,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import Config, CovInfo, KeyframePolicy, PairInfo, SolverParams, check
+from ._lib import Config, CovInfo, KeyframePolicy, PairInfo, PgoInfo, PgoParams, SolverParams, check
 
 SUBGRAD_REF, GN, LM = 0, 1, 2
 JAC_REFERENCE, JAC_EXACT = 0, 1
@@ -46,7 +46,7 @@ def undistort(img, K, D):
 
 
 def records(raw, cls):
-    """ctypes array of `cls` (PairInfo, CovInfo) from the raw records align_pairs(device=True) returns as a uint8 CUDA tensor."""
+    """ctypes array of `cls` (PairInfo, CovInfo, PgoInfo) from the raw records align_pairs(device=True) returns as a uint8 CUDA tensor."""
     return (cls * raw.shape[0]).from_buffer_copy(raw.cpu().numpy().tobytes())
 
 
@@ -360,3 +360,41 @@ class BatchAligner:
         out = np.empty((nseq, nframes, 19), np.float64)
         check(self.lib.dvo_gop_compose(self.h, nseq, nframes, _ptr(kind), _ptr(rel), _ptr(out), MEM_HOST), "dvo_gop_compose")
         return out
+
+    def optimize_pose_graph(self, edge_ref, edge_now, meas, cov, poses0, max_lag, max_iterations=100, lambda0=1e-4, rel_tol=1e-10,
+                            marginals=False, device=False):
+        """dvo_pose_graph_optimize: G graphs of N nodes and E edges each; edge e of graph k constrains G_b = G_a Z with covariance
+        cov, a = edge_ref[k, e], b = edge_now[k, e], 1 <= |a - b| <= max_lag <= 8; node 0 stays at its input pose.
+        Shapes: edge_ref / edge_now (G, E), meas (G, E, 12), cov (G, E, 6, 6), poses0 (G, N, 12).  Returns (poses, info) or, with
+        marginals=True, (poses, info, node_cov (G, N, 6, 6)).  Host (device=False): numpy arrays and a ctypes array of PgoInfo;
+        bad edge indices raise.  device=True: int32 / float64 CUDA tensors in, CUDA tensors out (info as raw uint8 records for
+        `records(raw, PgoInfo)`), asynchronous on the context stream; bad indices give info status bit 0."""
+        prm = PgoParams(int(max_iterations), float(lambda0), float(rel_tol))
+        if device:
+            import torch
+            G, E = int(edge_ref.shape[0]), int(edge_ref.shape[1])
+            N = int(poses0.shape[1])
+            dev = poses0.device
+            poses = poses0.detach().clone().contiguous()
+            info = torch.empty((G, C.sizeof(PgoInfo)), dtype=torch.uint8, device=dev)
+            ncov = torch.empty((G, N, 6, 6), dtype=torch.float64, device=dev) if marginals else None
+            ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())  # noqa: E731
+            check(self.lib.dvo_pose_graph_optimize(self.h, G, N, E, int(max_lag), ptr(edge_ref.contiguous()), ptr(edge_now.contiguous()),
+                                                   ptr(meas.contiguous()), ptr(cov.contiguous()), ptr(poses), C.byref(prm), ptr(ncov),
+                                                   ptr(info), MEM_DEVICE), "dvo_pose_graph_optimize")
+        else:
+            edge_ref = np.ascontiguousarray(edge_ref, np.int32)
+            edge_now = np.ascontiguousarray(edge_now, np.int32)
+            G, E = edge_ref.shape
+            poses = np.array(poses0, np.float64, order="C", copy=True)
+            N = poses.shape[1]
+            if edge_now.shape != (G, E) or poses.shape != (G, N, 12):
+                raise ValueError("edge_now must be (G, E) like edge_ref and poses0 (G, N, 12)")
+            meas = np.ascontiguousarray(meas, np.float64).reshape(G, E, 12)
+            cov = np.ascontiguousarray(cov, np.float64).reshape(G, E, 6, 6)
+            info = (PgoInfo * max(G, 1))()
+            ncov = np.empty((G, N, 6, 6), np.float64) if marginals else None
+            check(self.lib.dvo_pose_graph_optimize(self.h, G, N, E, int(max_lag), _ptr(edge_ref), _ptr(edge_now), _ptr(meas), _ptr(cov),
+                                                   _ptr(poses), C.byref(prm), _ptr(ncov), C.cast(info, C.c_void_p), MEM_HOST),
+                  "dvo_pose_graph_optimize")
+        return (poses, info, ncov) if marginals else (poses, info)

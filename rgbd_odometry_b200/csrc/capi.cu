@@ -968,6 +968,59 @@ int dvo_gop_compose(dvo_ctx* c, int nseq, int nframes, const int* kind, const do
     return DVO_OK;
 }
 
+int dvo_pose_graph_optimize(dvo_ctx* c, int ngraphs, int nnodes, int nedges, int max_lag, const int* edge_ref, const int* edge_now,
+                            const double* meas12, const double* cov36, double* poses12, const dvo_pgo_params* prm, double* node_cov36,
+                            dvo_pgo_info* info, int mem) {
+    if (c) { const int jr = join_aux(c); if (jr) return jr; }
+    if (!c || ngraphs < 0 || nnodes < 2 || nedges < 0 || max_lag < 1 || max_lag > DVO_PGO_MAX_LAG || !poses12 || !prm ||
+        (nedges > 0 && (!edge_ref || !edge_now || !meas12 || !cov36)) || (mem != DVO_MEM_HOST && mem != DVO_MEM_DEVICE) ||
+        prm->max_iterations < 0 || !(prm->lambda0 > 0.0) || !(prm->rel_tol >= 0.0)) {
+        dvo_set_error("dvo_pose_graph_optimize: bad argument"); return DVO_ERR_ARG;
+    }
+    const size_t G = (size_t)ngraphs, E = (size_t)nedges, N = (size_t)nnodes;
+    if (mem == DVO_MEM_HOST)                             // device indices are checked by the kernel (status bit 0)
+        for (size_t k = 0; k < G * E; ++k) {
+            const int a = edge_ref[k], b = edge_now[k];
+            if (a < 0 || a >= nnodes || b < 0 || b >= nnodes || a == b || abs(a - b) > max_lag) {
+                dvo_set_error("dvo_pose_graph_optimize: graph %zu edge %zu joins nodes (%d, %d): outside [0, %d), equal, or more than %d apart",
+                              k / (E ? E : 1), k % (E ? E : 1), a, b, nnodes, max_lag);
+                return DVO_ERR_ARG;
+            }
+        }
+    if (ngraphs == 0) return DVO_OK;
+    size_t dbl = 0, ints = 0;
+    pgo_scratch_size(nnodes, nedges, max_lag, &dbl, &ints);
+    int rc = DVO_OK;
+    auto A = [&](int r) { if (rc == DVO_OK) rc = r; };
+    // growth replaces buffers work in flight may use
+    if (c->pgo_dscr.n < G * dbl || c->pgo_iscr.n < G * ints) DVO_CUDA(cudaStreamSynchronize(c->stream));
+    A(c->pgo_dscr.reserve(G * dbl)); A(c->pgo_iscr.reserve(G * ints));
+    if (rc) return rc;
+    if (mem == DVO_MEM_DEVICE)
+        return launch_pose_graph(c, ngraphs, nnodes, nedges, max_lag, edge_ref, edge_now, meas12, cov36, poses12, prm, node_cov36, info,
+                                 c->pgo_dscr, c->pgo_iscr);
+    if (c->pgo_ref.n < G * E || c->pgo_meas.n < 12 * G * E || c->pgo_cov.n < 36 * G * E || c->pgo_pose.n < 12 * G * N ||
+        (node_cov36 && c->pgo_ncov.n < 36 * G * N) || c->pgo_info.n < G)
+        DVO_CUDA(cudaStreamSynchronize(c->stream));
+    A(c->pgo_ref.reserve(G * E)); A(c->pgo_now.reserve(G * E)); A(c->pgo_meas.reserve(12 * G * E)); A(c->pgo_cov.reserve(36 * G * E));
+    A(c->pgo_pose.reserve(12 * G * N)); A(c->pgo_info.reserve(G));
+    if (node_cov36) A(c->pgo_ncov.reserve(36 * G * N));
+    if (rc) return rc;
+    DVO_CUDA(cudaMemcpyAsync(c->pgo_ref, edge_ref, sizeof(int) * G * E, cudaMemcpyHostToDevice, c->stream));
+    DVO_CUDA(cudaMemcpyAsync(c->pgo_now, edge_now, sizeof(int) * G * E, cudaMemcpyHostToDevice, c->stream));
+    DVO_CUDA(cudaMemcpyAsync(c->pgo_meas, meas12, sizeof(double) * 12 * G * E, cudaMemcpyHostToDevice, c->stream));
+    DVO_CUDA(cudaMemcpyAsync(c->pgo_cov, cov36, sizeof(double) * 36 * G * E, cudaMemcpyHostToDevice, c->stream));
+    DVO_CUDA(cudaMemcpyAsync(c->pgo_pose, poses12, sizeof(double) * 12 * G * N, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = launch_pose_graph(c, ngraphs, nnodes, nedges, max_lag, c->pgo_ref, c->pgo_now, c->pgo_meas, c->pgo_cov, c->pgo_pose, prm,
+                                node_cov36 ? c->pgo_ncov.get() : nullptr, c->pgo_info, c->pgo_dscr, c->pgo_iscr)))
+        return rc;
+    DVO_CUDA(cudaMemcpyAsync(poses12, c->pgo_pose, sizeof(double) * 12 * G * N, cudaMemcpyDeviceToHost, c->stream));
+    if (node_cov36) DVO_CUDA(cudaMemcpyAsync(node_cov36, c->pgo_ncov, sizeof(double) * 36 * G * N, cudaMemcpyDeviceToHost, c->stream));
+    if (info) DVO_CUDA(cudaMemcpyAsync(info, c->pgo_info, sizeof(dvo_pgo_info) * G, cudaMemcpyDeviceToHost, c->stream));
+    DVO_CUDA(cudaStreamSynchronize(c->stream));
+    return DVO_OK;
+}
+
 // ---- device-resident storage blobs (PyramidalStorageStruct keeps caller-provided level arrays on the device) ----
 struct dvo_blob { DevBuf<unsigned char> d; size_t bytes; int device; };
 

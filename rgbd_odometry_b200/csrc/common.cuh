@@ -135,6 +135,10 @@ struct dvo_ctx {
     // device staging of dvo_set_frames_raw with host buffers (allocated on first use)
     DevBuf<uint8_t> raw_bgr; DevBuf<float> raw_depth;
 
+    // dvo_pose_graph_optimize: per-graph scratch, and the device copies of host inputs / outputs, grown on demand
+    DevBuf<double> pgo_dscr; DevBuf<int> pgo_iscr;
+    DevBuf<int> pgo_ref, pgo_now; DevBuf<double> pgo_meas, pgo_cov, pgo_pose, pgo_ncov; DevBuf<dvo_pgo_info> pgo_info;
+
     bool timing;
     cudaEvent_t ev_a, ev_b;
     float stage_ms[DVO_STAGE_COUNT];
@@ -176,6 +180,11 @@ int launch_gop(dvo_ctx* c, int nseq, int nframes, const int* d_kind, const doubl
 int launch_promote(dvo_ctx* c, int first, int count);
 int launch_ingest_raw(dvo_ctx* c, int frame, int first, int count, const uint8_t* d_bgr, const float* d_depth_m);
 int launch_copy_bytes(dvo_ctx* c, void* dst, const void* src, size_t n);
+// pose-graph optimisation (posegraph.cu): per-graph scratch sizes in doubles / ints, and the one-CTA-per-graph launch on device arrays
+int pgo_scratch_size(int nnodes, int nedges, int max_lag, size_t* dbl, size_t* ints);
+int launch_pose_graph(dvo_ctx* c, int ngraphs, int nnodes, int nedges, int max_lag, const int* d_ref, const int* d_now, const double* d_meas,
+                      const double* d_cov, double* d_poses, const dvo_pgo_params* prm, double* d_node_cov, dvo_pgo_info* d_info, double* d_dscr,
+                      int* d_iscr);
 
 // ---- arithmetic policies for the per-point fp32 math ----
 // EXACT: one IEEE rounding per written operation, never contracted -> bit-identical to the oracle compiled with
