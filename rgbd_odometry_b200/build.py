@@ -53,7 +53,7 @@ def build_cuda(force=False, verbose=False):
         obj = os.path.join(OBJ_DIR, name[:-3] + ".o")
         objs.append(obj)
         if force or _stale(obj, [src] + deps):
-            extra = os.environ.get("DVO_NVCC_EXTRA", "").split()          # experiments only (e.g. -DDVO_SOLVE_DEPTH_SWEEP)
+            extra = os.environ.get("DVO_NVCC_EXTRA", "").split()          # experiments only (e.g. preprocess.cu's -DDVO_NMS_* knobs)
             cmd = [_nvcc()] + COMPILE_FLAGS + PER_FILE_FLAGS.get(name, []) + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", "-o", obj, src]
             subprocess.check_call(cmd, cwd=CSRC)
             relink = True

@@ -4,106 +4,11 @@
 // round trip.  Follows SolveDVO::runIterations (src/SolveDVO.cpp:619-1017), computeJacobianOfNowFrame
 // (:306-414) and getReprojectedEpsilons (:425-462); see SURVEY.md Appendix A for the restated arithmetic.
 #include "common.cuh"
+#include "se3.cuh"
 
 namespace {
 
 constexpr int EVAL_THREADS = 256;     // inspection kernel
-// compile-time experiment knobs (tools/solve_variants.sh rebuilds with -D...): measured per 1024 pairs, GN 10 it / SUBGRAD 50 it:
-//   escape path out of line + run-time weight mode 4.06 / 17.96 ms; escape path inline 4.07 / 17.43; + weight mode specialised 4.01 / 17.19
-#ifndef DVO_GN_THREADS_PER_SM
-#define DVO_GN_THREADS_PER_SM 512     // resident threads per SM the 29-accumulator kernel is compiled for (768 = 85 registers, spills)
-#endif
-#ifndef DVO_SOLVE_PIPE_GN
-#define DVO_SOLVE_PIPE_GN 4           // ring depth of the shipped configuration's sweep, 29-accumulator kernel (0 = register pipeline, one gather ahead)
-#endif
-#ifndef DVO_SOLVE_PIPE_SG
-#define DVO_SOLVE_PIPE_SG 2           // same, 8-accumulator (sub-gradient) kernel
-#endif
-
-#ifndef DVO_ESCAPE_INLINE
-#define DVO_ESCAPE_INLINE 1
-#endif
-#if DVO_ESCAPE_INLINE
-#define DVO_ESCAPE_ATTR __device__ __forceinline__
-#else
-#define DVO_ESCAPE_ATTR __device__ __noinline__
-#endif
-#ifndef DVO_WMODE_SPECIALIZE
-#define DVO_WMODE_SPECIALIZE 1
-#endif
-
-// ------------------------------------------------------------------ fp64 3x3 / SE(3) helpers (device)
-__device__ __forceinline__ void m3_mul(const double* A, const double* B, double* C) {
-    double r[9];
-#pragma unroll
-    for (int i = 0; i < 3; ++i)
-#pragma unroll
-        for (int j = 0; j < 3; ++j) r[3 * i + j] = A[3 * i] * B[j] + A[3 * i + 1] * B[3 + j] + A[3 * i + 2] * B[6 + j];
-#pragma unroll
-    for (int i = 0; i < 9; ++i) C[i] = r[i];
-}
-__device__ __forceinline__ void m3_vec(const double* A, const double* v, double* o) {
-    const double a = A[0] * v[0] + A[1] * v[1] + A[2] * v[2];
-    const double b = A[3] * v[0] + A[4] * v[1] + A[5] * v[2];
-    const double c = A[6] * v[0] + A[7] * v[1] + A[8] * v[2];
-    o[0] = a; o[1] = b; o[2] = c;
-}
-
-// SE(3) exponential, tangent = (upsilon, omega), translation first (Sophus::SE3d::exp, src/SolveDVO.cpp:905).
-__device__ __forceinline__ void se3_exp_dev(const double* psi, double* R, double* t) {
-    const double wx = psi[3], wy = psi[4], wz = psi[5];
-    const double th2 = wx * wx + wy * wy + wz * wz, th = sqrt(th2);
-    double A, B, C;
-    if (th < 1e-5) { A = 1.0 - th2 / 6.0; B = 0.5 - th2 / 24.0; C = 1.0 / 6.0 - th2 / 120.0; }
-    else { double s, c; sincos(th, &s, &c); const double ith = 1.0 / th, ith2 = ith * ith; A = s * ith; B = (1.0 - c) * ith2; C = (th - s) * (ith2 * ith); }
-    const double O[9] = {0, -wz, wy, wz, 0, -wx, -wy, wx, 0};
-    double O2[9]; m3_mul(O, O, O2);
-    double V[9];
-#pragma unroll
-    for (int i = 0; i < 9; ++i) {
-        const double I = (i % 4 == 0) ? 1.0 : 0.0;
-        R[i] = I + A * O[i] + B * O2[i];
-        V[i] = I + B * O[i] + C * O2[i];
-    }
-    m3_vec(V, psi, t);
-}
-
-// rotation matrix -> unit quaternion (x,y,z,w), Shepperd's branches
-__device__ __forceinline__ void rot_to_quat_dev(const double* R, double* q) {
-    const double tr = R[0] + R[4] + R[8];
-    if (tr > 0) {
-        double s = sqrt(tr + 1.0); q[3] = 0.5 * s; s = 0.5 / s;
-        q[0] = (R[7] - R[5]) * s; q[1] = (R[2] - R[6]) * s; q[2] = (R[3] - R[1]) * s;
-    } else {
-        int i = 0; if (R[4] > R[0]) i = 1; if (R[8] > R[4 * i]) i = 2;
-        const int j = (i + 1) % 3, k = (j + 1) % 3;
-        double s = sqrt(R[4 * i] - R[4 * j] - R[4 * k] + 1.0);
-        q[i] = 0.5 * s; s = 0.5 / s;
-        q[3] = (R[3 * k + j] - R[3 * j + k]) * s;
-        q[j] = (R[3 * j + i] + R[3 * i + j]) * s;
-        q[k] = (R[3 * k + i] + R[3 * i + k]) * s;
-    }
-}
-
-// SE(3) logarithm (Sophus::SE3d::log of setRotationMatrix(cR), translation cT; src/SolveDVO.cpp:736-739)
-__device__ __forceinline__ void se3_log_dev(const double* R, const double* t, double* psi) {
-    double q[4]; rot_to_quat_dev(R, q);
-    const double qn = sqrt(q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3]);
-    double sgn = (q[3] < 0 ? -1.0 : 1.0) / qn;
-    const double x = q[0] * sgn, y = q[1] * sgn, z = q[2] * sgn, w = q[3] * sgn;
-    const double n2 = x * x + y * y + z * z, n = sqrt(n2);
-    const double k = (n < 1e-10) ? (2.0 / w - 2.0 * n2 / (3.0 * w * w * w)) : (2.0 * atan2(n, w) / n);
-    const double ox = k * x, oy = k * y, oz = k * z;
-    const double th2 = ox * ox + oy * oy + oz * oz, th = sqrt(th2);
-    const double O[9] = {0, -oz, oy, oz, 0, -ox, -oy, ox, 0};
-    double O2[9]; m3_mul(O, O, O2);
-    const double D = (th < 1e-5) ? (1.0 / 12.0 + th2 / 720.0) : ((1.0 - th * sin(th) / (2.0 * (1.0 - cos(th)))) / th2);
-    double Vi[9];
-#pragma unroll
-    for (int i = 0; i < 9; ++i) Vi[i] = ((i % 4 == 0) ? 1.0 : 0.0) - 0.5 * O[i] + D * O2[i];
-    m3_vec(Vi, t, psi);
-    psi[3] = ox; psi[4] = oy; psi[5] = oz;
-}
 
 // SolveDVO::rotationize (src/SolveDVO.cpp:1269-1282) returns U V^T of the SVD, i.e. the orthogonal polar factor.
 // Computed here by Newton's iteration X <- (X + X^-T)/2, which converges quadratically; the input is within
@@ -208,7 +113,7 @@ __device__ __forceinline__ bool unpack_texel(const uint2 t, Stencil& s) {
     s.d = s.c + ((int)(t.y << 2) >> 22);
     return (int)t.x >= 0;
 }
-DVO_ESCAPE_ATTR void stencil_from_d2(const int32_t* __restrict__ d2, int w, int h, int x, int y, Stencil& s) {
+__device__ __forceinline__ void stencil_from_d2(const int32_t* __restrict__ d2, int w, int h, int x, int y, Stencil& s) {
     const int32_t* d = d2 + y * w + x;
     s.c = __ldg(d);
     const bool bx = (x == 0 || x == w - 1), by = (y == 0 || y == h - 1);
@@ -249,6 +154,30 @@ __device__ __forceinline__ LevelCam make_level_cam(const Intr& K, const PyrGeom&
     cam.M11_lo = __fdiv_rn(cam.M11, __int_as_float(DVO_Z_BELOW_ONE));
     cam.tw = geom.tw[l];
     return cam;
+}
+
+// The frames every solver kernel reads: the reference slots' edge points and the now slots' distance transforms.
+struct FrameArgs {
+    PyrGeom geom; Intr K;
+    const float *X, *Y, *Z; const int* npts; const unsigned* nedge_now;
+    const uint2* tex8; const int32_t* d2; const unsigned* maxd2;
+};
+
+// Level l of the reference points of slot rb against the now frame of slot nb.  Builds the now frame's lookup tables into
+// lut; they are visible after the caller's next barrier.
+struct LevelSrc { const float *X, *Y, *Z; LevelCam cam; TexSrc tex; };
+template <int THREADS>
+__device__ __forceinline__ LevelSrc level_source(const FrameArgs& f, int l, int rb, int nb, float* lut) {
+    LevelSrc o;
+    const long long base = lvl_at(f.geom, l, rb);
+    o.X = f.X + base; o.Y = f.Y + base; o.Z = f.Z + base;
+    o.cam = make_level_cam(f.K, f.geom, l);
+    o.tex.tex8 = f.tex8 + tex_at(f.geom, l, nb); o.tex.d2 = f.d2 + lvl_at(f.geom, l, nb); o.tex.lut = lut;
+    const long long at = (long long)nb * f.geom.L + l;
+    const unsigned mx2 = f.maxd2[at];
+    o.tex.scale = dtn_scale(mx2, f.nedge_now[at]);
+    build_lut<THREADS>(lut, mx2, o.tex.scale);
+    return o;
 }
 
 // Reprojection of one reference edge point (computeJacobianOfNowFrame "Step 2/3", src/SolveDVO.cpp:327-345).
@@ -314,7 +243,7 @@ __device__ __forceinline__ void finish_point(const Proj& q, const float4 t, cons
         Jr[5] = A::diff2(a, q.py, b, q.px);
     }
     e = t.x;                                                                     // :446
-    if (weight_mode == DVO_WEIGHT_REF_CAUCHY) wgt = (ARITH == DVO_ARITH_EXACT) ? t.w : A::weight_ref(e);   // :450, :1051 (precomputed per texel)
+    if (weight_mode == DVO_WEIGHT_REF_CAUCHY) wgt = (ARITH == DVO_ARITH_EXACT) ? t.w : A::weight_ref(e);
     else if (weight_mode == DVO_WEIGHT_HUBER) { const float ae = fabsf(e); wgt = ae <= huber_k ? 1.0f : A::div(huber_k, ae); }
     else wgt = 1.0f;
 }
@@ -356,6 +285,27 @@ template <bool NEED_H> struct AccN { static constexpr int N = NEED_H ? 29 : 8; }
 // The covariance sweep (WSQ) appends [29] sum w eps^2 to the Gauss-Newton layout.
 constexpr int COV_NACC = AccN<true>::N + 1;
 
+// One visible point's terms (:714-720, :777): g += J w eps, sum eps^2, sum eps, (NEED_H) H += J w J^T, (WSQ) sum w eps^2.
+template <int ARITH, bool NEED_H, bool WSQ>
+__device__ __forceinline__ void accumulate_point(const float* Jr, float e, float wgt, double* acc, int& nvis) {
+    typedef Ar<ARITH> A;
+    ++nvis;
+    const double de = (double)e;
+    acc[6] = fma(de, de, acc[6]);
+    acc[7] += de;
+    if constexpr (WSQ) acc[COV_NACC - 1] = fma((double)wgt * de, de, acc[COV_NACC - 1]);   // double(w) * double(eps) is exact
+    double Jw[6];
+#pragma unroll
+    for (int k = 0; k < 6; ++k) { Jw[k] = (double)A::mul(Jr[k], wgt); acc[k] = fma(Jw[k], de, acc[k]); }
+    if (NEED_H) {
+        int idx = 8;
+#pragma unroll
+        for (int r = 0; r < 6; ++r)
+#pragma unroll
+            for (int c = r; c < 6; ++c) { acc[idx] = fma(Jw[r], (double)Jr[c], acc[idx]); ++idx; }
+    }
+}
+
 // Software-pipelined sweep over a thread's points: the coordinates are loaded two points ahead and the (random)
 // texel gather of the next point is in flight while the current point's Jacobian / fp64 accumulation executes.
 // (A counted loop with unconditional look-ahead loads into slack behind the arrays, unrolled by 1 / 2 / 3, was measured slower:
@@ -394,21 +344,7 @@ __device__ __forceinline__ void accumulate_points(const float* __restrict__ X, c
                 if (weight_mode == DVO_WEIGHT_REF_CAUCHY) wgt = A::weight_ref(e);
                 else if (weight_mode == DVO_WEIGHT_HUBER) { const float ae = fabsf(e); wgt = ae <= huber_k ? 1.0f : A::div(huber_k, ae); }
             }
-            ++nvis;
-            const double de = (double)e;
-            acc[6] = fma(de, de, acc[6]);
-            acc[7] += de;
-            if constexpr (WSQ) acc[COV_NACC - 1] = fma((double)wgt * de, de, acc[COV_NACC - 1]);   // double(w) * double(eps) is exact
-            double Jw[6];
-#pragma unroll
-            for (int k = 0; k < 6; ++k) { Jw[k] = (double)A::mul(Jr[k], wgt); acc[k] = fma(Jw[k], de, acc[k]); }   // :714-720, :777
-            if (NEED_H) {
-                int idx = 8;
-#pragma unroll
-                for (int r = 0; r < 6; ++r)
-#pragma unroll
-                    for (int c = r; c < 6; ++c) { acc[idx] = fma(Jw[r], (double)Jr[c], acc[idx]); ++idx; }
-            }
+            accumulate_point<ARITH, NEED_H, WSQ>(Jr, e, wgt, acc, nvis);
         } else {
 #pragma unroll
             for (int k = 0; k < 6; ++k) Jr[k] = 0.f;
@@ -443,7 +379,6 @@ __device__ __forceinline__ void accumulate_points_ring(const float* __restrict__
                                                        const PoseF& P, const LevelCam& cam, const TexSrc& S, double* acc, int& nvis,
                                                        unsigned char* ring) {
     static_assert((D & (D - 1)) == 0 && D >= 2, "ring depth must be a power of two");
-    typedef Ar<DVO_ARITH_EXACT> A;
     float4* ringP = reinterpret_cast<float4*>(ring);                               // [D][THREADS] {X, Y, Z, texel index}
     float2* ringUV = reinterpret_cast<float2*>(ring + D * THREADS * 16);            // [D][THREADS] reprojection (escape path only)
     uint2* ringT = reinterpret_cast<uint2*>(ring + D * THREADS * 24);               // [D][THREADS] texel, filled by cp.async
@@ -474,20 +409,7 @@ __device__ __forceinline__ void accumulate_points_ring(const float* __restrict__
             const float4 tv = resolve_texel(S, cam, q, ringT[slot]);
             float Jr[6], e, wgt;
             finish_point<DVO_ARITH_EXACT, JAC, DVO_WEIGHT_REF_CAUCHY>(q, tv, P, cam, DVO_WEIGHT_REF_CAUCHY, 0.f, Jr, e, wgt);
-            ++nvis;
-            const double de = (double)e;
-            acc[6] = fma(de, de, acc[6]);
-            acc[7] += de;
-            double Jw[6];
-#pragma unroll
-            for (int c = 0; c < 6; ++c) { Jw[c] = (double)A::mul(Jr[c], wgt); acc[c] = fma(Jw[c], de, acc[c]); }
-            if (NEED_H) {
-                int idx = 8;
-#pragma unroll
-                for (int r = 0; r < 6; ++r)
-#pragma unroll
-                    for (int c = r; c < 6; ++c) { acc[idx] = fma(Jw[r], (double)Jr[c], acc[idx]); ++idx; }
-            }
+            accumulate_point<DVO_ARITH_EXACT, NEED_H, false>(Jr, e, wgt, acc, nvis);
         }
     }
     cp_async_wait<0>();
@@ -502,18 +424,25 @@ __device__ __forceinline__ void accumulate_points_ring(const float* __restrict__
 // warp) is deliberate: a full [29][33] tile cost 61 KB per CTA of L1 capacity and slowed the gather-bound sweep.
 // The 8-accumulator sub-gradient case keeps the shuffle tree (its tile pass would not be shorter).
 // Stage 2: thread k sums the warp partials in warp order.
-template <int NACC> struct ReduceScratch {
+// The covariance's serial tail reuses scr as its 6x6 workspace.
+template <int NACC, int THREADS> struct ReduceScratch {
     static constexpr bool TRANSPOSED = (NACC > 8);
-    static constexpr int ROW = 36, PER_WARP = TRANSPOSED ? 8 * ROW : 1;
+    static constexpr int WARPS = THREADS / 32, ROW = 36, PER_WARP = TRANSPOSED ? 8 * ROW : 1;
+    double scr[TRANSPOSED ? WARPS * PER_WARP : 0];   // per-warp transposed tile (none for the shuffle tree)
+    double red[WARPS][NACC];        // warp partials
+    double tot[NACC];               // block sums
+    int nv[WARPS], nvtot;           // visible points per warp, per block
+    int stop;                       // solve: the lead's stop decision, read by every thread after the iteration's barrier
+                                    // (it fills the slot after nvtot: a flag of its own would move SolverState by 8 bytes and change
+                                    // how ptxas vectorises its stores)
 };
 
 template <int NACC, int THREADS>
-__device__ __forceinline__ void block_reduce(double* acc, int nvis, double* s_scr, double (*s_red)[NACC], int* s_nv, double* s_tot, int* s_nvtot) {
-    constexpr int SOLVE_WARPS = THREADS / 32;
-    typedef ReduceScratch<NACC> RS;
+__device__ __forceinline__ void block_reduce(double* acc, int nvis, ReduceScratch<NACC, THREADS>& R) {
+    typedef ReduceScratch<NACC, THREADS> RS;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (RS::TRANSPOSED) {
-        double* ws = s_scr + warp * RS::PER_WARP;
+        double* ws = R.scr + warp * RS::PER_WARP;
         const int r = lane >> 2, q = lane & 3;
 #pragma unroll
         for (int p0 = 0; p0 < NACC; p0 += 8) {
@@ -525,7 +454,7 @@ __device__ __forceinline__ void block_reduce(double* acc, int nvis, double* s_sc
             for (int j = 0; j < 8; ++j) v += ws[r * RS::ROW + 4 * j + q];
             v += __shfl_xor_sync(0xffffffffu, v, 1);
             v += __shfl_xor_sync(0xffffffffu, v, 2);
-            if (q == 0 && p0 + r < NACC) s_red[warp][p0 + r] = v;
+            if (q == 0 && p0 + r < NACC) R.red[warp][p0 + r] = v;
             __syncwarp();
         }
     } else {
@@ -534,19 +463,19 @@ __device__ __forceinline__ void block_reduce(double* acc, int nvis, double* s_sc
             double v = acc[k];
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-            if (lane == 0) s_red[warp][k] = v;
+            if (lane == 0) R.red[warp][k] = v;
         }
     }
     for (int o = 16; o > 0; o >>= 1) nvis += __shfl_down_sync(0xffffffffu, nvis, o);
-    if (lane == 0) s_nv[warp] = nvis;
+    if (lane == 0) R.nv[warp] = nvis;
     __syncthreads();
     if (threadIdx.x < NACC) {
         double v = 0.0;
 #pragma unroll
-        for (int wv = 0; wv < SOLVE_WARPS; ++wv) v += s_red[wv][threadIdx.x];
-        s_tot[threadIdx.x] = v;
+        for (int wv = 0; wv < RS::WARPS; ++wv) v += R.red[wv][threadIdx.x];
+        R.tot[threadIdx.x] = v;
     }
-    if (threadIdx.x == 32) { int n = 0; for (int wv = 0; wv < SOLVE_WARPS; ++wv) n += s_nv[wv]; *s_nvtot = n; }
+    if (threadIdx.x == 32) { int n = 0; for (int wv = 0; wv < RS::WARPS; ++wv) n += R.nv[wv]; R.nvtot = n; }
     __syncthreads();
 }
 
@@ -560,9 +489,7 @@ struct SolverState {
 };
 
 struct SolveArgs {
-    PyrGeom geom; Intr K;
-    const float *X, *Y, *Z; const int* npts; const unsigned* nedge_now;
-    const uint2* tex8; const int32_t* d2; const unsigned* maxd2;
+    FrameArgs f;
     const double* pose0; double* pose; dvo_pair_info* info; double* trace; int trace_iters; const int* order; const unsigned char* active;
     float* energy;
     dvo_solver_params prm; int first;
@@ -673,14 +600,16 @@ __device__ __forceinline__ void order_heaviest_first(int count, Work work, Id id
     }
 }
 
+// work of a launch entry whose reference data is slot s: sum_l iters[l] * npts[s][l]
+__device__ __forceinline__ unsigned slot_work(const int* __restrict__ npts, int L, const dvo_solver_params& prm, int s) {
+    unsigned wk = 0;
+    for (int l = 0; l < L; ++l) wk += (unsigned)max(prm.iters[l], 0) * (unsigned)npts[(long long)s * L + l];
+    return wk;
+}
+
 __global__ void __launch_bounds__(1024) solve_order_kernel(const int* __restrict__ npts, int L, dvo_solver_params prm, int first, int count,
                                                            int* __restrict__ order) {
-    auto work = [&](int i) {
-        unsigned wk = 0;
-        for (int l = 0; l < L; ++l) wk += (unsigned)max(prm.iters[l], 0) * (unsigned)npts[(long long)(first + i) * L + l];
-        return wk;
-    };
-    order_heaviest_first(count, work, [&](int i) { return first + i; }, order);
+    order_heaviest_first(count, [&](int i) { return slot_work(npts, L, prm, first + i); }, [&](int i) { return first + i; }, order);
 }
 
 // Pairs: the work of pair k is that of its reference slot (out-of-range slots weigh nothing); the list holds pair indices.
@@ -688,10 +617,7 @@ __global__ void __launch_bounds__(1024) pair_order_kernel(const int* __restrict_
                                                           const int* __restrict__ ref_slot, int* __restrict__ order) {
     auto work = [&](int k) {
         const int s = ref_slot[k];
-        unsigned wk = 0;
-        if (s < 0 || s >= Bmax) return wk;
-        for (int l = 0; l < L; ++l) wk += (unsigned)max(prm.iters[l], 0) * (unsigned)npts[(long long)s * L + l];
-        return wk;
+        return (s < 0 || s >= Bmax) ? 0u : slot_work(npts, L, prm, s);
     };
     order_heaviest_first(count, work, [](int k) { return k; }, order);
 }
@@ -709,24 +635,19 @@ template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, int 
 __device__ __forceinline__ void solve_body(const SolveArgs& a) {
     extern __shared__ float s_lut[];          // 2 * LUT_N floats, then the sweep's ring (PIPE > 0)
     constexpr int NACC = AccN<NEED_H>::N;
-    constexpr int SOLVE_WARPS = THREADS / 32;
-    __shared__ double s_scr[SOLVE_WARPS * ReduceScratch<NACC>::PER_WARP];
-    __shared__ double s_red[SOLVE_WARPS][NACC];
-    __shared__ double s_tot[NACC];
-    __shared__ int s_nv[SOLVE_WARPS];
-    __shared__ int s_nvtot, s_stop;
+    __shared__ ReduceScratch<NACC, THREADS> R;
     __shared__ PoseF s_pose;
     __shared__ SolverState S;
     __shared__ dvo_pair_info s_info;
 
     const int b = a.order[blockIdx.x];
     if (!PAIRS && a.active && !a.active[b]) return;       // masked pass (gated key-frame switch): pose / info of the slot stay as they are
-    const int L = a.geom.L;
+    const int L = a.f.geom.L;
     const bool lead = (threadIdx.x == 0);
     int rb = b, nb = b;                                   // slot of the reference data, slot of the now data
     if constexpr (PAIRS) {
         rb = a.ref_slot[b]; nb = a.now_slot[b];
-        if (rb < 0 || rb >= a.geom.Bmax || nb < 0 || nb >= a.geom.Bmax) {                     // status bit 1, NaN pose
+        if (rb < 0 || rb >= a.f.geom.Bmax || nb < 0 || nb >= a.f.geom.Bmax) {                     // status bit 1, NaN pose
             if (lead) {
                 const double qnan = __longlong_as_double(0x7ff8000000000000ll);
                 for (int k = 0; k < 12; ++k) a.pose[12 * (long long)b + k] = qnan;
@@ -745,7 +666,7 @@ __device__ __forceinline__ void solve_body(const SolveArgs& a) {
         for (int k = 0; k < 3; ++k) S.cT[k] = a.pose0[12 * (long long)b + 9 + k];
         s_info.status = 0; s_info.laplacian_b = 0.f;
         for (int l = 0; l < DVO_MAX_LEVELS; ++l) {
-            s_info.npts[l] = (l < L) ? a.npts[(long long)rb * L + l] : 0; s_info.best_index[l] = -1; s_info.iterations_run[l] = 0;
+            s_info.npts[l] = (l < L) ? a.f.npts[(long long)rb * L + l] : 0; s_info.best_index[l] = -1; s_info.iterations_run[l] = 0;
             s_info.best_energy[l] = 0.f; s_info.visible_ratio[l] = 0.f;
         }
     }
@@ -754,19 +675,20 @@ __device__ __forceinline__ void solve_body(const SolveArgs& a) {
     for (int l = L - 1; l >= 0; --l) {
         const int iters = a.prm.iters[l];
         if (iters <= 0) continue;
-        const int N = a.npts[(long long)rb * L + l];
-        const unsigned ne = a.nedge_now[(long long)nb * L + l];
+        const int N = a.f.npts[(long long)rb * L + l];
+        const unsigned ne = a.f.nedge_now[(long long)nb * L + l];
         if (N <= 0 || ne == 0u) { if (lead) s_info.status |= 1; continue; }                  // reference asserts (:282)
-        const long long base = lvl_at(a.geom, l, rb);
-        const float* X = a.X + base; const float* Y = a.Y + base; const float* Z = a.Z + base;
-        const LevelCam cam = make_level_cam(a.K, a.geom, l);
-        TexSrc src;
-        src.tex8 = a.tex8 + tex_at(a.geom, l, nb); src.lut = s_lut;
-        if constexpr (PAIRS) src.d2 = a.d2 + lvl_at(a.geom, l, nb);
-        else src.d2 = a.d2 + base;
-        const unsigned mx2 = a.maxd2[(long long)nb * L + l];
-        src.scale = dtn_scale(mx2, ne);
-        build_lut<THREADS>(s_lut, mx2, src.scale);           // visible after the barrier below
+        // level_source spelled out: with d2 taken at lvl_at(l, nb) for slot launches too, ptxas allocates the slot kernels'
+        // registers differently and their spills change
+        const long long base = lvl_at(a.f.geom, l, rb);
+        LevelSrc lv; lv.X = a.f.X + base; lv.Y = a.f.Y + base; lv.Z = a.f.Z + base;
+        lv.cam = make_level_cam(a.f.K, a.f.geom, l);
+        lv.tex.tex8 = a.f.tex8 + tex_at(a.f.geom, l, nb); lv.tex.lut = s_lut;
+        if constexpr (PAIRS) lv.tex.d2 = a.f.d2 + lvl_at(a.f.geom, l, nb);
+        else lv.tex.d2 = a.f.d2 + base;
+        const unsigned mx2 = a.f.maxd2[(long long)nb * L + l];
+        lv.tex.scale = dtn_scale(mx2, ne);
+        build_lut<THREADS>(s_lut, mx2, lv.tex.scale);
         if (lead) {
             S.bestE = 1.0E10f; S.bestRatio = 1.0f; S.bestItr = -1; S.bestSumEps = 0.0;        // :642-650
             for (int k = 0; k < 9; ++k) S.bestR[k] = (k % 4 == 0) ? 1.0 : 0.0;
@@ -775,7 +697,7 @@ __device__ __forceinline__ void solve_body(const SolveArgs& a) {
             S.have_acc = 0; S.lambda = a.prm.lm_lambda0; S.accE = 0.f;
             for (int k = 0; k < 9; ++k) s_pose.R[k] = (float)S.cR[k];                          // :673-674
             for (int k = 0; k < 3; ++k) s_pose.T[k] = (float)S.cT[k];
-            s_stop = 0;
+            R.stop = 0;
         }
         __syncthreads();
         for (int itr = 0; itr < iters; ++itr) {
@@ -785,21 +707,22 @@ __device__ __forceinline__ void solve_body(const SolveArgs& a) {
             for (int k = 0; k < NACC; ++k) acc[k] = 0.0;
             int nvis = 0;
             if constexpr (PIPE > 0 && JAC == DVO_JAC_REFERENCE)
-                accumulate_points_ring<JAC, NEED_H, THREADS, PIPE>(X, Y, Z, N, P, cam, src, acc, nvis, reinterpret_cast<unsigned char*>(s_lut) + LUT_BYTES);
+                accumulate_points_ring<JAC, NEED_H, THREADS, PIPE>(lv.X, lv.Y, lv.Z, N, P, lv.cam, lv.tex, acc, nvis,
+                                                                   reinterpret_cast<unsigned char*>(s_lut) + LUT_BYTES);
             else
-                accumulate_points<ARITH, JAC, NEED_H, THREADS, false, RES, WMODE>(X, Y, Z, N, P, cam, src, a.prm.weight, a.prm.huber_k, acc, nvis,
-                                                      nullptr, nullptr, nullptr, nullptr, nullptr);
-            block_reduce<NACC, THREADS>(acc, nvis, s_scr, s_red, s_nv, s_tot, &s_nvtot);
+                accumulate_points<ARITH, JAC, NEED_H, THREADS, false, RES, WMODE>(lv.X, lv.Y, lv.Z, N, P, lv.cam, lv.tex, a.prm.weight, a.prm.huber_k,
+                                                                                  acc, nvis, nullptr, nullptr, nullptr, nullptr, nullptr);
+            block_reduce<NACC, THREADS>(acc, nvis, R);
             if (lead) {
                 double* tr = nullptr;
                 if (!PAIRS && a.trace && itr < a.trace_iters)
                     tr = a.trace + (((long long)b * L + l) * a.trace_iters + itr) * DVO_TRACE_DOUBLES;
-                s_stop = solver_step<!PAIRS>(S, s_tot, s_nvtot, N, itr, a.prm, NEED_H, &s_info, l, tr, a.energy + ((long long)b * L + l) * DVO_ENERGY_ITERS);
+                R.stop = solver_step<!PAIRS>(S, R.tot, R.nvtot, N, itr, a.prm, NEED_H, &s_info, l, tr, a.energy + ((long long)b * L + l) * DVO_ENERGY_ITERS);
                 for (int k = 0; k < 9; ++k) s_pose.R[k] = (float)S.cR[k];                      // pose of the next iteration (:673-674)
                 for (int k = 0; k < 3; ++k) s_pose.T[k] = (float)S.cT[k];
             }
             __syncthreads();
-            if (s_stop) break;
+            if (R.stop) break;
         }
         if (lead) {
             for (int k = 0; k < 9; ++k) S.cR[k] = S.bestR[k];                                  // :997-1001
@@ -818,19 +741,36 @@ __device__ __forceinline__ void solve_body(const SolveArgs& a) {
 }
 
 template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, int PIPE>
-__global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768) / THREADS) solve_kernel(SolveArgs a) {
+__global__ void __launch_bounds__(THREADS, (NEED_H ? 512 : 768) / THREADS) solve_kernel(SolveArgs a) {
     solve_body<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE, false>(a);
 }
 template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, int PIPE>
-__global__ void __launch_bounds__(THREADS, (NEED_H ? DVO_GN_THREADS_PER_SM : 768) / THREADS) solve_pairs_kernel(SolveArgs a) {
+__global__ void __launch_bounds__(THREADS, (NEED_H ? 512 : 768) / THREADS) solve_pairs_kernel(SolveArgs a) {
     solve_body<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE, true>(a);
 }
 
 // ------------------------------------------------------------------ single evaluation (parity inspection)
+// The normal equations at pose P of the N reference points of slot rb against the now frame of slot nb at level l, with the
+// run-time weight mode: one sweep with H (plus sum w eps^2 when WSQ), then the block reduction.  The sums are in R.tot and
+// R.nvtot on every thread after the return.
+template <int ARITH, int JAC, int THREADS, int RES, bool OUT, bool WSQ>
+__device__ __forceinline__ void eval_normal_equations(const FrameArgs& f, int l, int rb, int nb, int N, const PoseF& P, int weight,
+                                                      float huber_k, float* lut, ReduceScratch<WSQ ? COV_NACC : AccN<true>::N, THREADS>& R,
+                                                      float* o_eps, float* o_w, float* o_u, float* o_v, float* o_J) {
+    constexpr int NACC = WSQ ? COV_NACC : AccN<true>::N;
+    const LevelSrc lv = level_source<THREADS>(f, l, rb, nb, lut);
+    __syncthreads();
+    double acc[NACC];
+#pragma unroll
+    for (int k = 0; k < NACC; ++k) acc[k] = 0.0;
+    int nvis = 0;
+    accumulate_points<ARITH, JAC, true, THREADS, OUT, RES, -1, WSQ>(lv.X, lv.Y, lv.Z, N, P, lv.cam, lv.tex, weight, huber_k, acc, nvis,
+                                                                     o_eps, o_w, o_u, o_v, o_J);
+    block_reduce<NACC, THREADS>(acc, nvis, R);
+}
+
 struct EvalArgs {
-    PyrGeom geom; Intr K;
-    const float *X, *Y, *Z; const int* npts;
-    const uint2* tex8; const int32_t* d2; const unsigned* maxd2; const unsigned* nedge_now;
+    FrameArgs f;
     const double* pose; int slot, level, weight; float huber_k;
     double* out;            // g[6], H[36], sumsq, nvis
     float *eps, *w, *u, *v, *J;
@@ -839,38 +779,18 @@ struct EvalArgs {
 template <int ARITH, int JAC, int RES>
 __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs a) {
     extern __shared__ float s_lut[];
-    constexpr int NACC = AccN<true>::N;
-    constexpr int SOLVE_WARPS = EVAL_THREADS / 32;
-    __shared__ double s_scr[SOLVE_WARPS * ReduceScratch<NACC>::PER_WARP];
-    __shared__ double s_red[SOLVE_WARPS][NACC];
-    __shared__ double s_tot[NACC];
-    __shared__ int s_nv[SOLVE_WARPS];
-    __shared__ int s_nvtot;
-    const int b = a.slot, l = a.level, L = a.geom.L;
-    const int N = a.npts[(long long)b * L + l];
-    const long long base = lvl_at(a.geom, l, b);
+    __shared__ ReduceScratch<AccN<true>::N, EVAL_THREADS> R;
+    const int b = a.slot, l = a.level;
     PoseF P;
     for (int k = 0; k < 9; ++k) P.R[k] = (float)a.pose[k];
     for (int k = 0; k < 3; ++k) P.T[k] = (float)a.pose[9 + k];
-    const LevelCam cam = make_level_cam(a.K, a.geom, l);
-    TexSrc src;
-    src.tex8 = a.tex8 + tex_at(a.geom, l, b); src.d2 = a.d2 + base; src.lut = s_lut;
-    const unsigned mx2 = a.maxd2[(long long)b * L + l];
-    src.scale = dtn_scale(mx2, a.nedge_now[(long long)b * L + l]);
-    build_lut<EVAL_THREADS>(s_lut, mx2, src.scale);
-    __syncthreads();
-    double acc[NACC];
-#pragma unroll
-    for (int k = 0; k < NACC; ++k) acc[k] = 0.0;
-    int nvis = 0;
-    accumulate_points<ARITH, JAC, true, EVAL_THREADS, true, RES, -1>(a.X + base, a.Y + base, a.Z + base, N, P, cam, src, a.weight, a.huber_k,
-                                        acc, nvis, a.eps, a.w, a.u, a.v, a.J);
-    block_reduce<NACC, EVAL_THREADS>(acc, nvis, s_scr, s_red, s_nv, s_tot, &s_nvtot);
+    eval_normal_equations<ARITH, JAC, EVAL_THREADS, RES, true, false>(a.f, l, b, b, a.f.npts[(long long)b * a.f.geom.L + l], P, a.weight,
+                                                                      a.huber_k, s_lut, R, a.eps, a.w, a.u, a.v, a.J);
     if (threadIdx.x == 0) {
-        for (int k = 0; k < 6; ++k) a.out[k] = s_tot[k];
+        for (int k = 0; k < 6; ++k) a.out[k] = R.tot[k];
         int idx = 8;
-        for (int r = 0; r < 6; ++r) for (int c = r; c < 6; ++c) { a.out[6 + 6 * r + c] = s_tot[idx]; a.out[6 + 6 * c + r] = s_tot[idx]; ++idx; }
-        a.out[42] = s_tot[6]; a.out[43] = (double)s_nvtot;
+        for (int r = 0; r < 6; ++r) for (int c = r; c < 6; ++c) { a.out[6 + 6 * r + c] = R.tot[idx]; a.out[6 + 6 * c + r] = R.tot[idx]; ++idx; }
+        a.out[42] = R.tot[6]; a.out[43] = (double)R.nvtot;
     }
 }
 
@@ -881,9 +801,7 @@ __global__ void __launch_bounds__(EVAL_THREADS) eval_kernel(EvalArgs a) {
 // fixed (COV_THREADS), so a slot's result never depends on how many slots share the launch.  Reads c->pose only.
 constexpr int COV_THREADS = 256;
 struct CovArgs {
-    PyrGeom geom; Intr K;
-    const float *X, *Y, *Z; const int* npts;
-    const uint2* tex8; const int32_t* d2; const unsigned* maxd2; const unsigned* nedge_now;
+    FrameArgs f;
     const double* pose; int first, level, weight; float huber_k;
     double* cov;            // 36 doubles per slot, record of CTA k at cov + 36 * k * stride
     dvo_cov_info* info;     // optional, same indexing
@@ -935,23 +853,17 @@ __device__ __forceinline__ bool cov_from_normal_matrix(double* M, double s2, dou
 template <int RES, bool PAIRS>
 __device__ __forceinline__ void cov_body(const CovArgs& a) {
     extern __shared__ float s_lut[];
-    constexpr int NACC = COV_NACC;
-    constexpr int WARPS = COV_THREADS / 32;
-    __shared__ double s_scr[WARPS * ReduceScratch<NACC>::PER_WARP];
-    __shared__ double s_red[WARPS][NACC];
-    __shared__ double s_tot[NACC];
-    __shared__ int s_nv[WARPS];
-    __shared__ int s_nvtot;
-    const int b = a.first + blockIdx.x, l = a.level, L = a.geom.L;
+    __shared__ ReduceScratch<COV_NACC, COV_THREADS> R;
+    const int b = a.first + blockIdx.x, l = a.level, L = a.f.geom.L;
     if (!PAIRS && a.active && !a.active[b]) return;       // masked pass (key-frame switch): the slot's record stays as it is
     int rb = b, nb = b;                                   // slot of the reference data, slot of the now data
     bool in_range = true;
     if constexpr (PAIRS) {
         rb = a.ref_slot[b]; nb = a.now_slot[b];
-        in_range = rb >= 0 && rb < a.geom.Bmax && nb >= 0 && nb < a.geom.Bmax;
+        in_range = rb >= 0 && rb < a.f.geom.Bmax && nb >= 0 && nb < a.f.geom.Bmax;
     }
-    const int N = in_range ? a.npts[(long long)rb * L + l] : 0;
-    const unsigned ne = in_range ? a.nedge_now[(long long)nb * L + l] : 0u;
+    const int N = in_range ? a.f.npts[(long long)rb * L + l] : 0;
+    const unsigned ne = in_range ? a.f.nedge_now[(long long)nb * L + l] : 0u;
     double* out = a.cov + 36 * (long long)blockIdx.x * a.stride;
     dvo_cov_info* inf = a.info ? a.info + (long long)blockIdx.x * a.stride : nullptr;
     int status = 0, nvis = 0;
@@ -960,31 +872,16 @@ __device__ __forceinline__ void cov_body(const CovArgs& a) {
         PoseF P;
         for (int k = 0; k < 9; ++k) P.R[k] = (float)a.pose[12 * (long long)b + k];
         for (int k = 0; k < 3; ++k) P.T[k] = (float)a.pose[12 * (long long)b + 9 + k];
-        const long long base = lvl_at(a.geom, l, rb);
-        const LevelCam cam = make_level_cam(a.K, a.geom, l);
-        TexSrc src;
-        src.tex8 = a.tex8 + tex_at(a.geom, l, nb); src.lut = s_lut;
-        if constexpr (PAIRS) src.d2 = a.d2 + lvl_at(a.geom, l, nb);
-        else src.d2 = a.d2 + base;
-        const unsigned mx2 = a.maxd2[(long long)nb * L + l];
-        src.scale = dtn_scale(mx2, ne);
-        build_lut<COV_THREADS>(s_lut, mx2, src.scale);
-        __syncthreads();
-        double acc[NACC];
-#pragma unroll
-        for (int k = 0; k < NACC; ++k) acc[k] = 0.0;
-        int nv = 0;
-        accumulate_points<DVO_ARITH_EXACT, DVO_JAC_EXACT, true, COV_THREADS, false, RES, -1, true>(
-            a.X + base, a.Y + base, a.Z + base, N, P, cam, src, a.weight, a.huber_k, acc, nv, nullptr, nullptr, nullptr, nullptr, nullptr);
-        block_reduce<NACC, COV_THREADS>(acc, nv, s_scr, s_red, s_nv, s_tot, &s_nvtot);
+        eval_normal_equations<DVO_ARITH_EXACT, DVO_JAC_EXACT, COV_THREADS, RES, false, true>(a.f, l, rb, nb, N, P, a.weight, a.huber_k, s_lut, R,
+                                                                                           nullptr, nullptr, nullptr, nullptr, nullptr);
         if (threadIdx.x != 0) return;
-        nvis = s_nvtot;
+        nvis = R.nvtot;
         if (nvis < 7) status |= 2;
         else {
-            double* M = s_scr;                            // the reduction scratch is free again
+            double* M = R.scr;                            // the reduction scratch is free again
             int idx = 8;
-            for (int r = 0; r < 6; ++r) for (int c = r; c < 6; ++c) { M[6 * r + c] = s_tot[idx]; M[6 * c + r] = s_tot[idx]; ++idx; }
-            sigma2 = s_tot[NACC - 1] / (double)(nvis - 6);
+            for (int r = 0; r < 6; ++r) for (int c = r; c < 6; ++c) { M[6 * r + c] = R.tot[idx]; M[6 * c + r] = R.tot[idx]; ++idx; }
+            sigma2 = R.tot[COV_NACC - 1] / (double)(nvis - 6);
             double ldH = 0.0;
             if (cov_from_normal_matrix(M, sigma2, out, &ldH)) logdet = 6.0 * log(sigma2) - ldH;
             else status |= 4;
@@ -1009,23 +906,20 @@ __global__ void __launch_bounds__(COV_THREADS) cov_pairs_kernel(CovArgs a) { cov
 // ------------------------------------------------------------------ packed texels -> float images (parity inspection)
 // {DTn, gx, gy, w} of every pixel of one slot / level through exactly the code path the solver uses (packed texel or
 // escaped d2 stencil, lookup table or direct evaluation), so that dvo_get_level_buffer checks that path pixel by pixel.
-struct ResolveArgs { PyrGeom geom; const uint2* tex8; const int32_t* d2; const unsigned* maxd2; const unsigned* nedge_now; int slot, level; float4* out; };
+struct ResolveArgs { FrameArgs f; int slot, level; float4* out; };
 
 __global__ void __launch_bounds__(256) resolve_texels_kernel(ResolveArgs a) {
     extern __shared__ float s_lut[];
-    const int b = a.slot, l = a.level, L = a.geom.L;
-    const int w = a.geom.w[l], h = a.geom.h[l], tw = a.geom.tw[l];
-    const unsigned mx2 = a.maxd2[(long long)b * L + l];
-    const float scale = dtn_scale(mx2, a.nedge_now[(long long)b * L + l]);
-    build_lut<256>(s_lut, mx2, scale);
+    const LevelSrc lv = level_source<256>(a.f, a.level, a.slot, a.slot, s_lut);
     __syncthreads();
-    const uint2* __restrict__ tex = a.tex8 + tex_at(a.geom, l, b);
-    const int32_t* __restrict__ d2 = a.d2 + lvl_at(a.geom, l, b);
+    const int w = lv.cam.w, h = lv.cam.h;
+    const uint2* __restrict__ tex = lv.tex.tex8;
+    const int32_t* __restrict__ d2 = lv.tex.d2;
     for (int i = blockIdx.x * 256 + threadIdx.x; i < w * h; i += gridDim.x * 256) {
         const int y = i / w, x = i - y * w;
         Stencil s;
-        if (!unpack_texel(__ldg(tex + tex_index(x, y, tw)), s)) stencil_from_d2(d2, w, h, x, y, s);
-        a.out[i] = texel_values(s, s_lut, scale);
+        if (!unpack_texel(__ldg(tex + tex_index(x, y, lv.cam.tw)), s)) stencil_from_d2(d2, w, h, x, y, s);
+        a.out[i] = texel_values(s, s_lut, lv.tex.scale);
     }
 }
 
@@ -1113,8 +1007,9 @@ static cudaError_t optin_lut_smem(int device, int bytes = LUT_BYTES) {
 // PAIRS selects solve_pairs_kernel, the same configuration launched over pairs (dvo_align_pairs)
 template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, int WMODE, bool PAIRS>
 static cudaError_t launch_solve_w(dvo_ctx* c, const SolveArgs& a, int count) {
-    // the shipped configuration (reference Jacobian, getWeightOf weights) takes the ring sweep
-    constexpr int PIPE = (WMODE == DVO_WEIGHT_REF_CAUCHY && JAC == DVO_JAC_REFERENCE) ? (NEED_H ? DVO_SOLVE_PIPE_GN : DVO_SOLVE_PIPE_SG) : 0;
+    // the shipped configuration (reference Jacobian, getWeightOf weights) takes the ring sweep, 4 deep for the 29-accumulator
+    // kernel and 2 deep for the 8-accumulator (sub-gradient) one; every other configuration the register pipeline
+    constexpr int PIPE = (WMODE == DVO_WEIGHT_REF_CAUCHY && JAC == DVO_JAC_REFERENCE) ? (NEED_H ? 4 : 2) : 0;
     constexpr int SMEM = LUT_BYTES + PIPE * THREADS * 32;
     constexpr auto kern = PAIRS ? solve_pairs_kernel<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE> : solve_kernel<ARITH, JAC, NEED_H, THREADS, RES, WMODE, PIPE>;
     const cudaError_t e = optin_lut_smem<SolveArgs, kern>(c->cfg.device, SMEM);
@@ -1127,7 +1022,7 @@ static cudaError_t launch_solve_w(dvo_ctx* c, const SolveArgs& a, int count) {
 // compile time; every other combination takes the generic kernel that branches on the run-time value
 template <int ARITH, int JAC, bool NEED_H, int THREADS, int RES, bool PAIRS>
 static cudaError_t launch_solve_inst(dvo_ctx* c, const SolveArgs& a, int count) {
-    if (DVO_WMODE_SPECIALIZE && ARITH == DVO_ARITH_EXACT && RES == DVO_RESIDUAL_DT_FLOOR && a.prm.weight == DVO_WEIGHT_REF_CAUCHY)
+    if (ARITH == DVO_ARITH_EXACT && RES == DVO_RESIDUAL_DT_FLOOR && a.prm.weight == DVO_WEIGHT_REF_CAUCHY)
         return launch_solve_w<ARITH, JAC, NEED_H, THREADS, RES, (ARITH == DVO_ARITH_EXACT && RES == DVO_RESIDUAL_DT_FLOOR) ? DVO_WEIGHT_REF_CAUCHY : -1, PAIRS>(c, a, count);
     return launch_solve_w<ARITH, JAC, NEED_H, THREADS, RES, -1, PAIRS>(c, a, count);
 }
@@ -1166,12 +1061,18 @@ static cudaError_t dispatch_solve(dvo_ctx* c, const SolveArgs& a, int count, con
     return launch_solve_t<DVO_ARITH_FAST, DVO_JAC_EXACT, PAIRS>(c, a, count, need_h);
 }
 
+static FrameArgs frame_args(const dvo_ctx* c) {
+    FrameArgs f;
+    f.geom = c->geom; f.K = c->K; f.X = c->ptsX; f.Y = c->ptsY; f.Z = c->ptsZ; f.npts = c->npts;
+    f.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L;
+    f.tex8 = c->tex8; f.d2 = c->d2; f.maxd2 = c->maxd2;
+    return f;
+}
+
 static SolveArgs solve_args(dvo_ctx* c, const dvo_solver_params* p) {
     SolveArgs a;
     memset(&a, 0, sizeof(a));
-    a.geom = c->geom; a.K = c->K; a.X = c->ptsX; a.Y = c->ptsY; a.Z = c->ptsZ; a.npts = c->npts;
-    a.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L;
-    a.tex8 = c->tex8; a.d2 = c->d2; a.maxd2 = c->maxd2;
+    a.f = frame_args(c);
     a.prm = *p;
     return a;
 }
@@ -1213,8 +1114,7 @@ static cudaError_t launch_eval_inst(dvo_ctx* c, const EvalArgs& a) {
 int launch_eval(dvo_ctx* c, int slot, int level, const double* d_pose12, int jac, int weight, int arith, float huber_k, int residual,
                 double* d_out, float* d_eps, float* d_w, float* d_u, float* d_v, float* d_J) {
     EvalArgs a;
-    a.geom = c->geom; a.K = c->K; a.X = c->ptsX; a.Y = c->ptsY; a.Z = c->ptsZ; a.npts = c->npts;
-    a.tex8 = c->tex8; a.d2 = c->d2; a.maxd2 = c->maxd2; a.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L;
+    a.f = frame_args(c);
     a.pose = d_pose12; a.slot = slot; a.level = level; a.weight = weight; a.huber_k = huber_k; a.out = d_out;
     a.eps = d_eps; a.w = d_w; a.u = d_u; a.v = d_v; a.J = d_J;
     const bool ex = arith != DVO_ARITH_FAST, rj = jac != DVO_JAC_EXACT;
@@ -1234,8 +1134,7 @@ int launch_eval(dvo_ctx* c, int slot, int level, const double* d_pose12, int jac
 
 int launch_resolve_texels(dvo_ctx* c, int slot, int level, float4* d_out) {
     ResolveArgs a;
-    a.geom = c->geom; a.tex8 = c->tex8; a.d2 = c->d2; a.maxd2 = c->maxd2;
-    a.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L; a.slot = slot; a.level = level; a.out = d_out;
+    a.f = frame_args(c); a.slot = slot; a.level = level; a.out = d_out;
     DVO_CUDA((optin_lut_smem<ResolveArgs, resolve_texels_kernel>(c->cfg.device)));
     const int blocks = (c->geom.P[level] + 255) / 256;
     resolve_texels_kernel<<<blocks < 64 ? blocks : 64, 256, LUT_BYTES, c->stream>>>(a);
@@ -1258,8 +1157,7 @@ static int launch_cov_t(dvo_ctx* c, int first, int count, int level, const dvo_s
     if (count == 0) return DVO_OK;
     CovArgs a;
     memset(&a, 0, sizeof(a));
-    a.geom = c->geom; a.K = c->K; a.X = c->ptsX; a.Y = c->ptsY; a.Z = c->ptsZ; a.npts = c->npts;
-    a.tex8 = c->tex8; a.d2 = c->d2; a.maxd2 = c->maxd2; a.nedge_now = c->nedge + (size_t)DVO_FRAME_NOW * c->geom.Bmax * c->geom.L;
+    a.f = frame_args(c);
     a.pose = c->pose; a.first = first; a.level = level; a.weight = p->weight; a.huber_k = p->huber_k;
     a.cov = d_cov; a.info = d_info; a.stride = stride;
     if (PAIRS) { a.pose = c->pair_pose; a.ref_slot = c->pair_ref; a.now_slot = c->pair_now; }
